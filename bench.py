@@ -5,6 +5,7 @@ residual+Jacobian observations/s on the 24-camera x 1 M-point rig, 1/2/4/8 B200)
     python bench.py --gpus N --steps K --warmup W            # this engine (default: config 3)
     python bench.py --config {1,2,3,4,5} ...                 # BASELINE.json configs[config-1]
     python bench.py --impl reference --steps K --warmup W    # CPU path (scipy least_squares)
+    python bench.py ... --dump-outputs DIR                   # also save the last timed step's results
 
 A step is ONE trust-region (LM) outer iteration over the whole observation set:
 linearise -> reduced camera system -> Cholesky -> back-substitution -> trial cost ->
@@ -12,6 +13,12 @@ on-device accept/reject (reference equivalent: one pass of scipy trf.py:465-578)
 N > 1 shards the SAME problem by point (strong scaling, NCCL all-reduce of the reduced
 camera system); launch with torchrun (RANK/LOCAL_RANK/WORLD_SIZE in the env).
 Prints one JSON line on rank 0.
+
+--dump-outputs DIR writes, after the timed steps of the headline workload, what the last of them
+handed back to its caller, as float64 .npy files: cameras.npy (C x 11), points3d.npy (P x 3),
+cost.npy and optimality.npy.  The inputs depend on the arguments only (seeded), so two builds run
+with the same arguments can be compared file for file.  The files stay under DUMP_MAX_BYTES: above
+that, points3d.npy holds a fixed seeded sample of the rows, listed in points3d_rows.npy.
 """
 from __future__ import annotations
 
@@ -24,6 +31,8 @@ import time
 
 import numpy as np
 
+# the bench may run from a read-only checkout and must leave the tree as it found it
+sys.dont_write_bytecode = True
 REPO = os.path.dirname(os.path.abspath(__file__))
 if REPO not in sys.path:
     sys.path.insert(0, REPO)
@@ -43,6 +52,7 @@ CONFIGS = {
     5: dict(rig="ring64", points=10_000_000, pvis=0.5, what="64-camera rig, 10M points, p_vis 0.5 (8 GPUs)"),
 }
 N_CAMS = {"ring4": 4, "example18": 18, "ring24": 24, "wide8": 8, "ring64": 64, "ring8": 8}
+DUMP_MAX_BYTES = 64_000_000
 
 
 def load_peaks():
@@ -95,6 +105,23 @@ def pinned(a):
     import torch
     t = torch.from_numpy(np.ascontiguousarray(a)).pin_memory()
     return t.numpy(), t
+
+
+def dump_outputs(directory, cams, pts, cost, optimality):
+    """Write the solver's results as float64 .npy files (see the module docstring)."""
+    os.makedirs(directory, exist_ok=True)
+    out = {"cameras": np.asarray(cams, dtype=np.float64), "cost": np.array([cost], dtype=np.float64),
+           "optimality": np.array([optimality], dtype=np.float64)}
+    pts = np.asarray(pts, dtype=np.float64)
+    room = DUMP_MAX_BYTES - 5 * 128 - sum(a.nbytes for a in out.values())     # 128-byte .npy headers
+    if pts.nbytes > room:
+        # each sampled row costs 3 coordinates + its row number
+        rows = np.sort(np.random.default_rng(0).choice(pts.shape[0], room // (4 * 8), replace=False))
+        out["points3d_rows"] = rows.astype(np.float64)
+        pts = pts[rows]
+    out["points3d"] = pts
+    for name, a in out.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def workload_string(cfg_id, rig, points, pvis):
@@ -178,7 +205,12 @@ def main():
     ap.add_argument("--cpu-points", type=int, default=None)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl == "reference":
+        ap.error("--dump-outputs saves the results of this engine's timed steps; --impl reference has none")
     K, W = args.steps, max(args.warmup, 0)
     cfg = dict(CONFIGS[args.config])
     rig = args.rig or cfg["rig"]
@@ -245,9 +277,10 @@ def main():
     fp64_peak = FP64_PEAK_FALLBACK_TFLOPS
     tol = dict(ftol=1e-4, xtol=1e-8, gtol=1e-8, max_nfev=200)
 
-    def device_run(pb, k_steps, w_steps, sample_clocks=False, per_kernel=True):
+    def device_run(pb, k_steps, w_steps, sample_clocks=False, per_kernel=True, keep_params=False):
         """Device-resident rate of `k_steps` real outer iterations (bundleAdjust(1e-4) from the standard
-        perturbed x0, repeated from x0 until k_steps are done), plus per-kernel CUDA-event times."""
+        perturbed x0, repeated from x0 until k_steps are done), plus per-kernel CUDA-event times.
+        keep_params: also return the parameters the last timed step left (this rank's points)."""
         sh = D.shard_problem(pb["pts0"], pb["points_2d"], pb["camera_ind"], pb["point_ind"], None, rank, ws)
         eng = Engine(local)
         eng.set_problem(pb["cams0"], sh["pts"], sh["points_2d"], sh["camera_ind"], sh["point_ind"],
@@ -285,7 +318,10 @@ def main():
         clocks = sampler.stop() if sampler else None
         total_ms = max_over_ranks(dev_ms)
         out = dict(steps=steps_done, ms_per_step=total_ms / max(1, steps_done), launches=launches,
-                   final_cost=res.cost, nfev=int(res.nfev), clocks=clocks, shard=sh, engine=eng, prof={})
+                   final_cost=res.cost, optimality=res.optimality, nfev=int(res.nfev), clocks=clocks, shard=sh,
+                   engine=eng, prof={})
+        if keep_params:     # before the profiled pass below restarts from x0
+            out["params"] = eng.get_params()
         if per_kernel:
             barrier()
             out["prof"] = run_steps(k_steps, profile=True)[4]
@@ -364,8 +400,14 @@ def main():
     # ---- headline: device-resident run ----
     pb = make_rig(rig, points, seed=0, variant="volume", p_vis=pvis)
     C, P, N = pb["n_cams"], pb["n_points"], pb["n_obs"]
-    run = device_run(pb, K, W, sample_clocks=True)
+    run = device_run(pb, K, W, sample_clocks=True, keep_params=args.dump_outputs is not None)
     eng, sh = run["engine"], run["shard"]
+    if args.dump_outputs is not None:
+        cams_out, pts_out = run.pop("params")
+        pts_out = D.allgather_rows(pts_out, sh["bounds"])         # collective: every rank takes part
+        if rank == 0:
+            dump_outputs(args.dump_outputs, cams_out, pts_out, run["final_cost"], run["optimality"])
+        del cams_out, pts_out
     roof, roof_m1, ms_jac, ms_res = rooflines(pb, sh, run, eng)
     eng.close()
     n_loc = sh["point_ind"].size
