@@ -252,6 +252,12 @@ int lcba_debug_i8_plan(int32_t C, int64_t P, int32_t sm_count, int32_t* tiles_ou
                        int32_t* work_out, int32_t max_work, int32_t* nwork_out, int32_t* nrg_out,
                        int64_t* nkb_out);
 
+/* 1 when the last Schur pass of the int8 tensor-core path found a camera row whose largest |Y| entry is more
+ * than 4x the square root of its Schur diagonal (finer than the 48-bit digits resolve) and recomputed the
+ * pass with the FP64 DMMA kernel; 0 when the int8 result stood; -1 when the handle does not use the int8
+ * path.  Synchronises the handle's stream. */
+int lcba_debug_i8_fallback(lcba_t* h);
+
 /* Measurement switch (tools/peer_ab.py): all-reduce through NVLink peer memory (csrc/peer_reduce.cuh; needs LCBA_PEER_REDUCE=1 or 2 at
  * lcba_comm_init so that every rank has mapped every peer's block) or through ncclAllReduce, from the next call on.  Collective in the
  * sense that every rank must switch at the same point.  Returns 1 if the peer path is active afterwards. */

@@ -21,7 +21,8 @@ SYMBOLS = ["lcba_version", "lcba_create", "lcba_destroy", "lcba_last_error", "lc
            "lcba_get_trace", "lcba_get_grad", "lcba_get_profile", "lcba_linearize",
            "lcba_time_device", "lcba_nccl_unique_id", "lcba_comm_init", "lcba_debug_tr2d",
            "lcba_sq_normal", "lcba_debug_schur_stats", "lcba_debug_mma_plan",
-           "lcba_set_iteration_callback", "lcba_debug_i8_plan", "lcba_host_is_nondecreasing_i64", "lcba_debug_peer_reduce"]
+           "lcba_set_iteration_callback", "lcba_debug_i8_plan", "lcba_host_is_nondecreasing_i64", "lcba_debug_peer_reduce",
+           "lcba_debug_i8_fallback"]
 
 
 class Options(C.Structure):
@@ -109,6 +110,7 @@ def load():
     lib.lcba_debug_i8_plan.argtypes = [i32, i64, i32, vp, i32, vp, i32, C.POINTER(i32), C.POINTER(i32), C.POINTER(i64)]
     lib.lcba_host_is_nondecreasing_i64.argtypes = [vp, i64, i32]
     lib.lcba_debug_peer_reduce.argtypes = [vp, i32]
+    lib.lcba_debug_i8_fallback.argtypes = [vp]
     lib.lcba_debug_tr2d.argtypes = [dbl, dbl, dbl, dbl, dbl, dbl, pd, C.POINTER(C.c_int)]
     _lib = lib
     return lib
@@ -321,6 +323,11 @@ class Engine:
         self._check(self.lib.lcba_linearize(self.h, float(lam), _ptr(S), _ptr(rhs), _ptr(g),
                                             _ptr(sc), C.byref(cost)))
         return dict(S=S, rhs=rhs, grad=g, scale_inv=sc, cost=cost.value)
+
+    def i8_fell_back(self):
+        """1: the last Schur pass of the int8 path was recomputed on DMMA (rows finer than its digits resolve),
+        0: the int8 result stood, -1: this handle does not use the int8 path."""
+        return self.lib.lcba_debug_i8_fallback(self.h)
 
     def time_device(self, what, reps=10):
         ms = C.c_double()

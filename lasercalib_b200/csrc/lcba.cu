@@ -125,6 +125,9 @@ struct lcba_handle {
   unsigned char* d_i8planes = nullptr;
   double *d_i8partial = nullptr, *d_i8rmax = nullptr;
   int* d_i8erow = nullptr;
+  int* d_i8gate = nullptr;        // 1: the last Schur pass fell back to DMMA (k_i8_check)
+  double* d_i8mrow = nullptr;     // row maxima of Y (k_i8_rowexp -> k_i8_check)
+  bool i8_guard = true;          // LCBA_I8_GUARD=0: no resolution check (tests of the int8 kernels alone)
   int i8_gx_max = 0, i8_gx_make = 0, i8_groups = 0;
   // outputs on demand
   double2* d_rout = nullptr;
@@ -609,6 +612,13 @@ extern "C" int lcba_set_problem_shard(lcba_t* h, int32_t C, int64_t P, int64_t N
         LCBA_TRY(dev_alloc(h, &h->d_i8partial, ip.work.size() * 128 * 64));
         LCBA_TRY(dev_alloc(h, &h->d_i8rmax, (size_t)h->i8_gx_max * ip.NRG * 8));
         LCBA_TRY(dev_alloc(h, &h->d_i8erow, (size_t)ip.NRG * 8));
+        LCBA_TRY(dev_alloc(h, &h->d_i8gate, 1));
+        LCBA_TRY(dev_alloc(h, &h->d_i8mrow, (size_t)ip.NRG * 8));
+        LCBA_CUDA(h, cudaMemsetAsync(h->d_i8gate, 0, sizeof(int), st));
+        {
+          const char* ge = getenv("LCBA_I8_GUARD");
+          h->i8_guard = !(ge && atoi(ge) == 0);
+        }
       }
       bool pre = false;
       if (!h->use_i8) {
@@ -962,7 +972,8 @@ static int pass_schur(lcba_t* h, const double* lam_host_or_null) {
       const size_t smem_rm = ((size_t)I8_GROUP_CAMS * CAMTAB + 192) * 4;
       KL(h, "i8_rowmax", k_i8_rowmax<<<dim3(h->i8_gx_max, h->i8_groups), 192, smem_rm, h->stream>>>(
             h->d_tab[w], h->d_pts[w], h->d_pair_w, h->d_pair_start, h->d_mask, h->d_Lz, h->P, C, RP, h->d_i8rmax));
-      KL(h, "i8_rowmax", k_i8_rowexp<<<nblk(RP, 128), 128, 0, h->stream>>>(h->d_i8rmax, h->i8_gx_max, NCP * C + 1, RP, h->d_i8erow));
+      KL(h, "i8_rowmax", k_i8_rowexp<<<nblk(RP, 128), 128, 0, h->stream>>>(h->d_i8rmax, h->i8_gx_max, NCP * C + 1, RP,
+                                                                     h->d_i8erow, h->d_i8mrow));
       KL(h, "make_Y", k_i8_make<<<dim3(h->i8_gx_make, h->i8_groups), 192, i8_make_smem_bytes(), h->stream>>>(
             h->d_tab[w], h->d_pts[w], h->d_pair_w, h->d_pair_start, h->d_mask, h->d_Lz, h->P, C, ip.NRG, h->d_i8erow,
             h->d_i8planes));
@@ -975,6 +986,26 @@ static int pass_schur(lcba_t* h, const double* lam_host_or_null) {
       KL(h, "schur_reduce", k_i8_gather<<<dim3((unsigned)ip.tiles.size(), 16), 256, 0, h->stream>>>(
             h->d_i8partial, h->d_i8tiles, C, h->d_i8erow, pl.npairs, h->d_Sred));
       KL(h, "schur_reduce", k_add_cam_blocks<<<nblk(C * 121, 128), 128, 0, h->stream>>>(h->d_U, C, h->d_Sred));
+      // rows whose maximum comes from one point far above their Schur diagonal: the DMMA kernel (Y evaluated in
+      // place) redoes this pass; both launches return at once unless k_i8_check raised the gate
+      if (h->i8_guard) {
+        KL(h, "i8_check", k_i8_check<<<1, 256, 0, h->stream>>>(h->d_i8mrow, C, h->d_Sred, h->d_i8gate));
+#define LCBA_MMA_GATED(L)                                                                            \
+  KL(h, "i8_fallback", (k_schur_mma<L, false><<<dim3(mp.nslices, mp.nkinds), MMA_THREADS, mp.smem_bytes, h->stream>>>( \
+          nullptr, h->d_tab[w], h->d_pts[w], h->d_pair_w, h->d_pair_start, h->d_mask, h->d_Lz, h->P, h->n_pairs, C, \
+          h->d_mkinds, mp.nslices, pl.part_stride, pl.npairs, h->d_Spart, nullptr, h->d_i8gate)))
+        switch (last) {
+          case 1: LCBA_MMA_GATED(1); break;
+          case 2: LCBA_MMA_GATED(2); break;
+          case 3: LCBA_MMA_GATED(3); break;
+          case 4: LCBA_MMA_GATED(4); break;
+          case 5: LCBA_MMA_GATED(5); break;
+          default: LCBA_MMA_GATED(6); break;
+        }
+#undef LCBA_MMA_GATED
+        KL(h, "i8_fallback", k_i8_fallback_finish<<<h->sm_count, 256, 0, h->stream>>>(
+              h->d_i8gate, h->d_Spart, mp.nslices, pl.part_stride, h->d_U, C, h->d_Sred));
+      }
     } else {
     if (h->d_Yg) {
       const int pbk = MAKEY_THREADS / C, rpk = mp.kinds[0].rp;
@@ -1629,6 +1660,17 @@ extern "C" int lcba_debug_schur_stats(lcba_t* h, long long* out, int max_ctas, i
   *nkinds = nk;
   *nslices = ns;
   return LCBA_OK;
+}
+
+// test hook: 1 when the last Schur pass of the int8 path handed the pass to DMMA (k_i8_check), 0 when the int8
+// result stood, -1 when the handle does not use the int8 path
+extern "C" int lcba_debug_i8_fallback(lcba_t* h) {
+  if (!h || !h->have_problem || !h->use_i8 || !h->d_i8gate) return -1;
+  cudaSetDevice(h->device);
+  int v = 0;
+  if (cudaStreamSynchronize(h->stream) != cudaSuccess ||
+      cudaMemcpy(&v, h->d_i8gate, sizeof(int), cudaMemcpyDeviceToHost) != cudaSuccess) return -1;
+  return v;
 }
 
 // host-only test hook: the unit plan of the tensor-path Schur kernel for C cameras (no GPU needed).

@@ -21,6 +21,8 @@
 //                   0..6-i of the columns in ONE instruction, N <= 256, A kept in the collector, widest last);
 //                   K ranges per tile weighted by the measured cost of a K block (make_i8_plan)
 //   k_i8_gather   : per-CTA partials -> the pair-block layout of Sred (fixed order, no atomics)
+//   k_i8_check    : resolution guard: rows whose maximum lies far above their Schur diagonal hand the pass to
+//                   the DMMA kernel (k_schur_mma, gated) and k_i8_fallback_finish
 #pragma once
 #include <cuda.h>
 #include <algorithm>
@@ -378,8 +380,10 @@ k_i8_rowmax(const double* __restrict__ tab, const double* __restrict__ pts, cons
   }
 }
 
-// e_row[r]: |y| 2^-e < 0.25 (two bits of headroom: the top digit stays below 65); rows without data: 0
-__global__ void k_i8_rowexp(const double* __restrict__ rmax_part, int nb, int R, int RP, int* __restrict__ e_row) {
+// e_row[r]: |y| 2^-e < 0.25 (two bits of headroom: the top digit stays below 65); rows without data: 0.
+// m_row[r]: the row maximum itself (for k_i8_check)
+__global__ void k_i8_rowexp(const double* __restrict__ rmax_part, int nb, int R, int RP, int* __restrict__ e_row,
+                            double* __restrict__ m_row) {
   const int r = blockIdx.x * blockDim.x + threadIdx.x;
   if (r >= RP) return;
   double m = 0.0;
@@ -387,6 +391,7 @@ __global__ void k_i8_rowexp(const double* __restrict__ rmax_part, int nb, int R,
   int e = 0;
   if (m > 0.0 && m < 1e300) { frexp(m * 1.001, &e); e += 2; }    // maxima come from an FP32 evaluation: 1e-3 of slack
   e_row[r] = e;
+  m_row[r] = m;
 }
 
 // 48-bit integer T -> the 6 balanced digits as the bytes of one word: digit i (0 = most significant)
@@ -793,6 +798,54 @@ k_i8_gather(const double* __restrict__ partial, const I8Tile* __restrict__ tiles
     double* blk = Sred + (size_t)(cj * (cj + 1) / 2 + ck) * 121;
     blk[ra * NCP + cb] = v;
     if (cj == ck && ra != cb) blk[cb * NCP + ra] = v;
+  }
+}
+
+// Resolution guard.  The digits hold every entry of row r to 48 bits of the row's maximum m_r, so the error of
+// S_rc is ~ 2^-47 m_r m_c (measured 0.9 - 3.4 x that).  Where one point sets m_r far above the row's Schur
+// diagonal (a heavily weighted point close to a camera: m_r^2 = 1.4e3 S_rr, Jacobi-scaled error 3.3e-11),
+// that is coarser than FP64 needs.  One block: *gate = 1 when some camera row has m_r^2 > I8_RHO_MAX S_rr
+// (S_rr = the diagonal of this shard's U - Y Y^T: a sum of per-point PSD terms, so never above the global
+// one), then the DMMA kernel recomputes the slice partials and k_i8_fallback_finish replaces Sred.
+// I8_RHO_MAX = 16 keeps 2^-47 * 3.4 * 16 = 4e-13 under a 1e-12 Jacobi-scaled error; ordinary rigs stay
+// near 1e-3 (ring24, example18, ring64) and weights over six decades near 0.2.
+constexpr double I8_RHO_MAX = 16.0;
+__global__ void __launch_bounds__(256)
+k_i8_check(const double* __restrict__ m_row, int C, const double* __restrict__ Sred, int* __restrict__ gate) {
+  int bad = 0;
+  for (int r = threadIdx.x; r < NCP * C; r += blockDim.x) {
+    const double m = m_row[r];
+    if (m > 0.0) {
+      const int c = r / NCP, a = r % NCP;
+      const double d = Sred[(size_t)(c * (c + 1) / 2 + c) * 121 + a * NCP + a];
+      if (!(m * m <= I8_RHO_MAX * d)) bad = 1;
+    }
+  }
+  bad = __syncthreads_or(bad);
+  if (threadIdx.x == 0) *gate = bad;
+}
+
+// only when *gate: Sred = sum of the DMMA slice partials (fixed order) + U on the camera blocks
+__global__ void __launch_bounds__(256)
+k_i8_fallback_finish(const int* __restrict__ gate, const double* __restrict__ part, int nslices, size_t K,
+                     const double* __restrict__ U, int C, double* __restrict__ Sred) {
+  if (*gate == 0) return;
+  for (size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x; j < K; j += (size_t)gridDim.x * blockDim.x) {
+    double s = 0.0;
+    for (int b = 0; b < nslices; ++b) s += part[(size_t)b * K + j];
+    const size_t blk = j / 121;
+    if (j < (size_t)C * (C + 1) / 2 * 121) {
+      // camera blocks are pair blocks cj * (cj + 1) / 2 + cj
+      int c = (int)((sqrt(8.0 * (double)blk + 1.0) - 1.0) * 0.5);
+      while (c * (c + 1) / 2 > (long long)blk) --c;
+      while ((c + 1) * (c + 2) / 2 <= (long long)blk) ++c;
+      if ((size_t)(c * (c + 1) / 2 + c) == blk) {
+        const int e = (int)(j % 121), a = e / NCP, b2 = e % NCP;
+        const int lo = a < b2 ? a : b2, hi = a < b2 ? b2 : a;
+        s += U[c * CAMN_VALS + lo * NCP - lo * (lo - 1) / 2 + (hi - lo)];
+      }
+    }
+    Sred[j] = s;
   }
 }
 

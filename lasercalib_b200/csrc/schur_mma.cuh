@@ -318,7 +318,8 @@ k_schur_mma(const double* __restrict__ Yg, const double* __restrict__ tab, const
             const unsigned long long* __restrict__ mask, const double* __restrict__ Lz,
             long long P, long long N, int C, const MmaKind* __restrict__ kinds, int nslices,
             size_t part_stride, int npairs, double* __restrict__ part,
-            long long* __restrict__ stats) {
+            long long* __restrict__ stats, const int* __restrict__ gate = nullptr /* non-null: run only if *gate */) {
+  if (gate && *gate == 0) return;
   extern __shared__ __align__(16) double s_dyn[];
   const MmaKind& K = kinds[blockIdx.y];
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;

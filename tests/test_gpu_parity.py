@@ -368,8 +368,10 @@ def test_int8_tensor_core_schur_equals_fp64_paths(Engine, monkeypatch, C):
 
 
 def test_int8_tensor_core_schur_at_depth_and_trajectory(Engine, monkeypatch):
-    """ring24 x 20011 dense points (953 K blocks: ring laps, several TMEM flushes per CTA, ragged
-    last block) vs the oracle, then a full trajectory on ring24 x 5000 against oracle.trf_exact."""
+    """ring24 x 20011 dense points (953 K blocks, ragged last block) vs the oracle, then a full
+    trajectory on ring24 x 5000 against oracle.trf_exact.  On 148 SMs the longest K range of the plan
+    is 96 blocks, under I8_FLUSH = 224: every CTA flushes TMEM once.  The multi-flush path and the
+    default dispatch at >= 32768 points are tested in test_gpu_i8_scale.py."""
     monkeypatch.setenv("LCBA_SCHUR_I8", "1")
     pb = make_rig("ring24", 20011, seed=7, variant="volume", p_vis=1.0)
     S_or, rhs_or, cost_or = _oracle_reduced(pb, 1e-5)
