@@ -232,6 +232,33 @@ int lcba_comm_init(lcba_t* h, int32_t rank, int32_t nranks, const void* id128);
 int lcba_debug_tr2d(double B00, double B01, double B11, double g0, double g1, double Delta,
                     double* p_out2, int* newton_out);
 
+/* The dense camera solve of the solver (csrc/dense.cuh: k_copy_damped_rhs + k_chol_fused) on a host
+ * system: Cholesky of A + mu*diag(d^2) (A n x n row-major, lower triangle read; 1 <= n <= 704) and
+ * x = (A + mu*diag(d^2))^-1 rhs, with `grid` cooperative CTAs (0: the solver's own choice; above the
+ * co-resident limit: LCBA_E_ARG).  d may be NULL when mu == 0.  x_out n; factor_out (n+1) x n or NULL:
+ * the work buffer as the kernel leaves it (strict lower triangle L, 1 / l_jj on the diagonal, row n =
+ * z = L^-1 rhs, upper triangle untouched); fail_out: bit 0 = non-positive or NaN pivot, bit 1 = grid
+ * barrier timed out. */
+int lcba_debug_chol(lcba_t* h, int32_t n, const double* A, const double* rhs, double mu, const double* d,
+                    int32_t grid, double* x_out, double* factor_out, int32_t* fail_out);
+
+/* One Gauss-Newton step of the solver on the resident problem at its current x, through the same
+ * kernels lcba_solve launches: linearise (first-call scaling, Delta = |x * scale_inv|), the Cauchy
+ * reg_term, point factors and the reduced camera system damped with `lam` (it overrides reg_term,
+ * like lcba_linearize), the dense camera solve with extra damping mu * Dc^2, back-substitution and the
+ * 2-D subspace scalars.  mode 0: all parameters; 1: cameras fixed (fix_cameras); 2: shared
+ * intrinsics.  pc_out 11C (the camera step, expanded in mode 2; zeros in mode 1), pp_out 3P (the
+ * point step); scalars_out LCBA_STEP_SCALARS doubles:
+ *   [0] reg_term  [1] Delta  [2] Jg2 = |J D^-2 g|^2
+ *   [3] aa  [4] ab  [5] bb      (a = g_h = g / s, b = gn_h = p * s, scaled space)
+ *   [6] JAA [7] JAB [8] JBB     (|J D^-2 g|^2, (J D^-2 g).(J p), |J p|^2)
+ *   [9] gtgt [10] gtp [11] pp   (g~ = D^-2 g and p, unscaled)
+ *   [12] c0 [13] c1 [14] predicted [15] step_h_norm [16] step_norm  (step = c0 g~ + c1 p)
+ *   [17] fail word of the camera solve (as in lcba_debug_chol). */
+#define LCBA_STEP_SCALARS 18
+int lcba_debug_step(lcba_t* h, double lam, double mu, int32_t mode, double* pc_out, double* pp_out,
+                    double* scalars_out);
+
 /* ---- profiling hook --------------------------------------------------------------------
  * Per-CTA cycle counters of the last Schur launch (4 int64 per CTA, [kind][slice]); only
  * filled when the process runs with LCBA_SCHUR_STATS=1 (tools/schur_stats.py). */

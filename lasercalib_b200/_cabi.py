@@ -22,7 +22,11 @@ SYMBOLS = ["lcba_version", "lcba_create", "lcba_destroy", "lcba_last_error", "lc
            "lcba_time_device", "lcba_nccl_unique_id", "lcba_comm_init", "lcba_debug_tr2d",
            "lcba_sq_normal", "lcba_debug_schur_stats", "lcba_debug_mma_plan",
            "lcba_set_iteration_callback", "lcba_debug_i8_plan", "lcba_host_is_nondecreasing_i64", "lcba_debug_peer_reduce",
-           "lcba_debug_i8_fallback"]
+           "lcba_debug_i8_fallback", "lcba_debug_chol", "lcba_debug_step"]
+
+# scalars_out of lcba_debug_step, in order (include/lcba.h)
+STEP_SCALARS = ["reg_term", "Delta", "Jg2", "aa", "ab", "bb", "JAA", "JAB", "JBB", "gtgt", "gtp", "pp",
+                "c0", "c1", "predicted", "step_h_norm", "step_norm", "chol_fail"]
 
 
 class Options(C.Structure):
@@ -112,6 +116,8 @@ def load():
     lib.lcba_debug_peer_reduce.argtypes = [vp, i32]
     lib.lcba_debug_i8_fallback.argtypes = [vp]
     lib.lcba_debug_tr2d.argtypes = [dbl, dbl, dbl, dbl, dbl, dbl, pd, C.POINTER(C.c_int)]
+    lib.lcba_debug_chol.argtypes = [vp, i32, vp, vp, dbl, vp, i32, vp, vp, C.POINTER(i32)]
+    lib.lcba_debug_step.argtypes = [vp, dbl, dbl, i32, vp, vp, vp]
     _lib = lib
     return lib
 
@@ -328,6 +334,35 @@ class Engine:
         """1: the last Schur pass of the int8 path was recomputed on DMMA (rows finer than its digits resolve),
         0: the int8 result stood, -1: this handle does not use the int8 path."""
         return self.lib.lcba_debug_i8_fallback(self.h)
+
+    def debug_chol(self, A, rhs, mu=0.0, d=None, grid=0):
+        """The solver's dense camera solve on a host system (lcba_debug_chol): returns (x, factor, fail)
+        with factor the (n+1, n) work buffer (strict lower L, 1 / l_jj on the diagonal, row n = L^-1 rhs)."""
+        A = _f64(A)
+        n = A.shape[0]
+        if A.shape != (n, n):
+            raise ValueError("A must be square")
+        rhs = _f64(rhs).ravel()
+        d = None if d is None else _f64(d).ravel()
+        if rhs.size != n or (d is not None and d.size != n):
+            raise ValueError("rhs and d must have n entries")
+        x = np.empty(n)
+        factor = np.empty((n + 1, n))
+        fail = C.c_int32()
+        self._check(self.lib.lcba_debug_chol(self.h, n, _ptr(A), _ptr(rhs), float(mu), _ptr(d), int(grid),
+                                             _ptr(x), _ptr(factor), C.byref(fail)))
+        return x, factor, fail.value
+
+    STEP_FULL, STEP_FIX_CAMERAS, STEP_SHARED_INTRINSICS = 0, 1, 2
+
+    def debug_step(self, lam, mu=0.0, mode=0):
+        """One Gauss-Newton step of the solver's passes at the current x (lcba_debug_step), damped with
+        lam: (camera step 11 C, point step 3 P, dict of the STEP_SCALARS)."""
+        pc = np.empty(11 * self.C)
+        pp = np.empty(3 * self.P)
+        sc = np.empty(len(STEP_SCALARS))
+        self._check(self.lib.lcba_debug_step(self.h, float(lam), float(mu), int(mode), _ptr(pc), _ptr(pp), _ptr(sc)))
+        return pc, pp, dict(zip(STEP_SCALARS, sc.tolist()))
 
     def time_device(self, what, reps=10):
         ms = C.c_double()

@@ -11,6 +11,7 @@ struct Ctl {
   double c0, c1, predicted, actual, ratio, step_norm, step_h_norm, mu;
   double camp[4];       // camera parts of (|g_h|^2, |x*scl|^2, |x|^2, max|g|)
   double BS[3], gS0, R00, R01, R11, gtgt, gtp, pp;   // 2-D model in the orthonormal basis
+  double aa, ab, bb, JAA, JAB, JBB;                  // Gram totals of k_ctl_sub (lcba_debug_step)
   double ftol, xtol;
   int accept, term, chol_fail, nonfinite, first, retry, degenerate, pad;
 };
@@ -223,6 +224,8 @@ k_ctl_sub(const double* __restrict__ red, const double* __restrict__ g_c,
   ctl->gtgt = red[6] + w[3];
   ctl->gtp = red[7] + w[4];
   ctl->pp = red[8] + w[5];
+  ctl->aa = aa; ctl->ab = ab; ctl->bb = bb;
+  ctl->JAA = JAA; ctl->JAB = JAB; ctl->JBB = JBB;
   ctl->chol_fail = *chol_fail;
   const double chk = JAB + JBB + ab + bb;
   ctl->retry = (!(chk - chk == 0.0) || ctl->chol_fail) ? 1 : 0;

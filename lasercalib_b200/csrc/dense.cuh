@@ -24,6 +24,9 @@ constexpr int CH_NB = 32;
 //     exchange; the pivot is inverted once (rsqrt) and the DIAGONAL OF THE FACTOR STORES
 //     1 / l_jj, so that panel rows and both substitutions multiply instead of divide;
 //   * panel rows and trailing tiles are spread over the grid; two grid barriers per panel;
+//   * the factored diagonal block goes back to A (CTA 0, from shared memory) only after the
+//     panel's first grid barrier, when no CTA can still be reading the original block; so the
+//     factor and the solution depend on the input alone, bit-identical for every grid size;
 //   * CTA 0 finishes with the blocked back substitution L^T x = z.
 // The grid barrier is a monotonic counter in global memory (release add / acquire poll);
 // the launch is cooperative so all CTAs are co-resident, and the poll is bounded: a stuck
@@ -93,6 +96,17 @@ k_chol_fused(double* A, int n, double* __restrict__ out, int* sync, long long* d
   unsigned phase = 0;
   long long tm[6] = {0, 0, 0, 0, 0, 0}, tc = dbg ? clock64() : 0;
 #define CH_TICK(i) do { if (dbg) { const long long now_ = clock64(); tm[i] += now_ - tc; tc = now_; } } while (0)
+  // CTA 0 stores the factored diagonal block of panel k (strict lower L_kk, 1 / l_jj on the
+  // diagonal) from shared memory.  Every CTA reads the ORIGINAL block in its own step 1, so the
+  // store waits for the first grid barrier of the panel (the closing barrier for the last one);
+  // nobody reads the global block in between.
+  auto store_diag = [&](int k, int nb) {
+    if (b != 0) return;
+    for (int e = t; e < CH_NB * CH_NB; e += 256) {
+      const int r = e / CH_NB, c = e % CH_NB;
+      if (r < nb && c <= r) A[(size_t)(k + r) * n + k + c] = (c < r) ? D[r][c] : rinv[r];
+    }
+  };
 
   for (int k = 0; k < n; k += CH_NB) {
     const int nb = min(CH_NB, n - k);
@@ -112,22 +126,14 @@ k_chol_fused(double* A, int n, double* __restrict__ out, int* sync, long long* d
 #pragma unroll
       for (int j = 0; j < CH_NB; ++j)
         if (lane == j) rinv[j] = dg[j];
-      if (b == 0 && lane < nb) {
-#pragma unroll
-        for (int j = 0; j < CH_NB; ++j) {
-          if (j < lane) A[(size_t)(k + lane) * n + k + j] = a[j];
-          if (j == lane) A[(size_t)(k + lane) * n + k + j] = dg[j];
-        }
-      }
     }
     __syncthreads();
     CH_TICK(0);
     // 2. panel rows below (and the rhs row n):  x L^T = a, one row per thread, rows dealt
-    //    round-robin over the CTAs
+    //    round-robin over the CTAs (up to n + 1 - 32 rows: small grids take several per thread)
     {
       const int rows = n + 1 - (k + nb);
-      const int i = t * G + b;
-      if (i < rows) {
+      for (int i = t * G + b; i < rows; i += 256 * G) {
         double* row = A + (size_t)(k + nb + i) * n + k;
         double x[CH_NB];
 #pragma unroll
@@ -149,6 +155,7 @@ k_chol_fused(double* A, int n, double* __restrict__ out, int* sync, long long* d
     CH_TICK(1);
     grid_barrier(counter, (++phase) * G, fail);
     CH_TICK(2);
+    store_diag(k, nb);
     // 3. trailing update, 32 x 32 tiles (ti >= tj), rows up to n (rhs), columns < n, dealt
     //    round-robin over the CTAs; thread = (column lane, rows wid + 8 m)
     {
@@ -199,6 +206,8 @@ k_chol_fused(double* A, int n, double* __restrict__ out, int* sync, long long* d
   }
   grid_barrier(counter, (++phase) * G, fail);
   if (b != 0) return;
+  store_diag(CH_NB * ((n - 1) / CH_NB), n - CH_NB * ((n - 1) / CH_NB));
+  __syncthreads();
   CH_TICK(4);
   // 4. back substitution L^T x = z (z = row n), CTA 0; the diagonal holds 1 / l_jj
   for (int i = t; i < n; i += 256) y[i] = __ldcg(A + (size_t)n * n + i);

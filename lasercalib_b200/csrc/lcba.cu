@@ -1067,6 +1067,19 @@ static int pass_schur(lcba_t* h, const double* lam_host_or_null) {
   return check_launch(h, "schur pass");
 }
 
+// grid of k_chol_fused = trailing tiles of the first panel (one tile per CTA), capped at
+// LCBA_CHOL_GRID (read once per process, default 64) and the SM count; all CTAs co-resident
+static int chol_grid(int n, int sm_count) {
+  int tiles = 1;
+  if (n > CH_NB) {
+    const int ntr = (n + 1 - CH_NB + CH_NB - 1) / CH_NB, ntc = (n - CH_NB + CH_NB - 1) / CH_NB;
+    tiles = 0;
+    for (int ti = 0; ti < ntr; ++ti) tiles += std::min(ti + 1, ntc);
+  }
+  static const int cap = getenv("LCBA_CHOL_GRID") ? atoi(getenv("LCBA_CHOL_GRID")) : 64;
+  return std::max(1, std::min(tiles, std::min(cap, sm_count)));
+}
+
 // Cholesky of S + mu*Dc^2, solve for the camera step
 static int pass_camera_solve(lcba_t* h, double mu) {
   NvtxRange nvtx_("lcba:camera_solve");
@@ -1077,15 +1090,7 @@ static int pass_camera_solve(lcba_t* h, double mu) {
   {
     KL(h, "chol_copy", k_copy_damped_rhs<<<nblk((long long)(n + 1) * n, 256), 256, 0, h->stream>>>(
           h->d_S, n, mu, scl, h->d_rhs, h->d_Lf));
-    // grid = trailing tiles of the first panel (one tile per CTA), capped; all CTAs co-resident
-    int tiles = 1;
-    if (n > CH_NB) {
-      const int ntr = (n + 1 - CH_NB + CH_NB - 1) / CH_NB, ntc = (n - CH_NB + CH_NB - 1) / CH_NB;
-      tiles = 0;
-      for (int ti = 0; ti < ntr; ++ti) tiles += std::min(ti + 1, ntc);
-    }
-    static const int cap = getenv("LCBA_CHOL_GRID") ? atoi(getenv("LCBA_CHOL_GRID")) : 64;
-    int grid = std::max(1, std::min(tiles, std::min(cap, h->sm_count)));
+    const int grid = chol_grid(n, h->sm_count);
     double* A = h->d_Lf;
     int nn = n;
     int* sync = h->d_fail;
@@ -1799,6 +1804,92 @@ extern "C" int lcba_debug_tr2d(double B00, double B01, double B11, double g0, do
   p_out[0] = t.p0;
   p_out[1] = t.p1;
   if (newton_out) *newton_out = t.newton;
+  return LCBA_OK;
+}
+
+// test hook: k_copy_damped_rhs + k_chol_fused on a host matrix with an explicit cooperative grid
+extern "C" int lcba_debug_chol(lcba_t* h, int32_t n, const double* A, const double* rhs, double mu, const double* d,
+                               int32_t grid, double* x_out, double* factor_out, int32_t* fail_out) {
+  if (!h) return LCBA_E_ARG;
+  if (n < 1 || n > CH_MAXN || !A || !rhs || !x_out || (mu != 0.0 && !d)) {
+    set_error(h, "lcba_debug_chol: n outside 1..704, or a NULL array");
+    return LCBA_E_ARG;
+  }
+  cudaSetDevice(h->device);
+  int per_sm = 0;
+  LCBA_CUDA(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, (const void*)k_chol_fused, 256, 0));
+  if (grid == 0) grid = chol_grid(n, h->sm_count);
+  if (grid < 1 || grid > per_sm * h->sm_count) {
+    set_error(h, "lcba_debug_chol: grid outside 1.." + std::to_string(per_sm * h->sm_count) + " (co-resident CTAs)");
+    return LCBA_E_ARG;
+  }
+  cudaStream_t st = h->stream;
+  double *dA = nullptr, *drhs = nullptr, *dd = nullptr, *dL = nullptr, *dx = nullptr;
+  int* dsync = nullptr;
+  cudaError_t e = cudaMallocAsync(&dA, (size_t)n * n * 8, st);
+  if (e == cudaSuccess) e = cudaMallocAsync(&drhs, (size_t)n * 8, st);
+  if (e == cudaSuccess && d) e = cudaMallocAsync(&dd, (size_t)n * 8, st);
+  if (e == cudaSuccess) e = cudaMallocAsync(&dL, (size_t)(n + 1) * n * 8, st);
+  if (e == cudaSuccess) e = cudaMallocAsync(&dx, (size_t)n * 8, st);
+  if (e == cudaSuccess) e = cudaMallocAsync(&dsync, 2 * sizeof(int), st);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(dA, A, (size_t)n * n * 8, cudaMemcpyHostToDevice, st);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(drhs, rhs, (size_t)n * 8, cudaMemcpyHostToDevice, st);
+  if (e == cudaSuccess && d) e = cudaMemcpyAsync(dd, d, (size_t)n * 8, cudaMemcpyHostToDevice, st);
+  if (e == cudaSuccess) e = cudaMemsetAsync(dsync, 0, 2 * sizeof(int), st);
+  if (e == cudaSuccess) {
+    k_copy_damped_rhs<<<nblk((long long)(n + 1) * n, 256), 256, 0, st>>>(dA, n, mu, dd, drhs, dL);
+    long long* dbg = nullptr;
+    int nn = n;
+    void* args[] = {(void*)&dL, (void*)&nn, (void*)&dx, (void*)&dsync, (void*)&dbg};
+    e = cudaLaunchCooperativeKernel((const void*)k_chol_fused, dim3(grid), dim3(256), args, 0, st);
+    h->launches += 2;
+  }
+  int fail = 0;
+  if (e == cudaSuccess) e = cudaMemcpyAsync(x_out, dx, (size_t)n * 8, cudaMemcpyDeviceToHost, st);
+  if (e == cudaSuccess && factor_out) e = cudaMemcpyAsync(factor_out, dL, (size_t)(n + 1) * n * 8, cudaMemcpyDeviceToHost, st);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(&fail, dsync, sizeof(int), cudaMemcpyDeviceToHost, st);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+  void* tmp[] = {dA, drhs, dd, dL, dx, dsync};
+  for (void* q : tmp) if (q) cudaFreeAsync(q, st);
+  if (e != cudaSuccess) { set_error(h, std::string("lcba_debug_chol: ") + cudaGetErrorString(e)); return LCBA_E_CUDA; }
+  if (fail_out) *fail_out = fail;
+  return LCBA_OK;
+}
+
+// test hook: one Gauss-Newton step of the solver's passes on the resident problem, damped with the host's lam
+extern "C" int lcba_debug_step(lcba_t* h, double lam, double mu, int32_t mode, double* pc_out, double* pp_out,
+                               double* scalars_out) {
+  if (!h || !h->have_problem) { set_error(h, "lcba_debug_step: no problem set"); return LCBA_E_STATE; }
+  if (mode < 0 || mode > 2) { set_error(h, "lcba_debug_step: mode must be 0, 1 or 2"); return LCBA_E_ARG; }
+  cudaSetDevice(h->device);
+  Ctl init;
+  memset(&init, 0, sizeof(init));
+  init.term = -1;
+  LCBA_CUDA(h, cudaMemcpyAsync(h->d_ctl, &init, sizeof(Ctl), cudaMemcpyHostToDevice, h->stream));
+  h->fix_cameras = mode == 1 ? 1 : 0;
+  h->shared_intr = mode == 2 ? 1 : 0;
+  LCBA_TRY(pass_linearize(h, 1));
+  LCBA_TRY(pass_jdot(h));
+  if (h->fix_cameras) {
+    KL(h, "point_factor", k_point_factor<<<nblk(h->P, 256), 256, 0, h->stream>>>(
+          h->d_Vg, h->d_scl_p, lam, nullptr, h->P, h->d_Lz));
+    LCBA_CUDA(h, cudaMemsetAsync(h->d_pc, 0, (size_t)h->C * NCP * 8, h->stream));
+    LCBA_CUDA(h, cudaMemsetAsync(h->d_fail, 0, 2 * sizeof(int), h->stream));
+  } else {
+    LCBA_TRY(pass_schur(h, &lam));
+    LCBA_TRY(pass_camera_solve(h, mu));
+  }
+  LCBA_TRY(pass_backsub(h));
+  if (pc_out) LCBA_CUDA(h, cudaMemcpyAsync(pc_out, h->d_pc, (size_t)h->C * NCP * 8, cudaMemcpyDeviceToHost, h->stream));
+  if (pp_out) LCBA_CUDA(h, cudaMemcpyAsync(pp_out, h->d_gn_p, (size_t)h->P * 3 * 8, cudaMemcpyDeviceToHost, h->stream));
+  LCBA_TRY(read_ctl(h));
+  if (scalars_out) {
+    const Ctl& c = *h->h_ctl;
+    const double v[LCBA_STEP_SCALARS] = {c.reg_term, c.Delta, c.Jg2, c.aa, c.ab, c.bb, c.JAA, c.JAB, c.JBB,
+                                         c.gtgt, c.gtp, c.pp, c.c0, c.c1, c.predicted, c.step_h_norm,
+                                         c.step_norm, (double)c.chol_fail};
+    memcpy(scalars_out, v, sizeof(v));
+  }
   return LCBA_OK;
 }
 

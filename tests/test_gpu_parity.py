@@ -489,6 +489,29 @@ def test_trajectory_matches_exact_trf_oracle(Engine, golden, name):
     got = [row["reg_term"] for row in trace[1:]]
     np.testing.assert_allclose(got[:2], regs_o[:2], rtol=1e-7)
     np.testing.assert_allclose(got, regs_o, rtol=1e-2)      # later ones: tiny, noisy gradients
+    # the other columns of scipy's table: optimality of every row; step norm and cost reduction of
+    # the trial that ended the previous iteration (0 when it was rejected).  Rows 0 and 1 (x0 and
+    # the first step from it) agree to round-off: measured on a B200 (1000 W) 2.5e-10 relative at
+    # most.  After that the ~1e-7 differences of the iterates explained above move the gradient and
+    # the next step by that order of their INITIAL size, while both shrink by orders of magnitude:
+    # measured at most 6.6e-7 of row 0's optimality and 1.6e-6 of |x0| for the step norm (ring4),
+    # hence bounds of 2e-6 and 5e-6 on those scales.  The cost reduction is a difference of two
+    # costs: the cost tolerance against the row's cost (measured 9.6e-8).
+    x0n = np.linalg.norm(_x0(g))
+    opt_o = np.array([rec["g_norm"] for rec in ora.trace] + [ora.optimality])
+    opt_g = np.array([row["optimality"] for row in trace])
+    np.testing.assert_allclose(opt_g[:2], opt_o[:2], rtol=1e-8)
+    assert np.all(np.abs(opt_g - opt_o) <= 2e-6 * opt_o[0]), (opt_g, opt_o)
+    last = [rec["trials"][-1] for rec in ora.trace]
+    red_o = np.array([t["actual"] if t["actual"] > 0 else 0.0 for t in last])
+    step_o = np.array([t["step_norm"] if t["actual"] > 0 else 0.0 for t in last])
+    assert np.isnan(trace[0]["cost_reduction"]) and np.isnan(trace[0]["step_norm"])
+    step_g = np.array([row["step_norm"] for row in trace[1:]])
+    np.testing.assert_allclose(step_g[0], step_o[0], rtol=1e-9)
+    assert np.all(np.abs(step_g - step_o) <= 5e-6 * x0n), (step_g, step_o)
+    red_g = np.array([row["cost_reduction"] for row in trace[1:]])
+    np.testing.assert_allclose(red_g[0], red_o[0], rtol=1e-9)
+    assert np.all(np.abs(red_g - red_o) <= 3e-7 * np.array(costs_o[:-1])), (red_g, red_o)
     np.testing.assert_allclose(res.cost, ora.cost, rtol=1e-9)
     # final reprojection RMSE within 1e-6 px (north-star tolerance); observed ~1e-10
     assert abs(O.rmse_px(f) - O.rmse_px(ora.fun)) < 1e-6
