@@ -270,14 +270,25 @@ int lcba_debug_schur_stats(lcba_t* h, long long* out, int max_ctas, int* nkinds,
 int lcba_debug_mma_plan(int32_t C, int32_t sm_count, int32_t* units_out, int32_t max_kinds,
                         int32_t* nslices_out, int32_t* ok_out);
 
-/* Host-only: the tile / CTA plan of the int8 tensor-core Schur kernel (schur_i8.cuh) for C cameras and P
- * points.  tiles_out: per tile 8 ints (first row group of the rows, row groups; column block 1: first row
+/* Host-only: the strip plan of the int8 tensor-core Schur kernel (schur_i8.cuh) for C cameras and P
+ * points (the plan the kernel runs may be the cover plan instead: lcba_debug_i8_cover_plan).  tiles_out: per tile 8 ints (first row group of the rows, row groups; column block 1: first row
  * group, row groups; column block 2 (the folded left-over rows, transposed): first row group, row groups;
  * first CTA, CTAs); work_out: per CTA (index, first K block, end K block).
  * Returns the number of tiles (needs no GPU). */
 int lcba_debug_i8_plan(int32_t C, int64_t P, int32_t sm_count, int32_t* tiles_out, int32_t max_tiles,
                        int32_t* work_out, int32_t max_work, int32_t* nwork_out, int32_t* nrg_out,
                        int64_t* nkb_out);
+
+/* Host-only: a tile / CTA plan of the int8 tensor-core Schur kernel with both row ranges of its A operand.
+ * which: 0 = the plan the kernel runs (the cost model's choice, without LCBA_I8_PLAN), 1 = the strip plan,
+ * 2 = the cover plan.  tiles_out: per tile 10 ints (rows: range 1 first row group, row groups, range 2 first
+ * row group, row groups; column block 1 and 2: first row group, row groups each; first CTA, CTAs); work_out:
+ * per CTA (tile, first K block, end K block); model_out: 4 doubles (executed int8 ops of one launch, slowest
+ * CTA of the cost model in cycles of the MMA warp for this plan, the strip plan and the cover plan).
+ * *cover_out: 1 when the plan is the cover plan.  Returns the number of tiles (needs no GPU). */
+int lcba_debug_i8_cover_plan(int32_t C, int64_t P, int32_t sm_count, int32_t which, int32_t* tiles_out,
+                             int32_t max_tiles, int32_t* work_out, int32_t max_work, int32_t* nwork_out,
+                             int32_t* nrg_out, int64_t* nkb_out, int32_t* cover_out, double* model_out);
 
 /* 1 when the last Schur pass of the int8 tensor-core path found a camera row whose largest |Y| entry is more
  * than 4x the square root of its Schur diagonal (finer than the 48-bit digits resolve) and recomputed the

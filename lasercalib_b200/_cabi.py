@@ -22,7 +22,7 @@ SYMBOLS = ["lcba_version", "lcba_create", "lcba_destroy", "lcba_last_error", "lc
            "lcba_time_device", "lcba_nccl_unique_id", "lcba_comm_init", "lcba_debug_tr2d",
            "lcba_sq_normal", "lcba_debug_schur_stats", "lcba_debug_mma_plan",
            "lcba_set_iteration_callback", "lcba_debug_i8_plan", "lcba_host_is_nondecreasing_i64", "lcba_debug_peer_reduce",
-           "lcba_debug_i8_fallback", "lcba_debug_chol", "lcba_debug_step"]
+           "lcba_debug_i8_fallback", "lcba_debug_chol", "lcba_debug_step", "lcba_debug_i8_cover_plan"]
 
 # scalars_out of lcba_debug_step, in order (include/lcba.h)
 STEP_SCALARS = ["reg_term", "Delta", "Jg2", "aa", "ab", "bb", "JAA", "JAB", "JBB", "gtgt", "gtp", "pp",
@@ -112,6 +112,8 @@ def load():
     lib.lcba_debug_mma_plan.argtypes = [i32, i32, vp, i32, C.POINTER(i32), C.POINTER(i32)]
     lib.lcba_debug_schur_stats.argtypes = [vp, vp, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]
     lib.lcba_debug_i8_plan.argtypes = [i32, i64, i32, vp, i32, vp, i32, C.POINTER(i32), C.POINTER(i32), C.POINTER(i64)]
+    lib.lcba_debug_i8_cover_plan.argtypes = [i32, i64, i32, i32, vp, i32, vp, i32, C.POINTER(i32), C.POINTER(i32),
+                                             C.POINTER(i64), C.POINTER(i32), vp]
     lib.lcba_host_is_nondecreasing_i64.argtypes = [vp, i64, i32]
     lib.lcba_debug_peer_reduce.argtypes = [vp, i32]
     lib.lcba_debug_i8_fallback.argtypes = [vp]
@@ -334,6 +336,29 @@ class Engine:
         """1: the last Schur pass of the int8 path was recomputed on DMMA (rows finer than its digits resolve),
         0: the int8 result stood, -1: this handle does not use the int8 path."""
         return self.lib.lcba_debug_i8_fallback(self.h)
+
+    I8_PLAN_CHOSEN, I8_PLAN_STRIP, I8_PLAN_COVER = 0, 1, 2
+
+    @staticmethod
+    def i8_plan(n_cams, P, sm_count, which=0):
+        """A tile plan of the int8 tensor-core Schur kernel (lcba_debug_i8_cover_plan, host only): dict of
+        tiles (n, 10) int32 [range 1 first row group, row groups, range 2 first row group, row groups, column
+        block 1 first row group, row groups, block 2 first row group, row groups, first CTA, CTAs], work
+        (CTAs, 3) [tile, kb0, kb1], nrg, nkb, cover (bool), executed_ops (int8 ops of one launch) and the
+        cost model's slowest CTA in MMA-warp cycles: cycles (this plan), strip_cycles, cover_cycles."""
+        lib = load()
+        tiles = np.zeros((512, 10), dtype=np.int32)
+        work = np.zeros((1024, 3), dtype=np.int32)
+        nwork, nrg, nkb, cover = C.c_int32(), C.c_int32(), C.c_int64(), C.c_int32()
+        model = np.zeros(4)
+        nt = lib.lcba_debug_i8_cover_plan(int(n_cams), int(P), int(sm_count), int(which), _ptr(tiles), tiles.shape[0],
+                                          _ptr(work), work.shape[0], C.byref(nwork), C.byref(nrg), C.byref(nkb),
+                                          C.byref(cover), _ptr(model))
+        if nt < 0:
+            raise LcbaError(nt, "lcba_debug_i8_cover_plan: bad arguments")
+        return dict(tiles=tiles[:nt].copy(), work=work[:nwork.value].copy(), nrg=nrg.value, nkb=nkb.value,
+                    cover=bool(cover.value), executed_ops=model[0], cycles=model[1], strip_cycles=model[2],
+                    cover_cycles=model[3])
 
     def debug_chol(self, A, rhs, mu=0.0, d=None, grid=0):
         """The solver's dense camera solve on a host system (lcba_debug_chol): returns (x, factor, fail)

@@ -594,7 +594,12 @@ extern "C" int lcba_set_problem_shard(lcba_t* h, int32_t C, int64_t P, int64_t N
         h->use_i8 = ie ? atoi(ie) != 0 : P >= 32768;
       }
       if (h->use_i8) {
-        h->i8plan = make_i8_plan(C, P, h->sm_count);
+        {
+          // LCBA_I8_PLAN=strip|cover overrides the cost model's choice of tile plan
+          const char* pe = getenv("LCBA_I8_PLAN");
+          const int which = !pe ? 0 : (strcmp(pe, "strip") == 0 ? 1 : (strcmp(pe, "cover") == 0 ? 2 : 0));
+          h->i8plan = make_i8_best_plan(C, P, h->sm_count, which);
+        }
         const I8Plan& ip = h->i8plan;
         h->i8_groups = (C + I8_GROUP_CAMS - 1) / I8_GROUP_CAMS;
         h->i8_gx_max = (int)std::max<long long>(1, std::min<long long>(ip.nkb, (long long)h->sm_count * 4 / h->i8_groups));   // one wave: 4 blocks per SM
@@ -984,7 +989,7 @@ static int pass_schur(lcba_t* h, const double* lam_host_or_null) {
         KL(h, "schur", k_i8_syrk<false><<<(unsigned)ip.work.size(), I8_THREADS, ip.smem_bytes, h->stream>>>(
               h->i8maps, h->d_i8planes, ip.NRG, h->d_i8work, h->d_i8partial, h->d_fail, h->d_stats));
       KL(h, "schur_reduce", k_i8_gather<<<dim3((unsigned)ip.tiles.size(), 16), 256, 0, h->stream>>>(
-            h->d_i8partial, h->d_i8tiles, C, h->d_i8erow, pl.npairs, h->d_Sred));
+            h->d_i8partial, h->d_i8tiles, C, ip.cover ? 1 : 0, h->d_i8erow, pl.npairs, h->d_Sred));
       KL(h, "schur_reduce", k_add_cam_blocks<<<nblk(C * 121, 128), 128, 0, h->stream>>>(h->d_U, C, h->d_Sred));
       // rows whose maximum comes from one point far above their Schur diagonal: the DMMA kernel (Y evaluated in
       // place) redoes this pass; both launches return at once unless k_i8_check raised the gate
@@ -1695,7 +1700,8 @@ extern "C" int lcba_debug_mma_plan(int32_t C, int32_t sm_count, int32_t* units_o
   return pl.nkinds;
 }
 
-// host-only test hook: the tile / CTA plan of the int8 tensor-core Schur kernel (schur_i8.cuh).
+// host-only test hook: the strip plan of the int8 tensor-core Schur kernel (schur_i8.cuh make_i8_plan; the
+// cover plan and the choice between the two: lcba_debug_i8_cover_plan).
 // tiles_out: per tile 8 ints (m_rg0, m_nrg, n_rg0, n_nrg, n2_rg0, n2_nrg, first CTA, CTAs); work_out: per CTA
 // 3 ints (tile, kb0, kb1).  Returns the number of tiles; *nwork_out CTAs, *nrg_out row groups, *nkb_out K blocks.
 extern "C" int lcba_debug_i8_plan(int32_t C, int64_t P, int32_t sm_count, int32_t* tiles_out, int32_t max_tiles,
@@ -1715,6 +1721,43 @@ extern "C" int lcba_debug_i8_plan(int32_t C, int64_t P, int32_t sm_count, int32_
   if (nwork_out) *nwork_out = (int32_t)pl.work.size();
   if (nrg_out) *nrg_out = pl.NRG;
   if (nkb_out) *nkb_out = pl.nkb;
+  return (int)pl.tiles.size();
+}
+
+// host-only test hook: a tile plan of the int8 tensor-core Schur kernel with both row ranges of A.
+// which: 0 = the plan k_i8_syrk runs (the cost model's choice), 1 = the strip plan, 2 = the cover plan.
+// tiles_out: per tile 10 ints (m_rg0, m_nrg, m2_rg0, m2_nrg, n_rg0, n_nrg, n2_rg0, n2_nrg, first CTA, CTAs);
+// work_out: per CTA 3 ints (tile, kb0, kb1); model_out: 4 doubles (executed int8 ops of one launch, the
+// model's slowest-CTA cycles of this plan, of the strip plan, of the cover plan).  Returns the number of
+// tiles; *nwork_out CTAs, *nrg_out row groups, *nkb_out K blocks, *cover_out 1 for a cover plan.
+extern "C" int lcba_debug_i8_cover_plan(int32_t C, int64_t P, int32_t sm_count, int32_t which, int32_t* tiles_out,
+                                        int32_t max_tiles, int32_t* work_out, int32_t max_work, int32_t* nwork_out,
+                                        int32_t* nrg_out, int64_t* nkb_out, int32_t* cover_out, double* model_out) {
+  if (C < 1 || C > LCBA_MAX_CAMERAS || P < 1 || sm_count < 1 || which < 0 || which > 2 || !tiles_out) return LCBA_E_ARG;
+  const I8Plan pl = make_i8_best_plan(C, P, sm_count, which);
+  for (size_t i = 0; i < pl.tiles.size() && (int)i < max_tiles; ++i) {
+    const I8Tile& t = pl.tiles[i];
+    int32_t* o = tiles_out + 10 * i;
+    o[0] = t.m_rg0; o[1] = t.m_nrg; o[2] = t.m2_rg0; o[3] = t.m2_nrg; o[4] = t.n_rg0; o[5] = t.n_nrg;
+    o[6] = t.n2_rg0; o[7] = t.n2_nrg; o[8] = t.w0; o[9] = t.nw;
+  }
+  if (work_out)
+    for (size_t i = 0; i < pl.work.size() && (int)i < max_work; ++i) {
+      const I8Work& w = pl.work[i];
+      int ti = 0;
+      while (ti + 1 < (int)pl.tiles.size() && pl.tiles[ti + 1].w0 <= (int)i) ++ti;
+      work_out[3 * i] = ti; work_out[3 * i + 1] = w.kb0; work_out[3 * i + 2] = w.kb1;
+    }
+  if (nwork_out) *nwork_out = (int32_t)pl.work.size();
+  if (nrg_out) *nrg_out = pl.NRG;
+  if (nkb_out) *nkb_out = pl.nkb;
+  if (cover_out) *cover_out = pl.cover ? 1 : 0;
+  if (model_out) {
+    model_out[0] = i8_executed_ops(pl);
+    model_out[1] = pl.model_cycles;
+    model_out[2] = make_i8_plan(C, P, sm_count).model_cycles;
+    model_out[3] = make_i8_cover_plan(C, P, sm_count).model_cycles;
+  }
   return (int)pl.tiles.size();
 }
 

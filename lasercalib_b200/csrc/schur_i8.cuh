@@ -15,11 +15,12 @@
 //                   [K block of 64 kappa = 21 points + 1 zero][slice][row group of 8][k-step 2][k half 2][8][16]
 //   k_i8_syrk     : one CTA = one output tile (128 rows x <= 64 columns, the 7 anti-diagonals d = i + j
 //                   side by side in TMEM) x a range of K blocks; warps 0-3 epilogue (TMEM -> FP64 registers
-//                   before an int32 can overflow), warp 4 producer (three cp.async.bulk.tensor.4d loads per
-//                   K block = 2 k-steps: all six slices of A, B1, B2; fallback: one 1-D bulk copy per lane),
-//                   warp 5 MMA issuer (elect.sync, compile-time MMA plan: slice i of the rows against slices
-//                   0..6-i of the columns in ONE instruction, N <= 256, A kept in the collector, widest last);
-//                   K ranges per tile weighted by the measured cost of a K block (make_i8_plan)
+//                   before an int32 can overflow), warp 4 producer (up to three tensor loads per K block =
+//                   2 k-steps: all six slices of A (4-D, or 5-D for two row ranges), B1, B2; fallback: one 1-D
+//                   bulk copy per lane), warp 5 MMA issuer (elect.sync, compile-time MMA plan: slice i of the
+//                   rows against slices 0..6-i of the columns in ONE instruction, N <= 256, A kept in the
+//                   collector, widest last); tiles from the strip or the cover plan, K ranges per tile weighted
+//                   by the measured cost of a K block (i8_deal)
 //   k_i8_gather   : per-CTA partials -> the pair-block layout of Sred (fixed order, no atomics)
 //   k_i8_check    : resolution guard: rows whose maximum lies far above their Schur diagonal hand the pass to
 //                   the DMMA kernel (k_schur_mma, gated) and k_i8_fallback_finish
@@ -44,50 +45,113 @@ constexpr int I8_GROUP_CAMS = 8;          // cameras per k_i8_make block: 88 row
 constexpr int I8_GROUP_RG = 13;           // row groups of the last group at most: 8 cameras + z + even padding
 constexpr int I8_GROUP_ROWS = I8_GROUP_RG * 8;
 
-// One CTA of k_i8_syrk: rows = row groups [m_rg0, m_rg0 + m_nrg) (the A operand, <= 16), columns = block 1
+// One CTA of k_i8_syrk: rows = row groups [m_rg0, m_rg0 + m_nrg) and, optionally, a second range
+// [m2_rg0, +m2_nrg) stacked below them (the A operand, <= 16 row groups in all), columns = block 1
 // [n_rg0, +n_nrg) and, optionally, block 2 [n2_rg0, +n2_nrg): the few rows left over behind the last full
-// 128-row tile, handled as COLUMNS (the tile entry is S[column][row]); n_nrg + n2_nrg <= 8.  In the partial
-// tile [128][64] block 1 occupies columns [0, 8 n_nrg), block 2 the LAST 8 n2_nrg columns.
+// 128-row tile of the strip plan, handled as COLUMNS (the tile entry is S[column][row]); n_nrg + n2_nrg <= 8.
+// In the partial tile [128][64] block 1 occupies columns [0, 8 n_nrg), block 2 the LAST 8 n2_nrg columns.
 struct I8Work {
-  int m_rg0, m_nrg, n_rg0, n_nrg, n2_rg0, n2_nrg;
+  int m_rg0, m_nrg, m2_rg0, m2_nrg, n_rg0, n_nrg, n2_rg0, n2_nrg;
   int kb0, kb1;                           // K blocks [kb0, kb1)
-  int map_a, map_b1, map_b2, pad;         // tensor-map index (box height) of the three operand loads
+  int map_a, map_b1, map_b2, pad;         // tensor-map index of the three operand loads
 };
-// TMA tensor maps over the digit planes, one per box height that the plan uses: a 4-D tensor
-// (128 u32 = one 512-byte row group, NRG row groups, 6 digits, K blocks); a box of (128, h, 6, 1) lands
-// in shared memory as [digit][h row groups][512 B] = the UMMA operand of all six digits in ONE instruction
-// (the 1-D bulk-copy version needs one copy per digit and operand: 18 per K block, and the ~110 cycles of
-// issue per copy made the copy engine, not the tensor pipe, set the pace).
-constexpr int I8_MAX_MAPS = 6;
+// TMA tensor maps over the digit planes, one per (box height, range distance) that the plan uses.
+// delta = 0: a 4-D tensor (128 u32 = one 512-byte row group, NRG row groups, 6 digits, K blocks); a box of
+// (128, h, 6, 1) lands in shared memory as [digit][h row groups][512 B] = the UMMA operand of all six digits
+// in ONE instruction (the 1-D bulk-copy version needs one copy per digit and operand: 18 per K block, and the
+// ~110 cycles of issue per copy made the copy engine, not the tensor pipe, set the pace).
+// delta > 0: the two-range A operand, a 5-D tensor (128 u32, NRG - delta row groups, 2 ranges delta row
+// groups apart, 6 digits, K blocks); a box of (128, h, 2, 6, 1) lands as [digit][2 h row groups][512 B], the same
+// layout as one range of 2 h row groups.
+constexpr int I8_MAX_MAPS = 16;
 struct alignas(64) I8Maps { CUtensorMap m[I8_MAX_MAPS]; };
-struct I8Tile { int m_rg0, m_nrg, n_rg0, n_nrg, n2_rg0, n2_nrg, w0, nw; };
+struct I8Tile { int m_rg0, m_nrg, m2_rg0, m2_nrg, n_rg0, n_nrg, n2_rg0, n2_nrg, w0, nw; };
 
 struct I8Plan {
   int C = 0, R = 0, NRG = 0;
   long long nkb = 0;
-  int map_heights[I8_MAX_MAPS] = {0, 0, 0, 0, 0, 0};   // box heights (row groups) of the tensor maps
+  int map_heights[I8_MAX_MAPS] = {};                   // box heights (row groups per range) of the tensor maps
+  int map_delta[I8_MAX_MAPS] = {};                     // 0: one range; > 0: two ranges this many row groups apart
   int nmaps = 0;                                       // > I8_MAX_MAPS: too many shapes, use 1-D bulk copies
+  bool cover = false;                                  // made by make_i8_cover_plan
+  double model_cycles = 0.0;                           // slowest CTA in the cost model (MMA-warp cycles)
   std::vector<I8Tile> tiles;
   std::vector<I8Work> work;
   size_t plane_bytes = 0, smem_bytes = 0;
 };
 
-// Tiles.  Row tiles of 16 row groups (128 rows).  When the last row tile would hold <= 4 row groups
-// (24 cameras: 34 = 16 + 16 + 2) those rows are not given a 128-row tile of their own: they ride as column
-// block 2 of ONE tile of every full row tile (the operand rows A are the same, only 1-2 KB of extra B per K
-// block are loaded) plus a small corner tile; the column tiles are then 8 - last row groups wide so that
-// block 1 + block 2 <= 64 columns (7 anti-diagonals x 64 = 448 TMEM columns).  (First version: separate
-// 16-column tiles with their own K ranges streamed K positions nobody else was reading: 40 % of the
-// kernel's DRAM traffic for 11 % of its work, ncu r02.)
-// K ranges: every non-corner tile gets the SAME number of ranges, so that all CTAs of a K range walk the
-// same K blocks at the same time and share their operands in L2.
-inline I8Plan make_i8_plan(int C, long long P, int sm_count) {
+// Cost of one K block of a tile, in cycles of the MMA warp (measured per tile kind with LCBA_SCHUR_STATS=1,
+// tools/i8_stats.py, ring24 x 1 M): a fixed part (stage hand-over, waiting for operands) + one part per column
+// block that grows with its width -- narrow instructions are far from free: a 16-column block costs half a
+// 48-column one.  The row ranges of A do not enter: M is 128 in every instruction.
+inline double i8_block_cost(int nrg) {
+  return nrg <= 0 ? 0.0 : (nrg <= 2 ? 592.0 : (nrg <= 4 ? 812.0 : (nrg <= 6 ? 1181.0 : 1550.0)));
+}
+inline double i8_tile_cost(const I8Tile& t) { return 507.0 + i8_block_cost(t.n_nrg) + i8_block_cost(t.n2_nrg); }
+
+// K ranges per tile: one CTA per SM in total, dealt so that the slowest tile finishes as early as possible
+// (greedy over the cost model; the first version gave every main tile the same number of ranges: the tile that
+// carries a second column block was 13 % slower than the rest and set the kernel's time).  Fills pl.work, the
+// tensor-map shapes, the buffer sizes and the model's slowest-CTA cycles.
+inline void i8_deal(I8Plan& pl, int sm_count) {
+  std::vector<double> cost(pl.tiles.size());
+  std::vector<long long> nr(pl.tiles.size(), 1);
+  for (size_t ti = 0; ti < pl.tiles.size(); ++ti) cost[ti] = i8_tile_cost(pl.tiles[ti]);
+  for (long long left = (long long)sm_count - (long long)pl.tiles.size(); left > 0; --left) {
+    size_t worst = 0;
+    double tw = -1.0;
+    for (size_t ti = 0; ti < pl.tiles.size(); ++ti) {
+      const double tt = nr[ti] < pl.nkb ? cost[ti] / (double)nr[ti] : -1.0;
+      if (tt > tw) { tw = tt; worst = ti; }
+    }
+    if (tw < 0.0) break;                                    // every tile already has one CTA per K block
+    ++nr[worst];
+  }
+  pl.model_cycles = 0.0;
+  for (size_t ti = 0; ti < pl.tiles.size(); ++ti) {
+    I8Tile& t = pl.tiles[ti];
+    const long long n = std::min<long long>(nr[ti], pl.nkb);
+    t.w0 = (int)pl.work.size();
+    t.nw = (int)n;
+    auto map_of = [&](int h, int delta) {
+      if (h == 0) return 0;
+      for (int i = 0; i < pl.nmaps && i < I8_MAX_MAPS; ++i)
+        if (pl.map_heights[i] == h && pl.map_delta[i] == delta) return i;
+      if (pl.nmaps < I8_MAX_MAPS) { pl.map_heights[pl.nmaps] = h; pl.map_delta[pl.nmaps] = delta; }
+      return pl.nmaps++;
+    };
+    const int ma = map_of(t.m_nrg, t.m2_nrg > 0 ? t.m2_rg0 - t.m_rg0 : 0), mb1 = map_of(t.n_nrg, 0), mb2 = map_of(t.n2_nrg, 0);
+    for (long long q = 0; q < n; ++q) {
+      I8Work w{t.m_rg0, t.m_nrg, t.m2_rg0, t.m2_nrg, t.n_rg0, t.n_nrg, t.n2_rg0, t.n2_nrg,
+               (int)(pl.nkb * q / n), (int)(pl.nkb * (q + 1) / n), ma, mb1, mb2, 0};
+      pl.work.push_back(w);
+    }
+    pl.model_cycles = std::max(pl.model_cycles, cost[ti] * (double)((pl.nkb + n - 1) / n));
+  }
+  pl.plane_bytes = (size_t)pl.nkb * I8_NS * pl.NRG * I8_RG_BYTES;
+  pl.smem_bytes = (size_t)I8_STAGES * I8_NS * (16 + 8) * I8_RG_BYTES + 1024;
+}
+
+inline I8Plan i8_plan_base(int C, long long P) {
   I8Plan pl;
   pl.C = C;
   pl.R = NCP * C + 1;
   pl.NRG = (pl.R + 7) / 8;
   pl.NRG += pl.NRG & 1;                                   // MMA N is a multiple of 16
   pl.nkb = (P + I8_PTS - 1) / I8_PTS;
+  return pl;
+}
+
+// The strip plan.  Row tiles of 16 row groups (128 rows), each with its column tiles up to and including the
+// diagonal block, which is computed as a square (k_i8_gather drops its upper half).  When the last row tile
+// would hold <= 4 row groups (24 cameras: 34 = 16 + 16 + 2) those rows are not given a 128-row tile of their
+// own: they ride as column block 2 of ONE tile of every full row tile (the operand rows A are the same, only
+// 1-2 KB of extra B per K block are loaded) plus a small corner tile; the column tiles are then
+// 8 - last row groups wide so that block 1 + block 2 <= 64 columns (7 anti-diagonals x 64 = 448 TMEM columns).
+// (First version: separate 16-column tiles with their own K ranges streamed K positions nobody else was
+// reading: 40 % of the kernel's DRAM traffic for 11 % of its work, ncu r02.)
+inline I8Plan make_i8_plan(int C, long long P, int sm_count) {
+  I8Plan pl = i8_plan_base(C, P);
   const int NRG = pl.NRG;
   const int nmt = (NRG + 15) / 16;
   const int last_m = NRG - 16 * (nmt - 1);
@@ -100,55 +164,83 @@ inline I8Plan make_i8_plan(int C, long long P, int sm_count) {
     for (int n0 = 0; n0 < m0 + mn; n0 += col_w) {
       const int nn = std::min(col_w, m0 + mn - n0);
       const bool last = n0 + col_w >= m0 + mn;
-      I8Tile t{m0, mn, n0, nn, fold && last ? c0 : 0, fold && last ? last_m : 0, 0, 0};
+      I8Tile t{m0, mn, 0, 0, n0, nn, fold && last ? c0 : 0, fold && last ? last_m : 0, 0, 0};
       pl.tiles.push_back(t);
     }
   }
   if (fold) {
-    I8Tile t{c0, last_m, c0, last_m, 0, 0, 0, 0};         // the corner: left-over rows x left-over rows
+    I8Tile t{c0, last_m, 0, 0, c0, last_m, 0, 0, 0, 0};  // the corner: left-over rows x left-over rows
     pl.tiles.push_back(t);
   }
-  // K ranges per tile: one CTA per SM in total, dealt so that the slowest tile finishes as early as possible.
-  // Cost of one K block of a tile, in cycles of the MMA warp (measured per tile kind with LCBA_SCHUR_STATS=1,
-  // tools/i8_stats.py, ring24 x 1 M): a fixed part (stage hand-over, waiting for operands) + one part per column
-  // block that grows with its width -- narrow instructions are far from free: a 16-column block costs half a
-  // 48-column one.  (The first version gave every main tile the same number of ranges: the tile that carries a
-  // second column block was 13 % slower than the rest and set the kernel's time.)
-  auto block_cost = [](int nrg) { return nrg <= 0 ? 0.0 : (nrg <= 2 ? 592.0 : (nrg <= 4 ? 812.0 : (nrg <= 6 ? 1181.0 : 1550.0))); };
-  std::vector<double> cost(pl.tiles.size());
-  std::vector<long long> nr(pl.tiles.size(), 1);
-  for (size_t ti = 0; ti < pl.tiles.size(); ++ti) cost[ti] = 507.0 + block_cost(pl.tiles[ti].n_nrg) + block_cost(pl.tiles[ti].n2_nrg);
-  for (long long left = (long long)sm_count - (long long)pl.tiles.size(); left > 0; --left) {
-    size_t worst = 0;
-    double tw = -1.0;
-    for (size_t ti = 0; ti < pl.tiles.size(); ++ti) {
-      const double tt = nr[ti] < pl.nkb ? cost[ti] / (double)nr[ti] : -1.0;
-      if (tt > tw) { tw = tt; worst = ti; }
-    }
-    if (tw < 0.0) break;                                    // every tile already has one CTA per K block
-    ++nr[worst];
-  }
-  for (size_t ti = 0; ti < pl.tiles.size(); ++ti) {
-    I8Tile& t = pl.tiles[ti];
-    const long long n = std::min<long long>(nr[ti], pl.nkb);
-    t.w0 = (int)pl.work.size();
-    t.nw = (int)n;
-    auto map_of = [&](int h) {
-      if (h == 0) return 0;
-      for (int i = 0; i < pl.nmaps && i < I8_MAX_MAPS; ++i) if (pl.map_heights[i] == h) return i;
-      if (pl.nmaps < I8_MAX_MAPS) pl.map_heights[pl.nmaps] = h;
-      return pl.nmaps++;
-    };
-    const int ma = map_of(t.m_nrg), mb1 = map_of(t.n_nrg), mb2 = map_of(t.n2_nrg);
-    for (long long q = 0; q < n; ++q) {
-      I8Work w{t.m_rg0, t.m_nrg, t.n_rg0, t.n_nrg, t.n2_rg0, t.n2_nrg, (int)(pl.nkb * q / n), (int)(pl.nkb * (q + 1) / n),
-               ma, mb1, mb2, 0};
-      pl.work.push_back(w);
-    }
-  }
-  pl.plane_bytes = (size_t)pl.nkb * I8_NS * NRG * I8_RG_BYTES;
-  pl.smem_bytes = (size_t)I8_STAGES * I8_NS * (16 + 8) * I8_RG_BYTES + 1024;
+  i8_deal(pl, sm_count);
   return pl;
+}
+
+// The cover plan: only full 128 x 64 tiles where the strip plan computes square diagonal blocks and folds.
+// The row groups form G groups of 8 (g = row groups [8g, 8g + 8)) and a ragged rest E of NRG - 8G < 8 row
+// groups.  A tile (I, J) has the column group J (<= 8 row groups) and up to two row groups I (the two
+// ranges of A, 8 row groups each); S is symmetric, so a tile serves either orientation:
+//   - I = {x, z}, J = z: the triangle of z and the block x-z;  I = {x, y}, J = z: the blocks x-z and y-z.
+// Give every cross pair {x, z} of groups a column group (an orientation) so that each group z has an odd
+// number of pairs pointing to it: its own triangle and those pairs then fill whole tiles.  Start from
+// "pair {a, b}, a < b, points to b" (indegree of z = z) and flip the pair between two groups of the wrong
+// parity; at most one group stays even when G (G - 1) / 2 and G differ in parity.  E stays a column block
+// (<= 48 columns): its triangle rides with the last group (one contiguous range), the other groups go two at a
+// time.  k_i8_gather keeps each entry once: inside I and J both (the square of z) only rho >= sig.
+// 24 cameras (NRG = 34, G = 4): 8 tiles, 13 582 model cycles per K block against 16 517 for the strip plan.
+inline I8Plan make_i8_cover_plan(int C, long long P, int sm_count) {
+  I8Plan pl = i8_plan_base(C, P);
+  pl.cover = true;
+  const int G = pl.NRG / 8, r = pl.NRG - 8 * G;
+  std::vector<std::vector<int>> to(G);                  // to[z]: the groups x whose pair {x, z} has columns z
+  for (int b = 0; b < G; ++b)
+    for (int a = 0; a < b; ++a) to[b].push_back(a);
+  std::vector<int> even;
+  for (int z = 0; z < G; ++z) if (to[z].size() % 2 == 0) even.push_back(z);
+  for (size_t k = 0; k + 1 < even.size(); k += 2) {     // flip {u, v}, u < v: it pointed to v, now to u
+    const int u = even[k], v = even[k + 1];
+    to[v].erase(std::find(to[v].begin(), to[v].end(), u));
+    to[u].push_back(v);
+  }
+  auto tile = [&](int x, int y, int j0, int jn) {       // rows: group x (and group y >= 0), columns [j0, j0 + jn)
+    int a = std::min(x, y < 0 ? x : y), b = std::max(x, y);
+    I8Tile t{8 * a, 8, 0, 0, j0, jn, 0, 0, 0, 0};
+    if (y >= 0 && b == a + 1) t.m_nrg = 16;             // adjacent groups: one range of 16
+    else if (y >= 0) { t.m2_rg0 = 8 * b; t.m2_nrg = 8; }
+    pl.tiles.push_back(t);
+  };
+  for (int z = 0; z < G; ++z) {
+    std::vector<int> items(1, z);                       // z's own triangle, then the pairs pointing to z
+    items.insert(items.end(), to[z].begin(), to[z].end());
+    std::sort(items.begin() + 1, items.end());
+    for (size_t k = 0; k < items.size(); k += 2) tile(items[k], k + 1 < items.size() ? items[k + 1] : -1, 8 * z, 8);
+  }
+  if (r > 0) {
+    // E's triangle with the last group: rows [8 (G - 1), NRG) in one range
+    if (G > 0) pl.tiles.push_back(I8Tile{8 * (G - 1), 8 + r, 0, 0, 8 * G, r, 0, 0, 0, 0});
+    else pl.tiles.push_back(I8Tile{0, r, 0, 0, 0, r, 0, 0, 0, 0});
+    for (int x = 0; x + 1 < G; x += 2) tile(x, x + 2 < G ? x + 1 : -1, 8 * G, r);
+  }
+  i8_deal(pl, sm_count);
+  return pl;
+}
+
+// The plan k_i8_syrk runs: the cover plan where the cost model puts its slowest CTA below the strip plan's.
+// which: 0 = by the model, 1 = strip, 2 = cover (LCBA_I8_PLAN).
+inline I8Plan make_i8_best_plan(int C, long long P, int sm_count, int which) {
+  if (which == 1) return make_i8_plan(C, P, sm_count);
+  I8Plan cv = make_i8_cover_plan(C, P, sm_count);
+  if (which == 2) return cv;
+  I8Plan st = make_i8_plan(C, P, sm_count);
+  return cv.model_cycles < st.model_cycles ? cv : st;
+}
+
+// int8 ops (1 MAC = 2) one k_i8_syrk launch of a plan issues: 26 digit products of 128 rows x the plan's
+// columns x 64 kappa per K block.
+inline double i8_executed_ops(const I8Plan& pl) {
+  long long cols = 0;
+  for (const I8Tile& t : pl.tiles) cols += 8 * (t.n_nrg + t.n2_nrg);
+  return 26.0 * 2.0 * 128.0 * (double)cols * 64.0 * (double)pl.nkb;
 }
 
 // Encode the tensor maps of a plan over `planes` (host).  Returns false when the driver entry point is
@@ -165,15 +257,28 @@ inline bool i8_encode_maps(const I8Plan& pl, void* planes, I8Maps* out) {
     cudaGetLastError();
     return false;
   }
-  const cuuint64_t gdim[4] = {128, (cuuint64_t)pl.NRG, (cuuint64_t)I8_NS, (cuuint64_t)pl.nkb};
-  const cuuint64_t gstr[3] = {(cuuint64_t)I8_RG_BYTES, (cuuint64_t)pl.NRG * I8_RG_BYTES, (cuuint64_t)I8_NS * pl.NRG * I8_RG_BYTES};
-  const cuuint32_t estr[4] = {1, 1, 1, 1};
+  const cuuint64_t rg = I8_RG_BYTES, slice = (cuuint64_t)pl.NRG * I8_RG_BYTES, blk = (cuuint64_t)I8_NS * slice;
+  const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
   memset(out, 0, sizeof(*out));
   for (int i = 0; i < pl.nmaps; ++i) {
-    const cuuint32_t box[4] = {128, (cuuint32_t)pl.map_heights[i], (cuuint32_t)I8_NS, 1};
-    const CUresult r = ((EncodeFn)fn)(&out->m[i], CU_TENSOR_MAP_DATA_TYPE_UINT32, 4, planes, gdim, gstr, box, estr,
-                                      CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                                      CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    const cuuint32_t h = (cuuint32_t)pl.map_heights[i];
+    CUresult r;
+    if (pl.map_delta[i] == 0) {
+      const cuuint64_t gdim[4] = {128, (cuuint64_t)pl.NRG, (cuuint64_t)I8_NS, (cuuint64_t)pl.nkb};
+      const cuuint64_t gstr[3] = {rg, slice, blk};
+      const cuuint32_t box[4] = {128, h, (cuuint32_t)I8_NS, 1};
+      r = ((EncodeFn)fn)(&out->m[i], CU_TENSOR_MAP_DATA_TYPE_UINT32, 4, planes, gdim, gstr, box, estr,
+                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
+                         CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    } else {
+      // the row-group extent ends delta before NRG, so that the second range of any box stays inside the slice
+      const cuuint64_t gdim[5] = {128, (cuuint64_t)(pl.NRG - pl.map_delta[i]), 2, (cuuint64_t)I8_NS, (cuuint64_t)pl.nkb};
+      const cuuint64_t gstr[4] = {rg, (cuuint64_t)pl.map_delta[i] * rg, slice, blk};
+      const cuuint32_t box[5] = {128, h, 2, (cuuint32_t)I8_NS, 1};
+      r = ((EncodeFn)fn)(&out->m[i], CU_TENSOR_MAP_DATA_TYPE_UINT32, 5, planes, gdim, gstr, box, estr,
+                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
+                         CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    }
     if (r != CUDA_SUCCESS) return false;
   }
   return true;
@@ -183,6 +288,10 @@ inline bool i8_encode_maps(const I8Plan& pl, void* planes, I8Maps* out) {
 __device__ __forceinline__ void i8_tma_4d(uint32_t dst, const CUtensorMap* map, int c0, int c1, int c2, int c3, uint32_t bar) {
   asm volatile("cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5}], [%6];"
                ::"r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(bar) : "memory");
+}
+__device__ __forceinline__ void i8_tma_5d(uint32_t dst, const CUtensorMap* map, int c0, int c1, int c2, int c3, int c4, uint32_t bar) {
+  asm volatile("cp.async.bulk.tensor.5d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5, %6}], [%7];"
+               ::"r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4), "r"(bar) : "memory");
 }
 __device__ __forceinline__ uint32_t i8_smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void i8_mbar_init(uint32_t bar, uint32_t count) {
@@ -624,7 +733,8 @@ k_i8_syrk(const __grid_constant__ I8Maps maps, const unsigned char* __restrict__
   __shared__ uint32_t s_tmem;
   const I8Work W = work[blockIdx.x];
   const int tid = threadIdx.x, wid = tid >> 5, lane = tid & 31;
-  const uint32_t a_bytes = (uint32_t)W.m_nrg * I8_RG_BYTES, b_bytes = (uint32_t)W.n_nrg * I8_RG_BYTES;   // per slice
+  const uint32_t a1_bytes = (uint32_t)W.m_nrg * I8_RG_BYTES, a_bytes = a1_bytes + (uint32_t)W.m2_nrg * I8_RG_BYTES;
+  const uint32_t b_bytes = (uint32_t)W.n_nrg * I8_RG_BYTES;   // per slice
   const uint32_t b2_bytes = (uint32_t)W.n2_nrg * I8_RG_BYTES;
   const uint32_t B2_OFF = (uint32_t)I8_NS * b_bytes;          // block 2's B region follows block 1's
   constexpr uint32_t A_REGION = (uint32_t)I8_NS * 16 * I8_RG_BYTES;
@@ -659,15 +769,16 @@ k_i8_syrk(const __grid_constant__ I8Maps maps, const unsigned char* __restrict__
           i8_mbar_expect_tx(bar_full + 8 * st, (uint32_t)I8_NS * (a_bytes + b_bytes + b2_bytes));
           const uint32_t dstA = smem0 + st * STAGE_BYTES, dstB = dstA + A_REGION;
           const int kb = W.kb0 + it;
-          i8_tma_4d(dstA, &maps.m[W.map_a], 0, W.m_rg0, 0, kb, bar_full + 8 * st);
+          if (W.m2_nrg > 0) i8_tma_5d(dstA, &maps.m[W.map_a], 0, W.m_rg0, 0, 0, kb, bar_full + 8 * st);
+          else i8_tma_4d(dstA, &maps.m[W.map_a], 0, W.m_rg0, 0, kb, bar_full + 8 * st);
           i8_tma_4d(dstB, &maps.m[W.map_b1], 0, W.n_rg0, 0, kb, bar_full + 8 * st);
           if (W.n2_nrg > 0) i8_tma_4d(dstB + B2_OFF, &maps.m[W.map_b2], 0, W.n2_rg0, 0, kb, bar_full + 8 * st);
         }
       }
     } else {
-    // ---- producer, 1-D bulk copies: one per lane: (digit, operand) = A, B of block 1, B of block 2
-    const int ci = lane / 3, cb = lane - 3 * ci;
-    const bool mine = lane < 3 * I8_NS && (cb < 2 || W.n2_nrg > 0);
+    // ---- producer, 1-D bulk copies: one per lane: (digit, operand) = A range 1, A range 2, B of block 1, B of block 2
+    const int ci = lane / 4, cb = lane - 4 * ci;
+    const bool mine = lane < 4 * I8_NS && (cb == 0 || cb == 2 || (cb == 1 && W.m2_nrg > 0) || (cb == 3 && W.n2_nrg > 0));
     for (int it = 0; it < nkb; ++it) {
       const int st = it % I8_STAGES;
       if (it >= I8_STAGES) i8_mbar_wait<false>(bar_empty + 8 * st, ((it / I8_STAGES) - 1) & 1, fail);
@@ -676,8 +787,9 @@ k_i8_syrk(const __grid_constant__ I8Maps maps, const unsigned char* __restrict__
       if (mine) {
         const unsigned char* src = planes + (size_t)(W.kb0 + it) * I8_NS * NRG * I8_RG_BYTES + (size_t)ci * NRG * I8_RG_BYTES;
         const uint32_t dstA = smem0 + st * STAGE_BYTES, dstB = dstA + A_REGION;
-        if (cb == 0) i8_bulk_g2s(dstA + ci * a_bytes, src + (size_t)W.m_rg0 * I8_RG_BYTES, a_bytes, bar_full + 8 * st);
-        else if (cb == 1) i8_bulk_g2s(dstB + ci * b_bytes, src + (size_t)W.n_rg0 * I8_RG_BYTES, b_bytes, bar_full + 8 * st);
+        if (cb == 0) i8_bulk_g2s(dstA + ci * a_bytes, src + (size_t)W.m_rg0 * I8_RG_BYTES, a1_bytes, bar_full + 8 * st);
+        else if (cb == 1) i8_bulk_g2s(dstA + ci * a_bytes + a1_bytes, src + (size_t)W.m2_rg0 * I8_RG_BYTES, a_bytes - a1_bytes, bar_full + 8 * st);
+        else if (cb == 2) i8_bulk_g2s(dstB + ci * b_bytes, src + (size_t)W.n_rg0 * I8_RG_BYTES, b_bytes, bar_full + 8 * st);
         else i8_bulk_g2s(dstB + B2_OFF + ci * b2_bytes, src + (size_t)W.n2_rg0 * I8_RG_BYTES, b2_bytes, bar_full + 8 * st);
       }
     }
@@ -775,20 +887,30 @@ k_i8_syrk(const __grid_constant__ I8Maps maps, const unsigned char* __restrict__
 // gridDim.x = tiles, gridDim.y splits a tile's entries: sum the partials of its CTAs (fixed order), apply the row
 // exponents and write - Y Y^T into the pair-block layout of the slice partials (same convention as
 // mma_consume: lower pair blocks 11 x 11, same-camera blocks with both triangles, the z row = reduced
-// right-hand side).  Tile columns [0, 8 n_nrg) = block 1, the last 8 n2_nrg columns = block 2 (transposed).
+// right-hand side).  Tile rows [0, 8 m_nrg) = range 1, the rest = range 2; tile columns [0, 8 n_nrg) = block 1,
+// the last 8 n2_nrg columns = block 2.  An entry above the diagonal (rho < sig) stands for its transpose, except
+// where that transpose is computed elsewhere: strip plan (cover = 0): the column is one of the tile's rows (the
+// diagonal block's upper half; the rest of the row tile holds the transposes); cover plan: the entry lies in the
+// square of the tile's rows and columns.  Every entry of the lower triangle is then taken exactly once.
 __global__ void __launch_bounds__(256)
-k_i8_gather(const double* __restrict__ partial, const I8Tile* __restrict__ tiles, int C,
+k_i8_gather(const double* __restrict__ partial, const I8Tile* __restrict__ tiles, int C, int cover,
             const int* __restrict__ e_row, int npairs, double* __restrict__ Sred) {
   const I8Tile T = tiles[blockIdx.x];
   const int n = NCP * C;
-  const int nr = T.m_nrg * 8, nc1 = T.n_nrg * 8, nc2 = T.n2_nrg * 8, nc = nc1 + nc2;
+  const int nr1 = T.m_nrg * 8, nr = nr1 + T.m2_nrg * 8, nc1 = T.n_nrg * 8, nc2 = T.n2_nrg * 8, nc = nc1 + nc2;
   for (int idx = threadIdx.x + blockDim.x * blockIdx.y; idx < nr * nc; idx += blockDim.x * gridDim.y) {
     const int tr = idx / nc, tcl = idx - tr * nc;
     const bool second = tcl >= nc1;
     const int tc = second ? 64 - nc2 + (tcl - nc1) : tcl;               // column inside the 64-wide partial tile
-    int rho = T.m_rg0 * 8 + tr, sig = second ? T.n2_rg0 * 8 + (tcl - nc1) : T.n_rg0 * 8 + tcl;
-    if (second) { const int x = rho; rho = sig; sig = x; }
-    if (rho > n || sig >= n || sig > rho) continue;
+    int rho = tr < nr1 ? T.m_rg0 * 8 + tr : T.m2_rg0 * 8 + (tr - nr1);
+    int sig = second ? T.n2_rg0 * 8 + (tcl - nc1) : T.n_rg0 * 8 + tcl;
+    if (rho < sig) {
+      const int g = sig >> 3, gr = rho >> 3;
+      const bool col_in_rows = (g >= T.m_rg0 && g < T.m_rg0 + T.m_nrg) || (g >= T.m2_rg0 && g < T.m2_rg0 + T.m2_nrg);
+      if (col_in_rows && (!cover || (gr >= T.n_rg0 && gr < T.n_rg0 + T.n_nrg))) continue;
+      const int x = rho; rho = sig; sig = x;
+    }
+    if (rho > n || sig >= n) continue;
     double s = 0.0;
     for (int w = 0; w < T.nw; ++w) s += partial[((size_t)(T.w0 + w) * 128 + tr) * 64 + tc];
     const double v = -ldexp(s, e_row[rho] + e_row[sig]);

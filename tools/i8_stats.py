@@ -1,5 +1,5 @@
 """Per-CTA cycle counters of k_i8_syrk (LCBA_SCHUR_STATS=1): which tile kinds set the kernel's time.
-Usage: python tools/i8_stats.py [rig] [points]"""
+Usage: [LCBA_I8_PLAN=strip|cover] python tools/i8_stats.py [rig] [points]"""
 import ctypes as C, os, sys
 os.environ["LCBA_SCHUR_STATS"] = "1"
 os.environ.setdefault("LCBA_SCHUR_I8", "1")
@@ -17,15 +17,14 @@ nk, ns = C.c_int(), C.c_int()
 eng.lib.lcba_debug_schur_stats.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]
 rc = eng.lib.lcba_debug_schur_stats(eng.h, buf.ctypes.data_as(C.c_void_p), 1024, C.byref(nk), C.byref(ns))
 assert rc == 0, rc
-tiles = np.zeros((256, 8), dtype=np.int32); work = np.zeros((512, 3), dtype=np.int32)
-nwork, nrg, nkb = C.c_int32(), C.c_int32(), C.c_int64()
-nt = eng.lib.lcba_debug_i8_plan(pb["n_cams"], pb["n_points"], 148, tiles.ctypes.data_as(C.c_void_p), 256,
-                                work.ctypes.data_as(C.c_void_p), 512, C.byref(nwork), C.byref(nrg), C.byref(nkb))
-print("tiles %d, CTAs %d, K blocks %d" % (nt, nwork.value, nkb.value))
-for t in tiles[:nt]:
-    m0, mn, n0, nn, n20, n2n, w0, nw = t
+import torch
+sms = torch.cuda.get_device_properties(0).multi_processor_count
+plan = os.environ.get("LCBA_I8_PLAN")
+pl = Engine.i8_plan(pb["n_cams"], pb["n_points"], sms, {"strip": 1, "cover": 2}.get(plan, 0))
+print("%s plan: tiles %d, CTAs %d, K blocks %d" % ("cover" if pl["cover"] else "strip", len(pl["tiles"]), len(pl["work"]), pl["nkb"]))
+for m0, mn, m20, m2n, n0, nn, n20, n2n, w0, nw in pl["tiles"]:
     st = buf[w0:w0 + nw].astype(float)
-    kb = (work[w0:w0 + nw, 2] - work[w0:w0 + nw, 1]).astype(float)
-    print("tile rows rg %2d+%2d cols %2d+%d (+%d): %2d CTAs x %5.0f K blocks: MMA warp %.2f Mcyc (max %.2f) = %4.0f cyc / K block, waiting at FULL %4.1f %%"
-          % (m0, mn, n0, nn, n2n, nw, kb.mean(), st[:, 1].mean() / 1e6, st[:, 1].max() / 1e6, (st[:, 1] / kb).mean(),
+    kb = (pl["work"][w0:w0 + nw, 2] - pl["work"][w0:w0 + nw, 1]).astype(float)
+    print("tile rows rg %2d+%2d (+%2d+%d) cols %2d+%d (+%d): %2d CTAs x %5.0f K blocks: MMA warp %.2f Mcyc (max %.2f) = %4.0f cyc / K block, waiting at FULL %4.1f %%"
+          % (m0, mn, m20, m2n, n0, nn, n2n, nw, kb.mean(), st[:, 1].mean() / 1e6, st[:, 1].max() / 1e6, (st[:, 1] / kb).mean(),
              100 * st[:, 0].sum() / st[:, 1].sum()))
