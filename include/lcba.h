@@ -259,6 +259,16 @@ int lcba_debug_chol(lcba_t* h, int32_t n, const double* A, const double* rhs, do
 int lcba_debug_step(lcba_t* h, double lam, double mu, int32_t mode, double* pc_out, double* pp_out,
                     double* scalars_out);
 
+/* The digit planes of the int8 tensor-core Schur path on the resident problem at its current x: linearise,
+ * point factors damped with `lam`, row maxima and exponents, then `reps` launches of the plane kernel,
+ * k_i8_make (ref = 0) or the reference k_i8_make_ref (ref = 1).  poison 0..255: the plane buffer is filled
+ * with that byte before the launches (outside the timed window), so that bytes the kernel leaves unwritten
+ * show; -1: it is left as it is.  ms_out: CUDA-event time per launch of the plane kernel.  planes_out (may be
+ * NULL): the planes after the last launch, planes_bytes bytes, which must equal the plane buffer's size
+ * (K blocks x 6 digits x row groups x 512).  LCBA_E_STATE when the problem does not take the int8 path.  Synchronises the handle's stream; not part of lcba_solve. */
+int lcba_debug_i8_make(lcba_t* h, double lam, int32_t ref, int32_t reps, int32_t poison, double* ms_out,
+                       void* planes_out, int64_t planes_bytes);
+
 /* ---- profiling hook --------------------------------------------------------------------
  * Per-CTA cycle counters of the last Schur launch (4 int64 per CTA, [kind][slice]); only
  * filled when the process runs with LCBA_SCHUR_STATS=1 (tools/schur_stats.py). */

@@ -22,7 +22,8 @@ SYMBOLS = ["lcba_version", "lcba_create", "lcba_destroy", "lcba_last_error", "lc
            "lcba_time_device", "lcba_nccl_unique_id", "lcba_comm_init", "lcba_debug_tr2d",
            "lcba_sq_normal", "lcba_debug_schur_stats", "lcba_debug_mma_plan",
            "lcba_set_iteration_callback", "lcba_debug_i8_plan", "lcba_host_is_nondecreasing_i64", "lcba_debug_peer_reduce",
-           "lcba_debug_i8_fallback", "lcba_debug_chol", "lcba_debug_step", "lcba_debug_i8_cover_plan"]
+           "lcba_debug_i8_fallback", "lcba_debug_chol", "lcba_debug_step", "lcba_debug_i8_cover_plan",
+           "lcba_debug_i8_make"]
 
 # scalars_out of lcba_debug_step, in order (include/lcba.h)
 STEP_SCALARS = ["reg_term", "Delta", "Jg2", "aa", "ab", "bb", "JAA", "JAB", "JBB", "gtgt", "gtp", "pp",
@@ -120,8 +121,17 @@ def load():
     lib.lcba_debug_tr2d.argtypes = [dbl, dbl, dbl, dbl, dbl, dbl, pd, C.POINTER(C.c_int)]
     lib.lcba_debug_chol.argtypes = [vp, i32, vp, vp, dbl, vp, i32, vp, vp, C.POINTER(i32)]
     lib.lcba_debug_step.argtypes = [vp, dbl, dbl, i32, vp, vp, vp]
+    lib.lcba_debug_i8_make.argtypes = [vp, dbl, i32, i32, i32, pd, vp, i64]
     _lib = lib
     return lib
+
+
+def i8_plane_bytes(n_cams, n_points):
+    """Bytes of the int8 path's digit planes (schur_i8.cuh): K blocks of 21 points x 6 digits x row groups of 8
+    of the 11 C + 1 rows, rounded up to an even count, x 512."""
+    nrg = (11 * n_cams + 1 + 7) // 8
+    nrg += nrg & 1
+    return -(-n_points // 21) * 6 * nrg * 512
 
 
 def _ptr(a):
@@ -388,6 +398,20 @@ class Engine:
         sc = np.empty(len(STEP_SCALARS))
         self._check(self.lib.lcba_debug_step(self.h, float(lam), float(mu), int(mode), _ptr(pc), _ptr(pp), _ptr(sc)))
         return pc, pp, dict(zip(STEP_SCALARS, sc.tolist()))
+
+    def debug_i8_make(self, lam, ref=False, reps=1, planes=True, poison=0xA5):
+        """The digit planes of the int8 Schur path at the current x, damped with lam (lcba_debug_i8_make):
+        (ms per launch of k_i8_make, or of the reference k_i8_make_ref with ref=True, planes as a uint8 array or
+        None).  The plane buffer is filled with the byte `poison` first (None: left as it is).  The problem must
+        take the int8 path (LCBA_SCHUR_I8=1 when it is set, below 32 768 points)."""
+        ms = C.c_double()
+        buf, nbytes = None, 0
+        if planes:
+            nbytes = i8_plane_bytes(self.C, self.P)
+            buf = np.empty(nbytes, dtype=np.uint8)
+        self._check(self.lib.lcba_debug_i8_make(self.h, float(lam), int(bool(ref)), int(reps),
+                                                -1 if poison is None else int(poison), C.byref(ms), _ptr(buf), nbytes))
+        return ms.value, buf
 
     def time_device(self, what, reps=10):
         ms = C.c_double()

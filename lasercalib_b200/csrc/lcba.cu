@@ -128,7 +128,7 @@ struct lcba_handle {
   int* d_i8gate = nullptr;        // 1: the last Schur pass fell back to DMMA (k_i8_check)
   double* d_i8mrow = nullptr;     // row maxima of Y (k_i8_rowexp -> k_i8_check)
   bool i8_guard = true;          // LCBA_I8_GUARD=0: no resolution check (tests of the int8 kernels alone)
-  int i8_gx_max = 0, i8_gx_make = 0, i8_groups = 0;
+  int i8_gx_max = 0, i8_gx_make = 0, i8_gx_make_ref = 0, i8_groups = 0;
   // outputs on demand
   double2* d_rout = nullptr;
   double *d_Jc = nullptr, *d_Jp = nullptr;
@@ -334,6 +334,7 @@ extern "C" int lcba_create(lcba_t** out, int device) {
                                       (const void*)k_jdot_dense, (const void*)k_backsub_dense,
                                       (const void*)k_residual_pt, (const void*)k_jdot_pt, (const void*)k_backsub_pt,
                                       (const void*)k_i8_syrk<true>, (const void*)k_i8_syrk<false>, (const void*)k_i8_make,
+                                      (const void*)k_i8_make_ref,
                                       (const void*)k_jdot,      (const void*)k_jacobian_blocks};
     for (const void* f : big_smem_kernels) {
       cudaFuncAttributes fa;
@@ -603,7 +604,8 @@ extern "C" int lcba_set_problem_shard(lcba_t* h, int32_t C, int64_t P, int64_t N
         const I8Plan& ip = h->i8plan;
         h->i8_groups = (C + I8_GROUP_CAMS - 1) / I8_GROUP_CAMS;
         h->i8_gx_max = (int)std::max<long long>(1, std::min<long long>(ip.nkb, (long long)h->sm_count * 4 / h->i8_groups));   // one wave: 4 blocks per SM
-        h->i8_gx_make = (int)std::max<long long>(1, std::min<long long>(ip.nkb, (long long)h->sm_count * 3 / h->i8_groups));   // one wave: 3 blocks per SM
+        h->i8_gx_make = (int)std::max<long long>(1, std::min<long long>(ip.nkb, (long long)h->sm_count * 2 / h->i8_groups));   // one wave: 2 blocks per SM (87 KB of shared memory each)
+        h->i8_gx_make_ref = (int)std::max<long long>(1, std::min<long long>(ip.nkb, (long long)h->sm_count * 3 / h->i8_groups));   // one wave: 3 blocks per SM
         LCBA_TRY(dev_alloc(h, &h->d_i8work, ip.work.size()));
         LCBA_TRY(dev_alloc(h, &h->d_i8tiles, ip.tiles.size()));
         LCBA_CUDA(h, cudaMemcpyAsync(h->d_i8work, ip.work.data(), ip.work.size() * sizeof(I8Work), cudaMemcpyHostToDevice, st));
@@ -951,6 +953,28 @@ static int pass_jdot(lcba_t* h) {
   return check_launch(h, "jdot pass");
 }
 
+// int8 Schur path, the digit planes: row maxima and exponents of Y (after k_point_factor), then the planes
+static void launch_i8_rowexp(lcba_t* h) {
+  const int C = h->C, w = h->cur, RP = h->i8plan.NRG * 8;
+  const size_t smem_rm = ((size_t)I8_GROUP_CAMS * CAMTAB + 192) * 4;
+  KL(h, "i8_rowmax", k_i8_rowmax<<<dim3(h->i8_gx_max, h->i8_groups), 192, smem_rm, h->stream>>>(
+        h->d_tab[w], h->d_pts[w], h->d_pair_w, h->d_pair_start, h->d_mask, h->d_Lz, h->P, C, RP, h->d_i8rmax));
+  KL(h, "i8_rowmax", k_i8_rowexp<<<nblk(RP, 128), 128, 0, h->stream>>>(h->d_i8rmax, h->i8_gx_max, NCP * C + 1, RP,
+                                                                 h->d_i8erow, h->d_i8mrow));
+}
+// ref: k_i8_make_ref, only from lcba_debug_i8_make
+static void launch_i8_make(lcba_t* h, bool ref) {
+  const int C = h->C, w = h->cur, NRG = h->i8plan.NRG;
+  if (ref)
+    KL(h, "make_Y", k_i8_make_ref<<<dim3(h->i8_gx_make_ref, h->i8_groups), 192, i8_make_ref_smem_bytes(), h->stream>>>(
+          h->d_tab[w], h->d_pts[w], h->d_pair_w, h->d_pair_start, h->d_mask, h->d_Lz, h->P, C, NRG, h->d_i8erow,
+          h->d_i8planes));
+  else
+    KL(h, "make_Y", k_i8_make<<<dim3(h->i8_gx_make, h->i8_groups), I8_MK_THREADS, i8_make_smem_bytes(), h->stream>>>(
+          h->d_tab[w], h->d_pts[w], h->d_pair_w, h->d_pair_start, h->d_mask, h->d_Lz, h->P, C, NRG, h->d_i8erow,
+          h->d_i8planes));
+}
+
 static int pass_schur(lcba_t* h, const double* lam_host_or_null) {
   NvtxRange nvtx_("lcba:schur");
   const int C = h->C, w = h->cur, n = C * NCP;
@@ -973,15 +997,8 @@ static int pass_schur(lcba_t* h, const double* lam_host_or_null) {
     if (h->use_i8) {
       // 5th-generation tensor cores: digit planes of Y, exact int8 x int8 -> int32 SYRK, FP64 recombination
       const I8Plan& ip = h->i8plan;
-      const int RP = ip.NRG * 8;
-      const size_t smem_rm = ((size_t)I8_GROUP_CAMS * CAMTAB + 192) * 4;
-      KL(h, "i8_rowmax", k_i8_rowmax<<<dim3(h->i8_gx_max, h->i8_groups), 192, smem_rm, h->stream>>>(
-            h->d_tab[w], h->d_pts[w], h->d_pair_w, h->d_pair_start, h->d_mask, h->d_Lz, h->P, C, RP, h->d_i8rmax));
-      KL(h, "i8_rowmax", k_i8_rowexp<<<nblk(RP, 128), 128, 0, h->stream>>>(h->d_i8rmax, h->i8_gx_max, NCP * C + 1, RP,
-                                                                     h->d_i8erow, h->d_i8mrow));
-      KL(h, "make_Y", k_i8_make<<<dim3(h->i8_gx_make, h->i8_groups), 192, i8_make_smem_bytes(), h->stream>>>(
-            h->d_tab[w], h->d_pts[w], h->d_pair_w, h->d_pair_start, h->d_mask, h->d_Lz, h->P, C, ip.NRG, h->d_i8erow,
-            h->d_i8planes));
+      launch_i8_rowexp(h);
+      launch_i8_make(h, false);
       if (h->i8_tma)
         KL(h, "schur", k_i8_syrk<true><<<(unsigned)ip.work.size(), I8_THREADS, ip.smem_bytes, h->stream>>>(
               h->i8maps, h->d_i8planes, ip.NRG, h->d_i8work, h->d_i8partial, h->d_fail, h->d_stats));
@@ -1933,6 +1950,48 @@ extern "C" int lcba_debug_step(lcba_t* h, double lam, double mu, int32_t mode, d
                                          c.step_norm, (double)c.chol_fail};
     memcpy(scalars_out, v, sizeof(v));
   }
+  return LCBA_OK;
+}
+
+// test hook: the digit planes of the int8 Schur path at the current x, damped with the host's lam, from
+// k_i8_make (ref = 0) or k_i8_make_ref (ref = 1), which runs `reps` times on a plane buffer first filled with the
+// byte `poison` (>= 0), so that a byte the kernel does not write shows
+extern "C" int lcba_debug_i8_make(lcba_t* h, double lam, int32_t ref, int32_t reps, int32_t poison, double* ms_out,
+                                  void* planes_out, int64_t planes_bytes) {
+  if (!h || !h->have_problem) { set_error(h, "lcba_debug_i8_make: no problem set"); return LCBA_E_STATE; }
+  if (!h->use_i8) { set_error(h, "lcba_debug_i8_make: the problem does not take the int8 path (LCBA_SCHUR_I8)"); return LCBA_E_STATE; }
+  if (ref < 0 || ref > 1 || reps < 1 || poison < -1 || poison > 255 ||
+      (planes_out && planes_bytes != (int64_t)h->i8plan.plane_bytes)) {
+    set_error(h, "lcba_debug_i8_make: ref must be 0 or 1, reps >= 1, poison -1..255, planes_bytes = " +
+                     std::to_string(h->i8plan.plane_bytes));
+    return LCBA_E_ARG;
+  }
+  cudaSetDevice(h->device);
+  Ctl init;
+  memset(&init, 0, sizeof(init));
+  init.term = -1;
+  LCBA_CUDA(h, cudaMemcpyAsync(h->d_ctl, &init, sizeof(Ctl), cudaMemcpyHostToDevice, h->stream));
+  LCBA_TRY(pass_linearize(h, 1));
+  KL(h, "point_factor", k_point_factor<<<nblk(h->P, 256), 256, 0, h->stream>>>(
+        h->d_Vg, h->d_scl_p, lam, nullptr, h->P, h->d_Lz));
+  launch_i8_rowexp(h);
+  if (poison >= 0) LCBA_CUDA(h, cudaMemsetAsync(h->d_i8planes, poison, h->i8plan.plane_bytes, h->stream));
+  cudaEvent_t e0, e1;
+  LCBA_CUDA(h, cudaEventCreate(&e0));
+  if (cudaEventCreate(&e1) != cudaSuccess) { cudaEventDestroy(e0); set_error(h, "lcba_debug_i8_make: cudaEventCreate"); return LCBA_E_CUDA; }
+  cudaError_t e = cudaEventRecord(e0, h->stream);
+  for (int r = 0; r < reps && e == cudaSuccess; ++r) launch_i8_make(h, ref != 0);
+  if (e == cudaSuccess) e = cudaGetLastError();
+  if (e == cudaSuccess) e = cudaEventRecord(e1, h->stream);
+  if (e == cudaSuccess && planes_out)
+    e = cudaMemcpyAsync(planes_out, h->d_i8planes, h->i8plan.plane_bytes, cudaMemcpyDeviceToHost, h->stream);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+  float ms = 0.0f;
+  if (e == cudaSuccess) e = cudaEventElapsedTime(&ms, e0, e1);
+  cudaEventDestroy(e0);
+  cudaEventDestroy(e1);
+  if (e != cudaSuccess) { set_error(h, std::string("lcba_debug_i8_make: ") + cudaGetErrorString(e)); return LCBA_E_CUDA; }
+  if (ms_out) *ms_out = (double)ms / reps;
   return LCBA_OK;
 }
 

@@ -511,18 +511,30 @@ __device__ __forceinline__ unsigned long long i8_encode(double v, double scale) 
   return (unsigned long long)(T + 0x808080808080LL) ^ 0x808080808080ULL;
 }
 
+// i8_encode without the FP64 -> int64 conversion (F2I.S64.F64 issues at a fraction of the DFMA rate): for
+// finite |x| < 2^51, x + 1.5 * 2^52 rounded to nearest even holds rint(x) + 2^51 in its 52 fraction bits, so its
+// low 48 bits, the only ones the planes use, are those of __double2ll_rn(x) (here |x| < 2^47).  v * scale is exact
+// (scale is a power of two), so one FMA rounds exactly like the product followed by the addition.  A non-finite
+// Y gives other bytes than i8_encode (whose conversion saturates); both are meaningless, and k_i8_rowexp's fmax
+// passes a NaN by in either case.
+__device__ __forceinline__ unsigned long long i8_encode_fma(double v, double scale) {
+  const unsigned long long T = (unsigned long long)__double_as_longlong(fma(v, scale, 6755399441055744.0));
+  return (T + 0x808080808080ULL) ^ 0x808080808080ULL;
+}
+
 constexpr int I8_VAL_LD = 65;             // row stride (64-bit words) of the staging tile: conflict-free both ways
-inline size_t i8_make_smem_bytes() {
+inline size_t i8_make_ref_smem_bytes() {
   return (size_t)I8_GROUP_CAMS * CAMTAB * 8 + (size_t)I8_GROUP_ROWS * 8 + (size_t)I8_GROUP_ROWS * I8_VAL_LD * 8;
 }
 
+// The first k_i8_make, kept as the reference the tests compare k_i8_make's planes with (lcba_debug_i8_make).
 // planes[((kb * NS + i) * NRG + rg) * 512 + a * 256 + kh * 128 + r8 * 16 + kbyte], kappa_local = 32 a + 16 kh + kbyte.
 // block (kb stride, g).  Phase 1: thread = (point lane, camera) evaluates Y in FP64 and writes the 33
 // encoded integers to the staging tile [row][kappa] (one 64-bit store each).  Phase 2: a warp takes one
 // (row group, k-step, k half): lane = (row r8, kappa quad) reads 4 integers, picks byte 5 - i of each with
 // PRMT and stores one 32-bit word per slice: 128 contiguous bytes per warp and slice, straight to HBM.
 __global__ void __launch_bounds__(192, 3)
-k_i8_make(const double* __restrict__ tab, const double* __restrict__ pts, const double* __restrict__ wgt,
+k_i8_make_ref(const double* __restrict__ tab, const double* __restrict__ pts, const double* __restrict__ wgt,
           const uint32_t* __restrict__ obs_start, const unsigned long long* __restrict__ mask,
           const double* __restrict__ Lz, long long P, int C, int NRG, const int* __restrict__ e_row,
           unsigned char* __restrict__ planes) {
@@ -639,6 +651,193 @@ k_i8_make(const double* __restrict__ tab, const double* __restrict__ pts, const 
       }
     }
     __syncthreads();
+  }
+}
+
+// k_i8_make: the same planes as k_i8_make_ref, byte for byte, with evaluation and draining overlapped.
+// Warps 0-5 evaluate (thread = (point lane q, camera), as in k_i8_make_ref but q = slot: the 4 point lanes
+// of a warp then differ mod 4 and the 32-bit staging stores are conflict-free); warps 6-7 drain.  The
+// staging tile is double-buffered and split into the low 32 and the top 16 bits of each encoded integer
+// (48 bits of data, 6 B staged per entry instead of 8); the row strides (68 words, 72 halves = 36 words,
+// both 4 mod 32) make the drain's 16-byte loads of 8 rows conflict-free.  Named barriers hand a buffer
+// over: FULL[b] (evaluators arrive, drainers wait), EMPTY[b] (drainers arrive, evaluators wait two blocks
+// later), so an evaluator never waits for stores and a drainer never for FP64.  A drain lane = (row r8,
+// k half kh, k-step a) packs 16 kappa of one row, one core-matrix row per digit, and stores 16 B per
+// slice: a warp writes one whole 512-byte row group per slice.  The weight chain obs_start -> wgt is
+// prefetched in two stages (index two blocks ahead, weight one block ahead) with the mask, point and factor.
+constexpr int I8_MK_EVAL = 192;           // evaluator threads (warps 0-5)
+constexpr int I8_MK_DRAIN = 64;           // drainer threads (warps 6-7)
+constexpr int I8_MK_THREADS = I8_MK_EVAL + I8_MK_DRAIN;
+constexpr int I8_MK_LDL = 68;             // row stride of the low words (u32)
+constexpr int I8_MK_LDH = 72;             // row stride of the top halves (u16)
+constexpr int I8_MK_LO = I8_GROUP_ROWS * I8_MK_LDL;    // u32 per buffer
+constexpr int I8_MK_HI = I8_GROUP_ROWS * I8_MK_LDH;    // u16 per buffer
+inline size_t i8_make_smem_bytes() {
+  return (size_t)I8_GROUP_CAMS * CAMTAB * 8 + (size_t)I8_GROUP_ROWS * 8 + 2 * ((size_t)I8_MK_LO * 4 + (size_t)I8_MK_HI * 2);
+}
+// named barriers with immediate ids (a register id makes ptxas reserve all 16)
+template <int ID> __device__ __forceinline__ void i8_bar_sync() { asm volatile("bar.sync %0, %1;" ::"n"(ID), "n"(I8_MK_THREADS) : "memory"); }
+template <int ID> __device__ __forceinline__ void i8_bar_arrive() { asm volatile("bar.arrive %0, %1;" ::"n"(ID), "n"(I8_MK_THREADS) : "memory"); }
+
+__global__ void __launch_bounds__(I8_MK_THREADS, 2)
+k_i8_make(const double* __restrict__ tab, const double* __restrict__ pts, const double* __restrict__ wgt,
+          const uint32_t* __restrict__ obs_start, const unsigned long long* __restrict__ mask,
+          const double* __restrict__ Lz, long long P, int C, int NRG, const int* __restrict__ e_row,
+          unsigned char* __restrict__ planes) {
+  extern __shared__ __align__(16) unsigned char s_raw[];
+  double* s_tab = reinterpret_cast<double*>(s_raw);                                        // 8 * CAMTAB
+  double* s_scale = s_tab + I8_GROUP_CAMS * CAMTAB;                                        // I8_GROUP_ROWS: 2^(48 - e_row)
+  uint32_t* s_lo = reinterpret_cast<uint32_t*>(s_scale + I8_GROUP_ROWS);                   // [2][rows][I8_MK_LDL]
+  uint16_t* s_hi = reinterpret_cast<uint16_t*>(s_lo + 2 * I8_MK_LO);                       // [2][rows][I8_MK_LDH]
+  constexpr int BAR_FULL = 1, BAR_EMPTY = 3;                                               // + buffer
+  const int t = threadIdx.x, g = blockIdx.y;
+  const int c0 = g * I8_GROUP_CAMS, gc = min(I8_GROUP_CAMS, C - c0);
+  const int rg0 = 11 * g;
+  const int nrgl = (g == (int)gridDim.y - 1) ? NRG - rg0 : 11;
+  for (int i = t; i < gc * CAMTAB; i += blockDim.x) s_tab[i] = tab[c0 * CAMTAB + i];
+  for (int i = t; i < I8_GROUP_ROWS; i += blockDim.x)
+    s_scale[i] = (rg0 * 8 + i < NRG * 8) ? ldexp(1.0, 8 * I8_NS - e_row[rg0 * 8 + i]) : 0.0;
+  {
+    uint4* z = reinterpret_cast<uint4*>(s_lo);                 // padding rows / column 63 stay 0 in both buffers
+    const int n16 = (2 * I8_MK_LO * 4 + 2 * I8_MK_HI * 2) / 16;
+    for (int i = t; i < n16; i += blockDim.x) z[i] = make_uint4(0u, 0u, 0u, 0u);
+  }
+  __syncthreads();
+  const long long nkb = (P + I8_PTS - 1) / I8_PTS;
+  const long long G = gridDim.x;
+
+  if (t < I8_MK_EVAL) {
+    // ---------------------------------------------------------------- evaluators
+    const bool worker = t < I8_PTS * gc;
+    const int q = worker ? t / gc : 0, cl = worker ? t % gc : 0, cam = c0 + cl;
+    const bool zthread = (g == (int)gridDim.y - 1) && t >= 168 && t < 168 + I8_PTS;
+    const int zrow = NCP * C - rg0 * 8;
+    const unsigned long long below = (1ull << cam) - 1ull;
+    // stage 2 (two blocks ahead): mask and CSR offset; stage 1 (one block ahead): point, factor and weight
+    unsigned long long a_m = 0ull;
+    uint32_t a_os = 0u;
+    auto prefetch2 = [&](long long kb) {
+      a_m = 0ull;
+      const long long p = kb * I8_PTS + q;
+      if (worker && kb < nkb && p < P) { a_m = mask[p]; a_os = wgt ? obs_start[p] : 0u; }
+    };
+    unsigned long long n_m = 0ull;
+    double n_X[3] = {0, 0, 0}, n_li[6] = {0, 0, 0, 0, 0, 0}, n_w = 1.0;
+    auto prefetch1 = [&](long long kb) {     // takes the stage-2 values of block kb
+      n_m = a_m;
+      const long long p = kb * I8_PTS + q;
+      if (worker && kb < nkb && p < P) {
+#pragma unroll
+        for (int a = 0; a < 3; ++a) n_X[a] = pts[3 * p + a];
+#pragma unroll
+        for (int a = 0; a < 6; ++a) n_li[a] = Lz[p * 9 + a];
+        if (wgt && ((n_m >> cam) & 1ull)) n_w = wgt[(long long)a_os + __popcll(n_m & below)];
+      }
+    };
+    prefetch2(blockIdx.x);
+    prefetch1(blockIdx.x);
+    prefetch2(blockIdx.x + G);
+    int it = 0;
+    for (long long kb = blockIdx.x; kb < nkb; kb += G, ++it) {
+      const int b = it & 1;
+      const unsigned long long m = n_m;
+      const bool live = (m >> cam) & 1ull;
+      const double w = n_w;
+      double X[3], li[6];
+#pragma unroll
+      for (int a = 0; a < 3; ++a) X[a] = n_X[a];
+#pragma unroll
+      for (int a = 0; a < 6; ++a) li[a] = n_li[a];
+      prefetch1(kb + G);
+      prefetch2(kb + 2 * G);
+      if (it >= 2) { if (b) i8_bar_sync<BAR_EMPTY + 1>(); else i8_bar_sync<BAR_EMPTY>(); }                  // the drain of block kb - 2 G has read buffer b
+      uint32_t* lo = s_lo + b * I8_MK_LO;
+      uint16_t* hi = s_hi + b * I8_MK_HI;
+      if (worker) {
+        uint32_t* dlo = lo + (cl * NCP) * I8_MK_LDL + 3 * q;
+        uint16_t* dhi = hi + (cl * NCP) * I8_MK_LDH + 3 * q;
+        if (live) {
+          ObsLin L;
+          obs_linearize<false>(s_tab + cl * CAMTAB, X[0], X[1], X[2], 0.0, 0.0, w, L);
+          const double* sc = s_scale + cl * NCP;
+#pragma unroll
+          for (int k = 0; k < 3; ++k) {
+            double q0, q1;                                   // column k of Q = Jp L^-T
+            if (k == 0) { q0 = L.Jp[0][0] * li[0]; q1 = L.Jp[1][0] * li[0]; }
+            else if (k == 1) { q0 = fma(L.Jp[0][0], li[1], L.Jp[0][1] * li[2]); q1 = fma(L.Jp[1][0], li[1], L.Jp[1][1] * li[2]); }
+            else { q0 = fma(L.Jp[0][0], li[3], fma(L.Jp[0][1], li[4], L.Jp[0][2] * li[5]));
+                   q1 = fma(L.Jp[1][0], li[3], fma(L.Jp[1][1], li[4], L.Jp[1][2] * li[5])); }
+#pragma unroll
+            for (int a = 0; a < NCP; ++a) {
+              const double y = a < 9 ? fma(L.Jc[0][a], q0, L.Jc[1][a] * q1) : (a == 9 ? w * q0 : w * q1);
+              const unsigned long long v = i8_encode_fma(y, sc[a]);
+              dlo[a * I8_MK_LDL + k] = (uint32_t)v;
+              dhi[a * I8_MK_LDH + k] = (uint16_t)(v >> 32);
+            }
+          }
+        } else {
+          // invisible pairs and the ragged tail are exact zeros
+#pragma unroll
+          for (int k = 0; k < 3; ++k)
+#pragma unroll
+            for (int a = 0; a < NCP; ++a) { dlo[a * I8_MK_LDL + k] = 0u; dhi[a * I8_MK_LDH + k] = 0u; }
+        }
+      }
+      if (zthread) {
+        const int qq = t - 168;
+        const long long pz = kb * I8_PTS + qq;
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+          const unsigned long long v = pz < P ? i8_encode_fma(Lz[pz * 9 + 6 + k], s_scale[zrow]) : 0ull;
+          lo[zrow * I8_MK_LDL + 3 * qq + k] = (uint32_t)v;
+          hi[zrow * I8_MK_LDH + 3 * qq + k] = (uint16_t)(v >> 32);
+        }
+      }
+      __threadfence_block();
+      if (b) i8_bar_arrive<BAR_FULL + 1>(); else i8_bar_arrive<BAR_FULL>();
+    }
+  } else {
+    // ---------------------------------------------------------------- drainers
+    const int lane = t & 31, dw = (t - I8_MK_EVAL) >> 5;
+    const int r8 = lane & 7, kh = (lane >> 3) & 1, a = lane >> 4;
+    const int kap = 32 * a + 16 * kh;
+    const size_t sstride = (size_t)NRG * I8_RG_BYTES;
+    int it = 0;
+    for (long long kb = blockIdx.x; kb < nkb; kb += G, ++it) {
+      const int b = it & 1;
+      if (b) i8_bar_sync<BAR_FULL + 1>(); else i8_bar_sync<BAR_FULL>();
+      const uint32_t* lo = s_lo + b * I8_MK_LO + r8 * I8_MK_LDL + kap;
+      const uint16_t* hi = s_hi + b * I8_MK_HI + r8 * I8_MK_LDH + kap;
+      unsigned char* lane_dst = planes + (((size_t)kb * I8_NS) * NRG + rg0) * I8_RG_BYTES + a * 256 + kh * 128 + r8 * 16;
+      for (int rgl = dw; rgl < nrgl; rgl += I8_MK_DRAIN / 32) {
+        const uint4* sl = reinterpret_cast<const uint4*>(lo + rgl * 8 * I8_MK_LDL);
+        const uint4* sh = reinterpret_cast<const uint4*>(hi + rgl * 8 * I8_MK_LDH);
+        uint32_t x[16], hw[8];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) { const uint4 u = sl[j]; x[4 * j] = u.x; x[4 * j + 1] = u.y; x[4 * j + 2] = u.z; x[4 * j + 3] = u.w; }
+#pragma unroll
+        for (int j = 0; j < 2; ++j) { const uint4 u = sh[j]; hw[4 * j] = u.x; hw[4 * j + 1] = u.y; hw[4 * j + 2] = u.z; hw[4 * j + 3] = u.w; }
+        // out[i][j]: slice i, kappa 4 j .. 4 j + 3.  Slices 0, 1 = bytes 1, 0 of the top halves (two per word);
+        // slices 2..5 = bytes 3..0 of the low words (a 4 x 4 byte transpose per kappa quad)
+        uint32_t out[I8_NS][4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          out[0][j] = __byte_perm(hw[2 * j], hw[2 * j + 1], 0x7531);
+          out[1][j] = __byte_perm(hw[2 * j], hw[2 * j + 1], 0x6420);
+          const uint32_t t0 = __byte_perm(x[4 * j], x[4 * j + 1], 0x5140), t1 = __byte_perm(x[4 * j + 2], x[4 * j + 3], 0x5140);
+          const uint32_t t2 = __byte_perm(x[4 * j], x[4 * j + 1], 0x7362), t3 = __byte_perm(x[4 * j + 2], x[4 * j + 3], 0x7362);
+          out[2][j] = __byte_perm(t2, t3, 0x7632);
+          out[3][j] = __byte_perm(t2, t3, 0x5410);
+          out[4][j] = __byte_perm(t0, t1, 0x7632);
+          out[5][j] = __byte_perm(t0, t1, 0x5410);
+        }
+        unsigned char* dst = lane_dst + (size_t)rgl * I8_RG_BYTES;
+#pragma unroll
+        for (int i = 0; i < I8_NS; ++i)
+          *reinterpret_cast<uint4*>(dst + (size_t)i * sstride) = make_uint4(out[i][0], out[i][1], out[i][2], out[i][3]);
+      }
+      if (kb + 2 * G < nkb) { if (b) i8_bar_arrive<BAR_EMPTY + 1>(); else i8_bar_arrive<BAR_EMPTY>(); }      // the evaluators refill buffer b for block kb + 2 G
+    }
   }
 }
 
