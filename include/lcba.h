@@ -137,6 +137,18 @@ int lcba_set_problem_shard(lcba_t* h, int32_t C, int64_t P, int64_t N, const dou
                            const int64_t* pt_idx, const double* weights_or_null, int64_t pt_offset);
 /* Replace the current parameter vector x = [cams.ravel(), pts.ravel()]. */
 int lcba_set_params(lcba_t* h, const double* cams, const double* pts);
+/* Hold parameters at their current values: cam_fixed C x 11 bytes (row-major like cams), pt_fixed one byte
+ * per point of THIS handle's P points (its shard on a point-sharded job); nonzero = held, NULL clears that
+ * mask.  A masked lcba_solve is scipy's trf_no_bounds on the free sub-vector with the same residuals: the
+ * Jacobi scaling, the initial Delta, reg_term, the 2-D subspace, |x| (xtol) and |g|_inf (gtol, optimality)
+ * run over free entries only, max_nfev defaults to 100 * n_free, and held entries of x come back
+ * bit-identical.  The masks apply to lcba_solve and lcba_debug_step (and lcba_debug_i8_make); lcba_get_grad
+ * after them returns 0 at held entries.  lcba_linearize stays the unmasked tap.  lcba_set_problem /
+ * lcba_set_problem_shard clear both masks, lcba_set_params keeps them.  The point mask combines with
+ * fix_cameras and shared_intrinsics; a camera mask with shared_intrinsics makes lcba_solve return
+ * LCBA_E_UNSUPPORTED, nothing free LCBA_E_ARG.  Sharded jobs: the camera mask must be the same on every
+ * rank (lcba_solve compares its count and checksum over the ranks and fails on every rank otherwise). */
+int lcba_set_fixed(lcba_t* h, const uint8_t* cam_fixed, const uint8_t* pt_fixed);
 /* PySBA.optimizedParams (pySBA.py:121-129): copy x back, split. */
 int lcba_get_params(lcba_t* h, double* cams_out, double* pts_out);
 
@@ -205,6 +217,7 @@ int lcba_get_profile(lcba_t* h, lcba_kernel_stat* stats, int32_t max_stats, int3
  * Linearise at the current x and form the damped reduced camera system
  *   S = U + lam*Dc^2 - sum_p W (V + lam*Dp^2)^-1 W^T,  rhs = gc - sum_p W (V+lam*Dp^2)^-1 gp
  * with D = column norms of J (first-call Jacobi scaling).  Any output may be NULL.
+ * Ignores the masks of lcba_set_fixed (every parameter free): the unmasked debug tap.
  * S_out (11C)^2 full symmetric, rhs_out 11C, grad_out 11C+3P, scale_inv_out 11C+3P. */
 int lcba_linearize(lcba_t* h, double lam, double* S_out, double* rhs_out, double* grad_out,
                    double* scale_inv_out, double* cost_out);
@@ -224,7 +237,8 @@ int lcba_nccl_unique_id(void* id_out128);
 /* id128 != NULL: create the process-wide communicator (collective over all ranks);
  * id128 == NULL: attach the communicator this process created earlier to another handle. */
 int lcba_comm_init(lcba_t* h, int32_t rank, int32_t nranks, const void* id128);
-/* total point count over all ranks is needed for max_nfev = 100*n and is all-reduced. */
+/* total point count over all ranks is needed for max_nfev = 100*n and is all-reduced, together with
+ * the held point count and the camera mask's count and checksum (lcba_set_fixed). */
 
 /* ---- test hook -----------------------------------------------------------------------
  * The 2-D trust-region sub-problem solver the device control kernel uses
@@ -247,7 +261,7 @@ int lcba_debug_chol(lcba_t* h, int32_t n, const double* A, const double* rhs, do
  * reg_term, point factors and the reduced camera system damped with `lam` (it overrides reg_term,
  * like lcba_linearize), the dense camera solve with extra damping mu * Dc^2, back-substitution and the
  * 2-D subspace scalars.  mode 0: all parameters; 1: cameras fixed (fix_cameras); 2: shared
- * intrinsics.  pc_out 11C (the camera step, expanded in mode 2; zeros in mode 1), pp_out 3P (the
+ * intrinsics; the masks of lcba_set_fixed apply (held entries of the step are 0).  pc_out 11C (the camera step, expanded in mode 2; zeros in mode 1), pp_out 3P (the
  * point step); scalars_out LCBA_STEP_SCALARS doubles:
  *   [0] reg_term  [1] Delta  [2] Jg2 = |J D^-2 g|^2
  *   [3] aa  [4] ab  [5] bb      (a = g_h = g / s, b = gn_h = p * s, scaled space)

@@ -23,7 +23,7 @@ SYMBOLS = ["lcba_version", "lcba_create", "lcba_destroy", "lcba_last_error", "lc
            "lcba_sq_normal", "lcba_debug_schur_stats", "lcba_debug_mma_plan",
            "lcba_set_iteration_callback", "lcba_debug_i8_plan", "lcba_host_is_nondecreasing_i64", "lcba_debug_peer_reduce",
            "lcba_debug_i8_fallback", "lcba_debug_chol", "lcba_debug_step", "lcba_debug_i8_cover_plan",
-           "lcba_debug_i8_make"]
+           "lcba_debug_i8_make", "lcba_set_fixed"]
 
 # scalars_out of lcba_debug_step, in order (include/lcba.h)
 STEP_SCALARS = ["reg_term", "Delta", "Jg2", "aa", "ab", "bb", "JAA", "JAB", "JBB", "gtgt", "gtp", "pp",
@@ -94,6 +94,7 @@ def load():
     lib.lcba_set_problem_shard.argtypes = [vp, i32, i64, i64, vp, vp, vp, vp, vp, vp, i64]
     lib.lcba_set_params.argtypes = [vp, vp, vp]
     lib.lcba_get_params.argtypes = [vp, vp, vp]
+    lib.lcba_set_fixed.argtypes = [vp, vp, vp]
     lib.lcba_rotate.argtypes = [vp, i64, vp, vp, vp]
     lib.lcba_project.argtypes = [vp, i64, vp, vp, vp]
     lib.lcba_unproject.argtypes = [vp, i64, vp, vp, i64, vp, vp, vp, vp, vp]
@@ -160,6 +161,7 @@ class Engine:
             raise LcbaError(rc, self.lib.lcba_last_error(None).decode())
         self.h = h
         self.C = self.P = self.N = 0
+        self.has_fixed = False     # a mask of set_fixed is in place (set_problem clears it)
         # bumped by every call that changes what the handle holds (observation set or x): lazy
         # readers (res.fun / res.grad / res.jac) compare it with the value they were created at
         self.generation = 0
@@ -196,12 +198,25 @@ class Engine:
                                                     _ptr(cams), _ptr(pts), _ptr(p2), _ptr(ci),
                                                     _ptr(pi), _ptr(w), int(pt_offset)))
         self.C, self.P, self.N = cams.shape[0], pts.shape[0], N
+        self.has_fixed = False
         self.generation += 1
 
     def set_params(self, cams, pts):
         self.generation += 1
         cams, pts = _f64(cams, (self.C, 11)), _f64(pts, (self.P, 3))
         self._check(self.lib.lcba_set_params(self.h, _ptr(cams), _ptr(pts)))
+
+    def set_fixed(self, cam_fixed=None, pt_fixed=None):
+        """Hold parameters at their current values in solve() and debug_step() (lcba_set_fixed):
+        cam_fixed bool (C, 11), pt_fixed bool (P,) over this handle's points; None clears that mask."""
+        cm = None if cam_fixed is None else np.ascontiguousarray(cam_fixed, dtype=np.uint8)
+        pm = None if pt_fixed is None else np.ascontiguousarray(pt_fixed, dtype=np.uint8)
+        if cm is not None and cm.shape != (self.C, 11):
+            raise ValueError("cam_fixed must have shape (%d, 11)" % self.C)
+        if pm is not None and pm.shape != (self.P,):
+            raise ValueError("pt_fixed must have shape (%d,)" % self.P)
+        self._check(self.lib.lcba_set_fixed(self.h, _ptr(cm), _ptr(pm)))
+        self.has_fixed = cm is not None or pm is not None
 
     def get_params(self, x_out=None):
         """(cams, pts) of the current iterate; with `x_out` (11 C + 3 P doubles, contiguous) the

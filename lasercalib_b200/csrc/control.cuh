@@ -120,10 +120,12 @@ __device__ inline void ctl_solve_subspace(Ctl* c) {
 
 // after k_linearize + reduction: camera scaling (common.py:598-610), g~_c, camera sums
 // camsum[c*22 + a] = g_c, camsum[c*22 + 11 + a] = diag(J^T J); camsum[22C] = sum r^2
+// cam_fixed (C x 11, may be NULL): entries held constant, like every entry under fix_cameras
 __global__ void __launch_bounds__(256)
 k_ctl_lin(const double* __restrict__ camsum, const double* __restrict__ cams,
           double* __restrict__ scl_c, double* __restrict__ gt_c, double* __restrict__ g_c, int C,
-          Ctl* __restrict__ ctl, int first, int fix_cameras, int shared_intr) {
+          Ctl* __restrict__ ctl, int first, int fix_cameras, const uint8_t* __restrict__ cam_fixed,
+          int shared_intr) {
   __shared__ double s_red[32];
   __shared__ double s_sh[6];   // shared-intrinsics mode: summed gradient / diag of (f, k1, k2)
   if (shared_intr) {
@@ -138,7 +140,7 @@ k_ctl_lin(const double* __restrict__ camsum, const double* __restrict__ cams,
   double gh2 = 0, xs2 = 0, x2 = 0, gmax = 0;
   for (int i = threadIdx.x; i < C * NCP; i += blockDim.x) {
     const int c = i / NCP, a = i % NCP;
-    if (fix_cameras) {          // cameras are constants: no gradient, no scale, no norm share
+    if (fix_cameras || (cam_fixed && cam_fixed[i])) {   // constants: no gradient, no scale, no norm share
       scl_c[i] = 1.0; g_c[i] = 0.0; gt_c[i] = 0.0;
       continue;
     }

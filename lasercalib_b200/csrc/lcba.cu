@@ -158,6 +158,13 @@ struct lcba_handle {
   ncclComm_t comm = nullptr;
   int rank = 0, nranks = 1;
   int fix_cameras = 0, shared_intr = 0;
+  // held parameters (lcba_set_fixed): C x 11 camera bytes and one byte per point of this shard, 1 = held.
+  // Allocated with the problem and zero when nothing is held; their addresses never change, so the
+  // captured graphs stay valid when the contents do.  masks_on = false: lcba_linearize, the unmasked tap.
+  uint8_t *d_cam_fixed = nullptr, *d_pt_fixed = nullptr;
+  long long n_cam_held = 0, n_pt_held = 0;
+  double cam_fixed_sum = 0.0;      // checksum of the camera mask (the same on every rank of a sharded job)
+  bool masks_on = true;
   double *d_pred = nullptr, *d_scl_red = nullptr;   // shared-intrinsics mode: reduced step / scale
   double *d_sqpart = nullptr, *d_sqout = nullptr, *d_theta = nullptr;   // squared-residual variants
   int sq_grid = 0, sq_K = 0;
@@ -411,6 +418,12 @@ extern "C" int lcba_set_problem_shard(lcba_t* h, int32_t C, int64_t P, int64_t N
   LCBA_TRY(dev_alloc(h, &h->d_pt, (size_t)N));
   LCBA_TRY(dev_alloc(h, &h->d_obs_start, (size_t)P + 1));
   LCBA_TRY(dev_alloc(h, &h->d_mask, (size_t)P));
+  LCBA_TRY(dev_alloc(h, &h->d_cam_fixed, (size_t)C * NCP));
+  LCBA_TRY(dev_alloc(h, &h->d_pt_fixed, (size_t)P));
+  LCBA_CUDA(h, cudaMemsetAsync(h->d_cam_fixed, 0, (size_t)C * NCP, h->stream));
+  LCBA_CUDA(h, cudaMemsetAsync(h->d_pt_fixed, 0, (size_t)P, h->stream));
+  h->n_cam_held = h->n_pt_held = 0;
+  h->cam_fixed_sum = 0.0;
 
   // temporaries (freed at the end of ingest)
   long long *t_cam = nullptr, *t_pt = nullptr;
@@ -691,6 +704,35 @@ extern "C" int lcba_set_params(lcba_t* h, const double* cams, const double* pts)
   return LCBA_OK;
 }
 
+extern "C" int lcba_set_fixed(lcba_t* h, const uint8_t* cam_fixed, const uint8_t* pt_fixed) {
+  if (!h || !h->have_problem) { set_error(h, "lcba_set_fixed: no problem set"); return LCBA_E_STATE; }
+  cudaSetDevice(h->device);
+  const size_t nc = (size_t)h->C * NCP;
+  long long nch = 0, nph = 0;
+  uint32_t chk = 0;
+  if (cam_fixed) {
+    for (size_t i = 0; i < nc; ++i)
+      if (cam_fixed[i]) { ++nch; chk = chk * 31u + (uint32_t)(i + 1); }
+    LCBA_CUDA(h, cudaMemcpyAsync(h->d_cam_fixed, cam_fixed, nc, cudaMemcpyHostToDevice, h->stream));
+  } else if (h->n_cam_held) {
+    LCBA_CUDA(h, cudaMemsetAsync(h->d_cam_fixed, 0, nc, h->stream));
+  }
+  if (pt_fixed) {
+    for (long long p = 0; p < h->P; ++p) nph += pt_fixed[p] != 0;
+    LCBA_CUDA(h, cudaMemcpyAsync(h->d_pt_fixed, pt_fixed, (size_t)h->P, cudaMemcpyHostToDevice, h->stream));
+  } else if (h->n_pt_held) {
+    LCBA_CUDA(h, cudaMemsetAsync(h->d_pt_fixed, 0, (size_t)h->P, h->stream));
+  }
+  LCBA_CUDA(h, cudaStreamSynchronize(h->stream));
+  h->n_cam_held = nch;
+  h->n_pt_held = nph;
+  h->cam_fixed_sum = (double)chk;
+  return LCBA_OK;
+}
+
+static const uint8_t* cam_mask(const lcba_t* h) { return h->masks_on ? h->d_cam_fixed : nullptr; }
+static const uint8_t* pt_mask(const lcba_t* h) { return h->masks_on ? h->d_pt_fixed : nullptr; }
+
 extern "C" int lcba_get_params(lcba_t* h, double* cams_out, double* pts_out) {
   if (!h || !h->have_problem) { set_error(h, "lcba_get_params: no problem set"); return LCBA_E_STATE; }
   cudaSetDevice(h->device);
@@ -920,12 +962,13 @@ static int pass_linearize(lcba_t* h, int first) {
   // all-reduce carries [camera sums | cost | point sums] and one max all-reduce |g|_inf
   double* pp = h->d_camsum + C * CAMSUM + 1;
   KL(h, "point_prep", k_point_prep<<<h->pt_grid, 256, 0, h->stream>>>(
-        h->d_Vg, h->d_pts[w], h->d_scl_p, h->d_gt_p, h->P, first, h->d_part));
+        h->d_Vg, h->d_pts[w], h->d_scl_p, h->d_gt_p, h->P, first, pt_mask(h), h->d_part));
   KL(h, "reduce", k_reduce_scalars<<<PP_K, 256, 0, h->stream>>>(h->d_part, h->pt_grid, PP_K, pp, 3));
   LCBA_TRY(allreduce(h, h->d_camsum, (size_t)C * CAMSUM + 1 + 3, NCCL_SUM));
   LCBA_TRY(allreduce(h, pp + 3, 1, NCCL_MAX));
   KL(h, "ctl", k_ctl_lin<<<1, 256, 0, h->stream>>>(h->d_camsum, h->d_cams[w], h->d_scl_c, h->d_gt_c,
-                                                   h->d_g_c, C, h->d_ctl, first, h->fix_cameras, h->shared_intr));
+                                                   h->d_g_c, C, h->d_ctl, first, h->fix_cameras, cam_mask(h),
+                                                   h->shared_intr));
   KL(h, "ctl", k_ctl_lin2<<<1, 1, 0, h->stream>>>(pp, h->d_ctl, first));
   return check_launch(h, "linearize pass");
 }
@@ -982,7 +1025,7 @@ static int pass_schur(lcba_t* h, const double* lam_host_or_null) {
   const double lam_arg = lam_host_or_null ? *lam_host_or_null : 0.0;
   const Ctl* ctl_arg = lam_host_or_null ? nullptr : h->d_ctl;
   KL(h, "point_factor", k_point_factor<<<nblk(h->P, 256), 256, 0, h->stream>>>(
-        h->d_Vg, h->d_scl_p, lam_arg, ctl_arg, h->P, h->d_Lz));
+        h->d_Vg, h->d_scl_p, lam_arg, ctl_arg, h->P, pt_mask(h), h->d_Lz));
   if (h->use_mma) {
     // dense rigs: SYRK on the FP64 tensor path + the camera blocks U from their own pass
     const MmaPlan& mp = h->mplan;
@@ -1084,7 +1127,7 @@ static int pass_schur(lcba_t* h, const double* lam_host_or_null) {
           h->d_scl_red));
   } else {
     KL(h, "assemble", k_assemble_S<<<nblk((long long)n * n, 256), 256, 0, h->stream>>>(
-          h->d_Sred, C, pl.npairs, h->d_camsum, h->d_scl_c, lam_arg, ctl_arg, h->d_S, h->d_rhs));
+          h->d_Sred, C, pl.npairs, h->d_camsum, h->d_scl_c, lam_arg, ctl_arg, cam_mask(h), h->d_S, h->d_rhs));
   }
   return check_launch(h, "schur pass");
 }
@@ -1261,16 +1304,31 @@ extern "C" int lcba_solve(lcba_t* h, const lcba_options* opt_in, lcba_result* re
   h->prof.clear();
   h->prof_on = opt.profile != 0;
   const long long launches0 = h->launches, replays0 = h->graph_replays;
-  if (h->comm) {   // total point count over the ranks (max_nfev = 100 n)
-    double v = (double)h->P;
-    LCBA_CUDA(h, cudaMemcpyAsync(h->d_red, &v, 8, cudaMemcpyHostToDevice, h->stream));
-    LCBA_TRY(allreduce(h, h->d_red, 1, NCCL_SUM));
-    LCBA_CUDA(h, cudaMemcpyAsync(&v, h->d_red, 8, cudaMemcpyDeviceToHost, h->stream));
+  long long pt_held_total = h->n_pt_held;
+  if (h->comm) {
+    // total point and held-point counts over the ranks (max_nfev = 100 n_free); the camera mask must be the
+    // same on every rank: max of (count, checksum) and of their negatives, so that every rank sees a mismatch
+    double v[6] = {(double)h->P, (double)h->n_pt_held, (double)h->n_cam_held, h->cam_fixed_sum,
+                   -(double)h->n_cam_held, -h->cam_fixed_sum};
+    LCBA_CUDA(h, cudaMemcpyAsync(h->d_red, v, sizeof(v), cudaMemcpyHostToDevice, h->stream));
+    LCBA_TRY(allreduce(h, h->d_red, 2, NCCL_SUM));
+    LCBA_TRY(allreduce(h, h->d_red + 2, 4, NCCL_MAX));
+    LCBA_CUDA(h, cudaMemcpyAsync(v, h->d_red, sizeof(v), cudaMemcpyDeviceToHost, h->stream));
     LCBA_CUDA(h, cudaStreamSynchronize(h->stream));
-    h->P_total = (long long)(v + 0.5);
+    h->P_total = (long long)(v[0] + 0.5);
+    pt_held_total = (long long)(v[1] + 0.5);
+    if (v[2] != -v[4] || v[3] != -v[5]) {
+      set_error(h, "lcba_solve: the ranks hold different camera masks (lcba_set_fixed)");
+      return LCBA_E_ARG;
+    }
   }
   h->fix_cameras = opt.fix_cameras ? 1 : 0;
   h->shared_intr = (opt.shared_intrinsics && !h->fix_cameras) ? 1 : 0;
+  h->masks_on = true;
+  if (h->shared_intr && h->n_cam_held) {
+    set_error(h, "lcba_solve: a camera mask together with shared_intrinsics is not supported");
+    return LCBA_E_UNSUPPORTED;
+  }
   {
     static const bool env_off = getenv("LCBA_GRAPH") && atoi(getenv("LCBA_GRAPH")) == 0;
     if (env_off) h->use_graphs = false;
@@ -1283,8 +1341,12 @@ extern "C" int lcba_solve(lcba_t* h, const lcba_options* opt_in, lcba_result* re
   const bool graphs = h->solves_on_problem >= 1 && !h->comm && h->N < (8LL << 20);
   h->solves_on_problem++;
   const int gkey = h->fix_cameras * 2 + h->shared_intr;
-  const long long n_cam = h->fix_cameras ? 0 : (h->shared_intr ? 3 + 8LL * h->C : (long long)h->C * NCP);
-  const long long n_total = n_cam + 3 * h->P_total;
+  const long long n_cam = h->fix_cameras ? 0 : (h->shared_intr ? 3 + 8LL * h->C : (long long)h->C * NCP - h->n_cam_held);
+  const long long n_total = n_cam + 3 * (h->P_total - pt_held_total);
+  if (n_total <= 0) {
+    set_error(h, "lcba_solve: every parameter is held (lcba_set_fixed): nothing to optimise");
+    return LCBA_E_ARG;
+  }
   const long long max_nfev = opt.max_nfev > 0 ? opt.max_nfev : 100 * n_total;
 
   struct EventPair {   // destroyed on every exit path
@@ -1340,7 +1402,7 @@ extern "C" int lcba_solve(lcba_t* h, const lcba_options* opt_in, lcba_result* re
       if (h->fix_cameras) {
         // points only: the normal equations are block diagonal, p_p = (V + lam Dp^2)^-1 g_p
         KL(h, "point_factor", k_point_factor<<<nblk(h->P, 256), 256, 0, h->stream>>>(
-              h->d_Vg, h->d_scl_p, 0.0, h->d_ctl, h->P, h->d_Lz));
+              h->d_Vg, h->d_scl_p, 0.0, h->d_ctl, h->P, pt_mask(h), h->d_Lz));
         LCBA_CUDA(h, cudaMemsetAsync(h->d_pc, 0, (size_t)h->C * NCP * 8, h->stream));
         LCBA_CUDA(h, cudaMemsetAsync(h->d_fail, 0, 2 * sizeof(int), h->stream));
       } else {
@@ -1504,6 +1566,7 @@ extern "C" int lcba_linearize(lcba_t* h, double lam, double* S_out, double* rhs_
   LCBA_CUDA(h, cudaMemcpyAsync(h->d_ctl, &init, sizeof(Ctl), cudaMemcpyHostToDevice, h->stream));
   h->fix_cameras = 0;
   h->shared_intr = 0;
+  h->masks_on = false;
   LCBA_TRY(pass_linearize(h, 1));
   LCBA_TRY(pass_schur(h, &lam));
   const int n = h->C * NCP;
@@ -1928,11 +1991,21 @@ extern "C" int lcba_debug_step(lcba_t* h, double lam, double mu, int32_t mode, d
   LCBA_CUDA(h, cudaMemcpyAsync(h->d_ctl, &init, sizeof(Ctl), cudaMemcpyHostToDevice, h->stream));
   h->fix_cameras = mode == 1 ? 1 : 0;
   h->shared_intr = mode == 2 ? 1 : 0;
+  h->masks_on = true;
+  if (h->shared_intr && h->n_cam_held) {
+    set_error(h, "lcba_debug_step: a camera mask together with shared intrinsics is not supported");
+    return LCBA_E_UNSUPPORTED;
+  }
+  if ((h->fix_cameras ? 0 : (h->shared_intr ? 3 + 8LL * h->C : (long long)h->C * NCP - h->n_cam_held)) +
+          3 * (h->P - h->n_pt_held) <= 0) {
+    set_error(h, "lcba_debug_step: every parameter is held (lcba_set_fixed)");
+    return LCBA_E_ARG;
+  }
   LCBA_TRY(pass_linearize(h, 1));
   LCBA_TRY(pass_jdot(h));
   if (h->fix_cameras) {
     KL(h, "point_factor", k_point_factor<<<nblk(h->P, 256), 256, 0, h->stream>>>(
-          h->d_Vg, h->d_scl_p, lam, nullptr, h->P, h->d_Lz));
+          h->d_Vg, h->d_scl_p, lam, nullptr, h->P, pt_mask(h), h->d_Lz));
     LCBA_CUDA(h, cudaMemsetAsync(h->d_pc, 0, (size_t)h->C * NCP * 8, h->stream));
     LCBA_CUDA(h, cudaMemsetAsync(h->d_fail, 0, 2 * sizeof(int), h->stream));
   } else {
@@ -1971,9 +2044,10 @@ extern "C" int lcba_debug_i8_make(lcba_t* h, double lam, int32_t ref, int32_t re
   memset(&init, 0, sizeof(init));
   init.term = -1;
   LCBA_CUDA(h, cudaMemcpyAsync(h->d_ctl, &init, sizeof(Ctl), cudaMemcpyHostToDevice, h->stream));
+  h->masks_on = true;
   LCBA_TRY(pass_linearize(h, 1));
   KL(h, "point_factor", k_point_factor<<<nblk(h->P, 256), 256, 0, h->stream>>>(
-        h->d_Vg, h->d_scl_p, lam, nullptr, h->P, h->d_Lz));
+        h->d_Vg, h->d_scl_p, lam, nullptr, h->P, pt_mask(h), h->d_Lz));
   launch_i8_rowexp(h);
   if (poison >= 0) LCBA_CUDA(h, cudaMemsetAsync(h->d_i8planes, poison, h->i8plan.plane_bytes, h->stream));
   cudaEvent_t e0, e1;

@@ -207,15 +207,23 @@ __global__ void k_reduce_scalars(const double* __restrict__ part, int nblocks, i
 // ---- per-point scaling ---------------------------------------------------------------
 // scl[p][a] = first ? (sqrt(Vaa) or 1 if 0) : max(sqrt(Vaa), scl) ; gt = g / scl^2.
 // partial[block][0..3] sums: |g_h|^2, |x*scl|^2, |x|^2 ; [3] max |g|
+// A held point (pt_fixed[p] != 0; pt_fixed may be NULL) is a constant of the problem: scl = 1,
+// gt = 0, g_p in Vg set to 0 (so the back-substitution and lcba_get_grad see no gradient), and no
+// share of the norms.
 constexpr int PP_K = 4;
 __global__ void __launch_bounds__(256)
-k_point_prep(const double* __restrict__ Vg, const double* __restrict__ pts,
+k_point_prep(double* __restrict__ Vg, const double* __restrict__ pts,
              double* __restrict__ scl, double* __restrict__ gt, long long P, int first,
-             double* __restrict__ part) {
+             const uint8_t* __restrict__ pt_fixed, double* __restrict__ part) {
   __shared__ double s_red[32];
   double gh2 = 0, xs2 = 0, x2 = 0, gmax = 0;
   const long long stride = (long long)gridDim.x * blockDim.x;
   for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < P; p += stride) {
+    if (pt_fixed && pt_fixed[p]) {
+#pragma unroll
+      for (int a = 0; a < 3; ++a) { scl[3 * p + a] = 1.0; gt[3 * p + a] = 0.0; Vg[p * 9 + 6 + a] = 0.0; }
+      continue;
+    }
     const double* v = Vg + p * 9;
     const double d[3] = {v[0], v[3], v[5]};
 #pragma unroll
@@ -284,11 +292,19 @@ k_jdot(const double* __restrict__ tab, const double* __restrict__ pts,
 // (rank-deficient V; never produced by the reference's pipeline, get_points3d.py:52-56)
 // give finite numbers.  lam comes from the device control block (solver loop: no host round
 // trip) when `ctl` is given, from the argument otherwise (lcba_linearize debug tap).
+// A held point (pt_fixed[p] != 0; pt_fixed may be NULL) gets L^-1 = 0 and z = 0: its Y = W L^-T
+// vanishes, so it subtracts nothing from S, and its step L^-T L^-1 (.) is exactly 0.
 __global__ void __launch_bounds__(256)
 k_point_factor(const double* __restrict__ Vg, const double* __restrict__ scl, double lam,
-               const Ctl* __restrict__ ctl, long long P, double* __restrict__ Lz) {
+               const Ctl* __restrict__ ctl, long long P, const uint8_t* __restrict__ pt_fixed,
+               double* __restrict__ Lz) {
   const long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (p >= P) return;
+  if (pt_fixed && pt_fixed[p]) {
+#pragma unroll
+    for (int e = 0; e < 9; ++e) Lz[p * 9 + e] = 0.0;
+    return;
+  }
   if (ctl) lam = ctl->reg_term;
   const double* v = Vg + p * 9;
   const double s0 = scl[3 * p], s1 = scl[3 * p + 1], s2 = scl[3 * p + 2];

@@ -490,15 +490,25 @@ k_schur(const double* __restrict__ tab, const double* __restrict__ pts,
 
 // S (n x n, both triangles) = reduced blocks + lam * diag(scl_c^2) ; rhs = g_c + rhs_red.
 // lam: the device control block's reg_term when `ctl` is given, the argument otherwise.
+// A held camera entry (cam_fixed[i] != 0; cam_fixed may be NULL) turns row and column i into
+// those of the identity and rhs[i] into 0: dropping camera columns commutes with eliminating the
+// points, so the free block is the reduced system of the free parameters, and the Cholesky returns
+// an exact 0 for entry i (scl_c[i] = 1 there, so the retries' mu damping keeps the row diagonal).
 __global__ void k_assemble_S(const double* __restrict__ red, int C, int npairs,
                              const double* __restrict__ camsum, const double* __restrict__ scl_c,
-                             double lam, const Ctl* __restrict__ ctl, double* __restrict__ S,
+                             double lam, const Ctl* __restrict__ ctl,
+                             const uint8_t* __restrict__ cam_fixed, double* __restrict__ S,
                              double* __restrict__ rhs) {
   if (ctl) lam = ctl->reg_term;
   const int n = C * NCP;
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= (long long)n * n) return;
   const int r = (int)(idx / n), c = (int)(idx % n);
+  if (cam_fixed && (cam_fixed[r] || cam_fixed[c])) {
+    S[idx] = r == c ? 1.0 : 0.0;
+    if (r == c) rhs[r] = 0.0;
+    return;
+  }
   const int hi = max(r, c), lo = min(r, c);
   const int j = hi / NCP, a = hi % NCP, k = lo / NCP, b = lo % NCP;
   double v;

@@ -75,6 +75,45 @@ class BAResult(OptimizeResult):
         return (OptimizeResult, (dict(self),))
 
 
+def normalize_fixed(fixed_camera_params, fixed_points, n_cameras, n_points):
+    """The masks of ``bundleAdjust(fixed_camera_params=..., fixed_points=...)`` as (C, 11) and (P,)
+    bool arrays, or None where nothing is held.
+
+    fixed_camera_params: bool array of shape (11,) (the same entries of every camera) or (C, 11).
+    fixed_points: bool array of shape (P,) or an integer array of point indices in [0, P).
+    Raises ValueError on any other shape, dtype or index."""
+    cam = pt = None
+    if fixed_camera_params is not None:
+        m = np.asarray(fixed_camera_params)
+        if m.dtype != np.bool_:
+            raise ValueError("fixed_camera_params must be a bool array, got dtype %s" % m.dtype)
+        if m.shape == (N_CAM_PARAMS,):
+            m = np.broadcast_to(m, (n_cameras, N_CAM_PARAMS))
+        elif m.shape != (n_cameras, N_CAM_PARAMS):
+            raise ValueError("fixed_camera_params must have shape (11,) or (%d, 11), got %s"
+                             % (n_cameras, m.shape))
+        if m.any():
+            cam = np.ascontiguousarray(m)
+    if fixed_points is not None:
+        m = np.asarray(fixed_points)
+        if m.dtype == np.bool_:
+            if m.shape != (n_points,):
+                raise ValueError("a bool fixed_points must have shape (%d,), got %s" % (n_points, m.shape))
+        elif m.dtype.kind in "iu":
+            if m.ndim != 1:
+                raise ValueError("fixed_points indices must be a 1-D array, got shape %s" % (m.shape,))
+            if m.size and (m.min() < 0 or m.max() >= n_points):
+                raise ValueError("fixed_points indices must lie in [0, %d)" % n_points)
+            idx = m
+            m = np.zeros(n_points, dtype=bool)
+            m[idx] = True
+        else:
+            raise ValueError("fixed_points must be a bool mask or an integer index array, got dtype %s" % m.dtype)
+        if m.any():
+            pt = np.ascontiguousarray(m)
+    return cam, pt
+
+
 def _print_header():
     # scipy/optimize/_lsq/common.py:545-548
     print("{:^15}{:^15}{:^15}{:^15}{:^15}{:^15}".format(
@@ -238,15 +277,25 @@ class PySBA:
 
     # ---- solver (pySBA.py:132-147) ----
     def bundleAdjust(self, ftol=1e-4, xtol=1e-8, gtol=1e-8, max_nfev=None, verbose=2,
-                     profile=False, max_iterations=0, _fix_cameras=False, _shared=False):
+                     profile=False, max_iterations=0, _fix_cameras=False, _shared=False,
+                     fixed_camera_params=None, fixed_points=None):
         """Returns the bundle adjusted parameters (scipy ``OptimizeResult`` layout) and
         stores them on ``self.cameraArray`` / ``self.points3D``.
 
         The keyword defaults reproduce the reference call
         ``least_squares(fun, x0, jac_sparsity=A, verbose=2, x_scale='jac', ftol=ftol,
-        method='trf', jac='3-point')``."""
+        method='trf', jac='3-point')``.
+
+        ``fixed_camera_params`` (bool, shape (11,) for every camera or (C, 11)) and
+        ``fixed_points`` (bool, shape (P,), or integer point indices) hold those parameters at
+        their input values: the solve is scipy's ``trf_no_bounds`` on the free sub-vector (scaling,
+        trust radius, ``|x|`` and ``|g|_inf`` over free entries, ``max_nfev`` = 100 * free count).
+        ``x`` and ``jac`` keep the full layout, held entries of ``x`` equal the input bit for bit,
+        ``grad`` is 0 there.  Holding camera 0's extrinsics and three non-collinear points (or one
+        scale coordinate) removes the 7-dimensional gauge freedom."""
         numCameras = self.cameraArray.shape[0]
         numPoints = self.points3D.shape[0]
+        cam_fixed, pt_fixed = normalize_fixed(fixed_camera_params, fixed_points, numCameras, numPoints)
         cams0 = np.ascontiguousarray(self.cameraArray, dtype=np.float64)
         pts0 = np.ascontiguousarray(self.points3D, dtype=np.float64)
         if _shared:
@@ -285,11 +334,15 @@ class PySBA:
                 eng._comm_ready = True
             if verbose and rank != 0:
                 verbose = 0
+            pt_fixed_local = None if pt_fixed is None else pt_fixed[shard["lo"]:shard["hi"]]
         else:
             eng = self._ensure_problem(cams0, pts0, self.cameraIndices, self.point2DIndices,
                                        self.points2D, self._pointWeights)
             if not self._fresh_problem or _shared:   # observations already resident: new x0 only
                 eng.set_params(cams0, pts0)
+            pt_fixed_local = pt_fixed
+        if cam_fixed is not None or pt_fixed_local is not None or eng.has_fixed:
+            eng.set_fixed(cam_fixed, pt_fixed_local)
         t_in1 = _time.perf_counter()
         live = None
         if verbose == 2:
@@ -348,9 +401,20 @@ class PySBA:
         def lazy_fun():
             return engine_at_result().residuals(None, want_cost=False)[0]
 
+        held = None
+        if cam_fixed is not None or pt_fixed is not None:
+            held = np.zeros(nc + 3 * numPoints, dtype=bool)
+            if cam_fixed is not None and not _fix_cameras:
+                held[:nc] = cam_fixed.ravel()
+            if pt_fixed is not None:
+                held[nc:] = np.repeat(pt_fixed, 3)
+
         def lazy_grad():
             e = engine_at_result()
-            return e.grad() if e.generation == gen else e.linearize(1.0)["grad"]
+            g = e.grad() if e.generation == gen else e.linearize(1.0)["grad"]
+            if held is not None:       # the unmasked tap on a re-uploaded problem: held entries -> 0
+                g[held] = 0.0
+            return g
 
         # wall-clock split of this call: ingest (H2D + validate/sort/narrow/CSR + plans), solve, results D2H
         self.last_timing = dict(ingest_ms=(t_in1 - t_in0) * 1e3, solve_wall_ms=(t_sol - t_in1) * 1e3,
