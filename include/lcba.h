@@ -314,6 +314,13 @@ int lcba_debug_i8_cover_plan(int32_t C, int64_t P, int32_t sm_count, int32_t whi
                              int32_t max_tiles, int32_t* work_out, int32_t max_work, int32_t* nwork_out,
                              int32_t* nrg_out, int64_t* nkb_out, int32_t* cover_out, double* model_out);
 
+/* Host-only: the K blocks every CTA of a tile plan (which as above) reads, under the K-major schedule (kmajor = 1, the
+ * default) or one contiguous K range per CTA (kmajor = 0, LCBA_I8_SCHED=range).  work_out: per CTA 6 ints (tile,
+ * kb0, kb1, kfirst, kc, kstride): the K blocks kfirst + (i / kc) kstride + i % kc for i < kb1 - kb0.  *window_out:
+ * how many K blocks a CTA may run ahead of the slowest one (0: no window).  Returns the number of CTAs. */
+int lcba_debug_i8_schedule(int32_t C, int64_t P, int32_t sm_count, int32_t which, int32_t kmajor, int32_t* work_out,
+                           int32_t max_work, int32_t* window_out);
+
 /* 1 when the last Schur pass of the int8 tensor-core path found a camera row whose largest |Y| entry is more
  * than 4x the square root of its Schur diagonal (finer than the 48-bit digits resolve) and recomputed the
  * pass with the FP64 DMMA kernel; 0 when the int8 result stood; -1 when the handle does not use the int8

@@ -23,7 +23,7 @@ SYMBOLS = ["lcba_version", "lcba_create", "lcba_destroy", "lcba_last_error", "lc
            "lcba_sq_normal", "lcba_debug_schur_stats", "lcba_debug_mma_plan",
            "lcba_set_iteration_callback", "lcba_debug_i8_plan", "lcba_host_is_nondecreasing_i64", "lcba_debug_peer_reduce",
            "lcba_debug_i8_fallback", "lcba_debug_chol", "lcba_debug_step", "lcba_debug_i8_cover_plan",
-           "lcba_debug_i8_make", "lcba_set_fixed"]
+           "lcba_debug_i8_make", "lcba_set_fixed", "lcba_debug_i8_schedule"]
 
 # scalars_out of lcba_debug_step, in order (include/lcba.h)
 STEP_SCALARS = ["reg_term", "Delta", "Jg2", "aa", "ab", "bb", "JAA", "JAB", "JBB", "gtgt", "gtp", "pp",
@@ -116,6 +116,7 @@ def load():
     lib.lcba_debug_i8_plan.argtypes = [i32, i64, i32, vp, i32, vp, i32, C.POINTER(i32), C.POINTER(i32), C.POINTER(i64)]
     lib.lcba_debug_i8_cover_plan.argtypes = [i32, i64, i32, i32, vp, i32, vp, i32, C.POINTER(i32), C.POINTER(i32),
                                              C.POINTER(i64), C.POINTER(i32), vp]
+    lib.lcba_debug_i8_schedule.argtypes = [i32, i64, i32, i32, i32, vp, i32, C.POINTER(i32)]
     lib.lcba_host_is_nondecreasing_i64.argtypes = [vp, i64, i32]
     lib.lcba_debug_peer_reduce.argtypes = [vp, i32]
     lib.lcba_debug_i8_fallback.argtypes = [vp]
@@ -384,6 +385,21 @@ class Engine:
         return dict(tiles=tiles[:nt].copy(), work=work[:nwork.value].copy(), nrg=nrg.value, nkb=nkb.value,
                     cover=bool(cover.value), executed_ops=model[0], cycles=model[1], strip_cycles=model[2],
                     cover_cycles=model[3])
+
+    @staticmethod
+    def i8_schedule(n_cams, P, sm_count, which=0, kmajor=True):
+        """The K blocks every CTA of a tile plan of the int8 Schur kernel reads (lcba_debug_i8_schedule, host
+        only): dict of work (CTAs, 6) int32 [tile, kb0, kb1, kfirst, kc, kstride] -- the K blocks
+        kfirst + (i // kc) kstride + i % kc for i < kb1 - kb0 -- and window (K blocks a CTA may run ahead of
+        the slowest one; 0 without a window).  kmajor=False: one contiguous range per CTA (LCBA_I8_SCHED=range)."""
+        lib = load()
+        work = np.zeros((1024, 6), dtype=np.int32)
+        window = C.c_int32()
+        n = lib.lcba_debug_i8_schedule(int(n_cams), int(P), int(sm_count), int(which), int(bool(kmajor)), _ptr(work),
+                                       work.shape[0], C.byref(window))
+        if n < 0:
+            raise LcbaError(n, "lcba_debug_i8_schedule: bad arguments")
+        return dict(work=work[:n].copy(), window=window.value)
 
     def debug_chol(self, A, rhs, mu=0.0, d=None, grid=0):
         """The solver's dense camera solve on a host system (lcba_debug_chol): returns (x, factor, fail)

@@ -121,6 +121,7 @@ struct lcba_handle {
   I8Maps i8maps;
   I8Plan i8plan;
   I8Work* d_i8work = nullptr;
+  unsigned long long* d_i8progress = nullptr;   // k_i8_syrk's window: one slot per CTA (zeroed once)
   I8Tile* d_i8tiles = nullptr;
   unsigned char* d_i8planes = nullptr;
   double *d_i8partial = nullptr, *d_i8rmax = nullptr;
@@ -609,10 +610,12 @@ extern "C" int lcba_set_problem_shard(lcba_t* h, int32_t C, int64_t P, int64_t N
       }
       if (h->use_i8) {
         {
-          // LCBA_I8_PLAN=strip|cover overrides the cost model's choice of tile plan
+          // LCBA_I8_PLAN=strip|cover overrides the cost model's choice of tile plan; LCBA_I8_SCHED=range gives each
+          // CTA one contiguous K range instead of the K-major schedule (A/B runs, tests)
           const char* pe = getenv("LCBA_I8_PLAN");
           const int which = !pe ? 0 : (strcmp(pe, "strip") == 0 ? 1 : (strcmp(pe, "cover") == 0 ? 2 : 0));
-          h->i8plan = make_i8_best_plan(C, P, h->sm_count, which);
+          const char* se = getenv("LCBA_I8_SCHED");
+          h->i8plan = make_i8_best_plan(C, P, h->sm_count, which, !(se && strcmp(se, "range") == 0));
         }
         const I8Plan& ip = h->i8plan;
         h->i8_groups = (C + I8_GROUP_CAMS - 1) / I8_GROUP_CAMS;
@@ -623,6 +626,8 @@ extern "C" int lcba_set_problem_shard(lcba_t* h, int32_t C, int64_t P, int64_t N
         LCBA_TRY(dev_alloc(h, &h->d_i8tiles, ip.tiles.size()));
         LCBA_CUDA(h, cudaMemcpyAsync(h->d_i8work, ip.work.data(), ip.work.size() * sizeof(I8Work), cudaMemcpyHostToDevice, st));
         LCBA_CUDA(h, cudaMemcpyAsync(h->d_i8tiles, ip.tiles.data(), ip.tiles.size() * sizeof(I8Tile), cudaMemcpyHostToDevice, st));
+        LCBA_TRY(dev_alloc(h, &h->d_i8progress, ip.work.size()));
+        LCBA_CUDA(h, cudaMemsetAsync(h->d_i8progress, 0, ip.work.size() * sizeof(unsigned long long), st));
         LCBA_TRY(dev_alloc(h, &h->d_i8planes, ip.plane_bytes));
         {
           const char* te = getenv("LCBA_I8_TMA");
@@ -1044,10 +1049,12 @@ static int pass_schur(lcba_t* h, const double* lam_host_or_null) {
       launch_i8_make(h, false);
       if (h->i8_tma)
         KL(h, "schur", k_i8_syrk<true><<<(unsigned)ip.work.size(), I8_THREADS, ip.smem_bytes, h->stream>>>(
-              h->i8maps, h->d_i8planes, ip.NRG, h->d_i8work, h->d_i8partial, h->d_fail, h->d_stats));
+              h->i8maps, h->d_i8planes, ip.NRG, h->d_i8work, h->d_i8partial, h->d_fail, h->d_i8progress, ip.window,
+              h->d_stats));
       else
         KL(h, "schur", k_i8_syrk<false><<<(unsigned)ip.work.size(), I8_THREADS, ip.smem_bytes, h->stream>>>(
-              h->i8maps, h->d_i8planes, ip.NRG, h->d_i8work, h->d_i8partial, h->d_fail, h->d_stats));
+              h->i8maps, h->d_i8planes, ip.NRG, h->d_i8work, h->d_i8partial, h->d_fail, h->d_i8progress, ip.window,
+              h->d_stats));
       KL(h, "schur_reduce", k_i8_gather<<<dim3((unsigned)ip.tiles.size(), 16), 256, 0, h->stream>>>(
             h->d_i8partial, h->d_i8tiles, C, ip.cover ? 1 : 0, h->d_i8erow, pl.npairs, h->d_Sred));
       KL(h, "schur_reduce", k_add_cam_blocks<<<nblk(C * 121, 128), 128, 0, h->stream>>>(h->d_U, C, h->d_Sred));
@@ -1839,6 +1846,25 @@ extern "C" int lcba_debug_i8_cover_plan(int32_t C, int64_t P, int32_t sm_count, 
     model_out[3] = make_i8_cover_plan(C, P, sm_count).model_cycles;
   }
   return (int)pl.tiles.size();
+}
+
+// host-only test hook: the K blocks of every CTA of a tile plan under a schedule (kmajor: 1 = K-major, the default;
+// 0 = one contiguous range per CTA, LCBA_I8_SCHED=range).  work_out: per CTA 6 ints (tile, kb0, kb1, kfirst, kc,
+// kstride): the K blocks kfirst + (i / kc) kstride + i % kc, i < kb1 - kb0.  *window_out: the window in K blocks.
+// Returns the number of CTAs.
+extern "C" int lcba_debug_i8_schedule(int32_t C, int64_t P, int32_t sm_count, int32_t which, int32_t kmajor,
+                                      int32_t* work_out, int32_t max_work, int32_t* window_out) {
+  if (C < 1 || C > LCBA_MAX_CAMERAS || P < 1 || sm_count < 1 || which < 0 || which > 2 || !work_out) return LCBA_E_ARG;
+  const I8Plan pl = make_i8_best_plan(C, P, sm_count, which, kmajor != 0);
+  for (size_t i = 0; i < pl.work.size() && (int)i < max_work; ++i) {
+    const I8Work& w = pl.work[i];
+    int ti = 0;
+    while (ti + 1 < (int)pl.tiles.size() && pl.tiles[ti + 1].w0 <= (int)i) ++ti;
+    int32_t* o = work_out + 6 * i;
+    o[0] = ti; o[1] = w.kb0; o[2] = w.kb1; o[3] = w.kfirst; o[4] = w.kc; o[5] = w.kstride;
+  }
+  if (window_out) *window_out = pl.window;
+  return (int)pl.work.size();
 }
 
 // ---- squared-residual variants (pySBA.py:151-206): cost, J^T f, J^T J in one pass ----------

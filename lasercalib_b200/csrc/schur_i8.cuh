@@ -19,8 +19,9 @@
 //                   2 k-steps: all six slices of A (4-D, or 5-D for two row ranges), B1, B2; fallback: one 1-D
 //                   bulk copy per lane), warp 5 MMA issuer (elect.sync, compile-time MMA plan: slice i of the
 //                   rows against slices 0..6-i of the columns in ONE instruction, N <= 256, A kept in the
-//                   collector, widest last); tiles from the strip or the cover plan, K ranges per tile weighted
-//                   by the measured cost of a K block (i8_deal)
+//                   collector, widest last); tiles from the strip or the cover plan, CTAs per tile weighted
+//                   by the measured cost of a K block, K blocks dealt K-major in chunks so that all tiles read a
+//                   K block at about the same time, a progress window between the CTAs (i8_deal)
 //   k_i8_gather   : per-CTA partials -> the pair-block layout of Sred (fixed order, no atomics)
 //   k_i8_check    : resolution guard: rows whose maximum lies far above their Schur diagonal hand the pass to
 //                   the DMMA kernel (k_schur_mma, gated) and k_i8_fallback_finish
@@ -44,16 +45,22 @@ constexpr int I8_RG_BYTES = 512;          // one row group of one slice of one K
 constexpr int I8_GROUP_CAMS = 8;          // cameras per k_i8_make block: 88 rows = 11 row groups exactly
 constexpr int I8_GROUP_RG = 13;           // row groups of the last group at most: 8 cameras + z + even padding
 constexpr int I8_GROUP_ROWS = I8_GROUP_RG * 8;
+constexpr int I8_KC = 8;                  // K blocks per chunk of the K-major schedule (0.8 MB of planes at 24 cameras)
+constexpr size_t I8_WINDOW_BYTES = 32u << 20;   // planes between the slowest and the fastest CTA of k_i8_syrk
+constexpr int I8_POLL_CAP = 2048;         // window polls after which a CTA stops waiting for the others
 
 // One CTA of k_i8_syrk: rows = row groups [m_rg0, m_rg0 + m_nrg) and, optionally, a second range
 // [m2_rg0, +m2_nrg) stacked below them (the A operand, <= 16 row groups in all), columns = block 1
 // [n_rg0, +n_nrg) and, optionally, block 2 [n2_rg0, +n2_nrg): the few rows left over behind the last full
 // 128-row tile of the strip plan, handled as COLUMNS (the tile entry is S[column][row]); n_nrg + n2_nrg <= 8.
 // In the partial tile [128][64] block 1 occupies columns [0, 8 n_nrg), block 2 the LAST 8 n2_nrg columns.
+// The K blocks of a CTA: positions [kb0, kb1) of its tile's K order, i.e. the K blocks
+// kfirst + (i / kc) kstride + i % kc for i < kb1 - kb0 (runs of kc K blocks, kstride apart).
 struct I8Work {
   int m_rg0, m_nrg, m2_rg0, m2_nrg, n_rg0, n_nrg, n2_rg0, n2_nrg;
-  int kb0, kb1;                           // K blocks [kb0, kb1)
-  int map_a, map_b1, map_b2, pad;         // tensor-map index of the three operand loads
+  int kb0, kb1;
+  int map_a, map_b1, map_b2;              // tensor-map index of the three operand loads
+  int kfirst, kc, kstride;
 };
 // TMA tensor maps over the digit planes, one per (box height, range distance) that the plan uses.
 // delta = 0: a 4-D tensor (128 u32 = one 512-byte row group, NRG row groups, 6 digits, K blocks); a box of
@@ -74,6 +81,8 @@ struct I8Plan {
   int map_delta[I8_MAX_MAPS] = {};                     // 0: one range; > 0: two ranges this many row groups apart
   int nmaps = 0;                                       // > I8_MAX_MAPS: too many shapes, use 1-D bulk copies
   bool cover = false;                                  // made by make_i8_cover_plan
+  bool kmajor = true;                                  // K-major schedule (else one contiguous K range per CTA)
+  int window = 0;                                      // K-major: K blocks a CTA may run ahead of the slowest
   double model_cycles = 0.0;                           // slowest CTA in the cost model (MMA-warp cycles)
   std::vector<I8Tile> tiles;
   std::vector<I8Work> work;
@@ -89,10 +98,18 @@ inline double i8_block_cost(int nrg) {
 }
 inline double i8_tile_cost(const I8Tile& t) { return 507.0 + i8_block_cost(t.n_nrg) + i8_block_cost(t.n2_nrg); }
 
-// K ranges per tile: one CTA per SM in total, dealt so that the slowest tile finishes as early as possible
+// CTAs per tile: one CTA per SM in total, dealt so that the slowest tile finishes as early as possible
 // (greedy over the cost model; the first version gave every main tile the same number of ranges: the tile that
-// carries a second column block was 13 % slower than the rest and set the kernel's time).  Fills pl.work, the
-// tensor-map shapes, the buffer sizes and the model's slowest-CTA cycles.
+// carries a second column block was 13 % slower than the rest and set the kernel's time).  The K blocks of a
+// tile's n CTAs:
+//   - range schedule (kmajor = false): CTA q takes the contiguous range [nkb q / n, nkb (q + 1) / n).  CTAs of
+//     tiles with different n read different K blocks at any moment, so only tiles with the same n share their
+//     operands through L2 (ring24 x 1 M: 13.9 GB of DRAM reads for 5.0 GB of planes, strip plan);
+//   - K-major schedule: the K blocks form chunks of kc = I8_KC; CTA q takes the chunks j = q mod n in
+//     increasing j.  n is roughly proportional to a tile's cost per K block, so every tile sweeps K at about
+//     the same rate and all tiles read a chunk at about the same time; k_i8_syrk's window bounds the drift
+//     that the rounding of the deal leaves (up to 4.5 % at 24 cameras: 2100 K blocks by the end of a launch).
+// Fills pl.work, the tensor-map shapes, the buffer sizes, the window and the model's slowest-CTA cycles.
 inline void i8_deal(I8Plan& pl, int sm_count) {
   std::vector<double> cost(pl.tiles.size());
   std::vector<long long> nr(pl.tiles.size(), 1);
@@ -108,6 +125,7 @@ inline void i8_deal(I8Plan& pl, int sm_count) {
     ++nr[worst];
   }
   pl.model_cycles = 0.0;
+  long long spread = 0;                                     // K-major: K blocks between a tile's first and last CTA
   for (size_t ti = 0; ti < pl.tiles.size(); ++ti) {
     I8Tile& t = pl.tiles[ti];
     const long long n = std::min<long long>(nr[ti], pl.nkb);
@@ -121,19 +139,43 @@ inline void i8_deal(I8Plan& pl, int sm_count) {
       return pl.nmaps++;
     };
     const int ma = map_of(t.m_nrg, t.m2_nrg > 0 ? t.m2_rg0 - t.m_rg0 : 0), mb1 = map_of(t.n_nrg, 0), mb2 = map_of(t.n2_nrg, 0);
+    // kc <= nkb / n: every CTA gets at least one chunk
+    const long long kc = pl.kmajor ? std::max(1LL, std::min<long long>(I8_KC, pl.nkb / n)) : 0;
+    const long long nch = pl.kmajor ? (pl.nkb + kc - 1) / kc : 0;
+    long long pos = 0, most = 0;
     for (long long q = 0; q < n; ++q) {
-      I8Work w{t.m_rg0, t.m_nrg, t.m2_rg0, t.m2_nrg, t.n_rg0, t.n_nrg, t.n2_rg0, t.n2_nrg,
-               (int)(pl.nkb * q / n), (int)(pl.nkb * (q + 1) / n), ma, mb1, mb2, 0};
+      I8Work w{t.m_rg0, t.m_nrg, t.m2_rg0, t.m2_nrg, t.n_rg0, t.n_nrg, t.n2_rg0, t.n2_nrg, 0, 0, ma, mb1, mb2, 0, 0, 0};
+      long long cnt;
+      if (pl.kmajor) {
+        cnt = ((nch - 1 - q) / n + 1) * kc - ((nch - 1) % n == q ? nch * kc - pl.nkb : 0);   // the last chunk may be short
+        w.kfirst = (int)(q * kc);
+        w.kc = (int)kc;
+        w.kstride = (int)(n * kc);
+      } else {
+        cnt = pl.nkb * (q + 1) / n - pl.nkb * q / n;
+        w.kfirst = (int)(pl.nkb * q / n);
+        w.kc = (int)std::max(1LL, cnt);
+      }
+      w.kb0 = (int)pos;
+      w.kb1 = (int)(pos + cnt);
+      pos += cnt;
+      most = std::max(most, cnt);
       pl.work.push_back(w);
     }
-    pl.model_cycles = std::max(pl.model_cycles, cost[ti] * (double)((pl.nkb + n - 1) / n));
+    pl.model_cycles = std::max(pl.model_cycles, cost[ti] * (double)most);
+    spread = std::max(spread, n * kc);
   }
+  // the window: about I8_WINDOW_BYTES of planes, and at least twice the spread of the CTAs of one tile, which
+  // are that far apart by construction
+  const long long kb_bytes = (long long)I8_NS * pl.NRG * I8_RG_BYTES;
+  pl.window = pl.kmajor ? (int)std::min(pl.nkb, std::max((long long)(I8_WINDOW_BYTES / kb_bytes), 2 * spread)) : 0;
   pl.plane_bytes = (size_t)pl.nkb * I8_NS * pl.NRG * I8_RG_BYTES;
   pl.smem_bytes = (size_t)I8_STAGES * I8_NS * (16 + 8) * I8_RG_BYTES + 1024;
 }
 
-inline I8Plan i8_plan_base(int C, long long P) {
+inline I8Plan i8_plan_base(int C, long long P, bool kmajor) {
   I8Plan pl;
+  pl.kmajor = kmajor;
   pl.C = C;
   pl.R = NCP * C + 1;
   pl.NRG = (pl.R + 7) / 8;
@@ -150,8 +192,8 @@ inline I8Plan i8_plan_base(int C, long long P) {
 // 8 - last row groups wide so that block 1 + block 2 <= 64 columns (7 anti-diagonals x 64 = 448 TMEM columns).
 // (First version: separate 16-column tiles with their own K ranges streamed K positions nobody else was
 // reading: 40 % of the kernel's DRAM traffic for 11 % of its work, ncu r02.)
-inline I8Plan make_i8_plan(int C, long long P, int sm_count) {
-  I8Plan pl = i8_plan_base(C, P);
+inline I8Plan make_i8_plan(int C, long long P, int sm_count, bool kmajor = true) {
+  I8Plan pl = i8_plan_base(C, P, kmajor);
   const int NRG = pl.NRG;
   const int nmt = (NRG + 15) / 16;
   const int last_m = NRG - 16 * (nmt - 1);
@@ -188,8 +230,8 @@ inline I8Plan make_i8_plan(int C, long long P, int sm_count) {
 // (<= 48 columns): its triangle rides with the last group (one contiguous range), the other groups go two at a
 // time.  k_i8_gather keeps each entry once: inside I and J both (the square of z) only rho >= sig.
 // 24 cameras (NRG = 34, G = 4): 8 tiles, 13 582 model cycles per K block against 16 517 for the strip plan.
-inline I8Plan make_i8_cover_plan(int C, long long P, int sm_count) {
-  I8Plan pl = i8_plan_base(C, P);
+inline I8Plan make_i8_cover_plan(int C, long long P, int sm_count, bool kmajor = true) {
+  I8Plan pl = i8_plan_base(C, P, kmajor);
   pl.cover = true;
   const int G = pl.NRG / 8, r = pl.NRG - 8 * G;
   std::vector<std::vector<int>> to(G);                  // to[z]: the groups x whose pair {x, z} has columns z
@@ -226,12 +268,12 @@ inline I8Plan make_i8_cover_plan(int C, long long P, int sm_count) {
 }
 
 // The plan k_i8_syrk runs: the cover plan where the cost model puts its slowest CTA below the strip plan's.
-// which: 0 = by the model, 1 = strip, 2 = cover (LCBA_I8_PLAN).
-inline I8Plan make_i8_best_plan(int C, long long P, int sm_count, int which) {
-  if (which == 1) return make_i8_plan(C, P, sm_count);
-  I8Plan cv = make_i8_cover_plan(C, P, sm_count);
+// which: 0 = by the model, 1 = strip, 2 = cover (LCBA_I8_PLAN); kmajor: the schedule (LCBA_I8_SCHED=range: false).
+inline I8Plan make_i8_best_plan(int C, long long P, int sm_count, int which, bool kmajor = true) {
+  if (which == 1) return make_i8_plan(C, P, sm_count, kmajor);
+  I8Plan cv = make_i8_cover_plan(C, P, sm_count, kmajor);
   if (which == 2) return cv;
-  I8Plan st = make_i8_plan(C, P, sm_count);
+  I8Plan st = make_i8_plan(C, P, sm_count, kmajor);
   return cv.model_cycles < st.model_cycles ? cv : st;
 }
 
@@ -921,12 +963,36 @@ __device__ __forceinline__ void i8_issue_block(bool first, uint32_t tmem, uint32
   }
 }
 
-// partial[cta][128][64] doubles: sum_d 2^-8(d+2) D_d  (row exponents are applied by k_i8_gather)
+// ------------------------------------------------------------------------------ the window of the K-major schedule
+// progress[cta] = (launch epoch << 32) | the first K block of the chunk the CTA's producer loads, or I8_DONE once it
+// has loaded its last one.  The epoch is the CTA's own slot's epoch + 1 (every CTA publishes in every launch, the
+// array is zeroed once at allocation), so a slot still holding the previous launch's value reads as "not started"
+// and graph replays need no memset.  The window only keeps the CTAs' reads close enough for L2 to serve them:
+// no data passes through it, so relaxed accesses suffice, and a CTA that has polled I8_POLL_CAP times stops
+// waiting for the rest of the launch (CTAs need not be co-resident for the kernel to finish).
+constexpr unsigned I8_DONE = 0x7fffffffu;
+__device__ __forceinline__ void i8_progress_put(unsigned long long* p, unsigned long long v) {
+  asm volatile("st.relaxed.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
+}
+// warp-collective: the smallest position of this launch over all CTAs (-1: a CTA that has not started)
+__device__ __forceinline__ int i8_progress_min(const unsigned long long* progress, int nctas, unsigned epoch, int lane) {
+  int m = 0x7fffffff;
+  for (int i = lane; i < nctas; i += 32) {
+    unsigned long long v;
+    asm volatile("ld.relaxed.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(progress + i) : "memory");
+    m = min(m, (unsigned)(v >> 32) == epoch ? (int)(unsigned)v : -1);
+  }
+  return __reduce_min_sync(0xffffffffu, m);
+}
+
+// partial[cta][128][64] doubles: sum_d 2^-8(d+2) D_d  (row exponents are applied by k_i8_gather).
+// window > 0: the K-major schedule's window in K blocks over progress[gridDim.x]; 0: no window.
 template <bool TMA>
 __global__ void __launch_bounds__(I8_THREADS, 1)
 k_i8_syrk(const __grid_constant__ I8Maps maps, const unsigned char* __restrict__ planes, int NRG,
           const I8Work* __restrict__ work, double* __restrict__ partial, int* __restrict__ fail,
-          long long* __restrict__ stats /* null, or per CTA: MMA warp (waiting at FULL, total), producer (waiting at EMPTY, total) cycles */) {
+          unsigned long long* __restrict__ progress, int window,
+          long long* __restrict__ stats /* null, or per CTA: MMA warp (waiting at FULL, total), producer (waiting for the window, total) cycles */) {
   extern __shared__ __align__(1024) uint8_t i8_smem[];
   __shared__ __align__(8) uint64_t s_bar[2 * I8_STAGES + 2];
   __shared__ uint32_t s_tmem;
@@ -959,40 +1025,52 @@ k_i8_syrk(const __grid_constant__ I8Maps maps, const unsigned char* __restrict__
   const int nkb = W.kb1 - W.kb0;
 
   if (wid == 4) {
-    if (TMA) {
-      // ---- producer, TMA: one tensor copy per operand (all six digits of A / B1 / B2), issued by one lane
-      if (lane == 0) {
-        for (int it = 0; it < nkb; ++it) {
-          const int st = it % I8_STAGES;
-          if (it >= I8_STAGES) i8_mbar_wait<false>(bar_empty + 8 * st, ((it / I8_STAGES) - 1) & 1, fail);
-          i8_mbar_expect_tx(bar_full + 8 * st, (uint32_t)I8_NS * (a_bytes + b_bytes + b2_bytes));
-          const uint32_t dstA = smem0 + st * STAGE_BYTES, dstB = dstA + A_REGION;
-          const int kb = W.kb0 + it;
+    // ---- producer: TMA, one tensor copy per operand (all six digits of A / B1 / B2) issued by lane 0; or 1-D bulk
+    // copies, one per lane: (digit, operand) = A range 1, A range 2, B of block 1, B of block 2.  The whole warp
+    // keeps the window.
+    const int ci = lane / 4, cb = lane - 4 * ci;
+    const bool mine = TMA ? lane == 0 : lane < 4 * I8_NS && (cb == 0 || cb == 2 || (cb == 1 && W.m2_nrg > 0) || (cb == 3 && W.n2_nrg > 0));
+    const long long t_begin = stats ? clock64() : 0;
+    long long t_window = 0;
+    unsigned epoch = 0;
+    if (window > 0) epoch = __shfl_sync(0xffffffffu, lane == 0 ? (unsigned)(progress[blockIdx.x] >> 32) + 1u : 0u, 0);
+    int lo = -1, polls = 0;                                   // lo: the slowest CTA's position as last seen
+    for (int it = 0; it < nkb; ++it) {
+      const int st = it % I8_STAGES;
+      const int kb = W.kfirst + (it / W.kc) * W.kstride + it % W.kc;
+      if (window > 0 && it % W.kc == 0) {
+        if (lane == 0) i8_progress_put(progress + blockIdx.x, ((unsigned long long)epoch << 32) | (unsigned)kb);
+        if (kb - window > lo && polls < I8_POLL_CAP) {
+          const long long w0 = clock64();
+          while (true) {
+            lo = i8_progress_min(progress, gridDim.x, epoch, lane);
+            if (kb - window <= lo || ++polls == I8_POLL_CAP) break;
+            __nanosleep(256);
+          }
+          t_window += clock64() - w0;
+        }
+      }
+      if (it >= I8_STAGES && (TMA ? lane == 0 : true)) i8_mbar_wait<false>(bar_empty + 8 * st, ((it / I8_STAGES) - 1) & 1, fail);
+      if (lane == 0) i8_mbar_expect_tx(bar_full + 8 * st, (uint32_t)I8_NS * (a_bytes + b_bytes + b2_bytes));
+      __syncwarp();
+      if (mine) {
+        const uint32_t dstA = smem0 + st * STAGE_BYTES, dstB = dstA + A_REGION;
+        if (TMA) {
           if (W.m2_nrg > 0) i8_tma_5d(dstA, &maps.m[W.map_a], 0, W.m_rg0, 0, 0, kb, bar_full + 8 * st);
           else i8_tma_4d(dstA, &maps.m[W.map_a], 0, W.m_rg0, 0, kb, bar_full + 8 * st);
           i8_tma_4d(dstB, &maps.m[W.map_b1], 0, W.n_rg0, 0, kb, bar_full + 8 * st);
           if (W.n2_nrg > 0) i8_tma_4d(dstB + B2_OFF, &maps.m[W.map_b2], 0, W.n2_rg0, 0, kb, bar_full + 8 * st);
+        } else {
+          const unsigned char* src = planes + (size_t)kb * I8_NS * NRG * I8_RG_BYTES + (size_t)ci * NRG * I8_RG_BYTES;
+          if (cb == 0) i8_bulk_g2s(dstA + ci * a_bytes, src + (size_t)W.m_rg0 * I8_RG_BYTES, a1_bytes, bar_full + 8 * st);
+          else if (cb == 1) i8_bulk_g2s(dstA + ci * a_bytes + a1_bytes, src + (size_t)W.m2_rg0 * I8_RG_BYTES, a_bytes - a1_bytes, bar_full + 8 * st);
+          else if (cb == 2) i8_bulk_g2s(dstB + ci * b_bytes, src + (size_t)W.n_rg0 * I8_RG_BYTES, b_bytes, bar_full + 8 * st);
+          else i8_bulk_g2s(dstB + B2_OFF + ci * b2_bytes, src + (size_t)W.n2_rg0 * I8_RG_BYTES, b2_bytes, bar_full + 8 * st);
         }
       }
-    } else {
-    // ---- producer, 1-D bulk copies: one per lane: (digit, operand) = A range 1, A range 2, B of block 1, B of block 2
-    const int ci = lane / 4, cb = lane - 4 * ci;
-    const bool mine = lane < 4 * I8_NS && (cb == 0 || cb == 2 || (cb == 1 && W.m2_nrg > 0) || (cb == 3 && W.n2_nrg > 0));
-    for (int it = 0; it < nkb; ++it) {
-      const int st = it % I8_STAGES;
-      if (it >= I8_STAGES) i8_mbar_wait<false>(bar_empty + 8 * st, ((it / I8_STAGES) - 1) & 1, fail);
-      if (lane == 0) i8_mbar_expect_tx(bar_full + 8 * st, (uint32_t)I8_NS * (a_bytes + b_bytes + b2_bytes));
-      __syncwarp();
-      if (mine) {
-        const unsigned char* src = planes + (size_t)(W.kb0 + it) * I8_NS * NRG * I8_RG_BYTES + (size_t)ci * NRG * I8_RG_BYTES;
-        const uint32_t dstA = smem0 + st * STAGE_BYTES, dstB = dstA + A_REGION;
-        if (cb == 0) i8_bulk_g2s(dstA + ci * a_bytes, src + (size_t)W.m_rg0 * I8_RG_BYTES, a1_bytes, bar_full + 8 * st);
-        else if (cb == 1) i8_bulk_g2s(dstA + ci * a_bytes + a1_bytes, src + (size_t)W.m2_rg0 * I8_RG_BYTES, a_bytes - a1_bytes, bar_full + 8 * st);
-        else if (cb == 2) i8_bulk_g2s(dstB + ci * b_bytes, src + (size_t)W.n_rg0 * I8_RG_BYTES, b_bytes, bar_full + 8 * st);
-        else i8_bulk_g2s(dstB + B2_OFF + ci * b2_bytes, src + (size_t)W.n2_rg0 * I8_RG_BYTES, b2_bytes, bar_full + 8 * st);
-      }
     }
-    }
+    if (window > 0 && lane == 0) i8_progress_put(progress + blockIdx.x, ((unsigned long long)epoch << 32) | I8_DONE);
+    if (stats && lane == 0) { stats[4 * blockIdx.x + 2] = t_window; stats[4 * blockIdx.x + 3] = clock64() - t_begin; }
   } else if (wid == 5) {
     // ---- MMA issuer: the highest warp id of its scheduler; one elected lane
     if (i8_elect_one()) {

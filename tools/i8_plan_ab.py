@@ -1,10 +1,12 @@
-"""A/B of the two tile plans of the int8 Schur SYRK (schur_i8.cuh: strip and cover) on one GPU, alternating
-inside one process: per round and plan, the device time of K solver iterations and the CUDA-event time of
-k_i8_syrk per launch (the "schur" entry of the solver's profile), plus the card's name and power limit.
+"""A/B of two settings of the int8 Schur SYRK on one GPU, alternating inside one process: by default its two tile
+plans (LCBA_I8_PLAN=strip,cover), or any other switch such as its two schedules (LCBA_I8_SCHED=range,kmajor).
+Per round and setting, the device time of K solver iterations and the CUDA-event time of k_i8_syrk per launch
+(the "schur" entry of the solver's profile), plus the card's name and power limit.
 
-    python tools/i8_plan_ab.py OUT_DIR [rig] [points] [rounds] [steps]
+    python tools/i8_plan_ab.py OUT_DIR [rig] [points] [rounds] [steps] [VAR=a,b]
 
-Writes OUT_DIR/i8_plan_ab.json and prints a summary (median and range per plan)."""
+Writes OUT_DIR/i8_plan_ab.json (OUT_DIR/<var>_ab.json for another switch) and prints a summary (median and
+range per setting)."""
 import json
 import os
 import subprocess
@@ -32,6 +34,8 @@ def main():
     points = int(sys.argv[3]) if len(sys.argv) > 3 else 1_000_000
     rounds = int(sys.argv[4]) if len(sys.argv) > 4 else 4
     steps = int(sys.argv[5]) if len(sys.argv) > 5 else 20
+    var, vals = (sys.argv[6] if len(sys.argv) > 6 else "LCBA_I8_PLAN=strip,cover").split("=")
+    vals = tuple(vals.split(","))
     os.makedirs(out_dir, exist_ok=True)
     from lasercalib_b200._cabi import Engine
     from lasercalib_b200.synth import make_rig
@@ -52,10 +56,10 @@ def main():
                     a[1] += v["total_ms"]
         return ms / done, prof
 
-    res = dict(card=card(), rig=rig, points=points, n_obs=int(pb["n_obs"]), steps=steps, runs=[])
+    res = dict(card=card(), rig=rig, points=points, n_obs=int(pb["n_obs"]), steps=steps, switch=var, runs=[])
     for rnd in range(rounds):
-        for plan in (("strip", "cover") if rnd % 2 == 0 else ("cover", "strip")):
-            os.environ["LCBA_I8_PLAN"] = plan
+        for plan in (vals if rnd % 2 == 0 else vals[::-1]):
+            os.environ[var] = plan
             eng = Engine()
             try:
                 eng.set_problem(pb["cams0"], pb["pts0"], pb["points_2d"], pb["camera_ind"], pb["point_ind"])
@@ -68,10 +72,10 @@ def main():
             res["runs"].append(dict(round=rnd, plan=plan, ms_per_step=ms_step, ms_k_i8_syrk=syrk,
                                     prof={k: v[1] / v[0] for k, v in prof.items()}))
             print("round %d %-5s: %.3f ms / step, k_i8_syrk %.3f ms / launch" % (rnd, plan, ms_step, syrk), flush=True)
-    os.environ.pop("LCBA_I8_PLAN")
+    os.environ.pop(var)
     res["card_after"] = card()
     summary = {}
-    for plan in ("strip", "cover"):
+    for plan in vals:
         s = np.array([r["ms_per_step"] for r in res["runs"] if r["plan"] == plan])
         k = np.array([r["ms_k_i8_syrk"] for r in res["runs"] if r["plan"] == plan])
         summary[plan] = dict(ms_per_step_median=float(np.median(s)), ms_per_step_min=float(s.min()), ms_per_step_max=float(s.max()),
@@ -80,7 +84,8 @@ def main():
             plan, summary[plan]["ms_per_step_median"], s.min(), s.max(), summary[plan]["syrk_median"], k.min(), k.max()))
     res["summary"] = summary
     print("card:", res["card"])
-    with open(os.path.join(out_dir, "i8_plan_ab.json"), "w") as f:
+    name = "i8_plan_ab.json" if var == "LCBA_I8_PLAN" else var.lower() + "_ab.json"
+    with open(os.path.join(out_dir, name), "w") as f:
         json.dump(res, f, indent=1)
 
 
