@@ -1,6 +1,6 @@
-// Streaming passes for DENSE rigs (most cameras see most points; no repeated (camera, point)
-// rows): the same arithmetic as linearize.cuh, organised so that a thread keeps ONE camera for
-// its whole life:
+// Linearisation for DENSE rigs (most cameras see most points; no repeated (camera, point) rows):
+// the same arithmetic as k_linearize, organised so that a thread keeps ONE camera for its whole
+// life:
 //     thread t of a 256-thread block  ->  camera c = t % C, point lane pl = t / C
 //     tile = PB = 256 / C consecutive points; observation of (point p, camera c) =
 //            obs_start[p] + popc(mask[p] & ((1 << c) - 1))        (point-major, camera-ascending)
@@ -38,7 +38,6 @@ struct DenseIdx {
 
 struct DenseItem {          // one (point, camera) work item
   double X[3];
-  double E[3];              // optional per-point 3-vector (g~_p)
   double2 ob;
   double w;
   int live;
@@ -58,10 +57,8 @@ __device__ __forceinline__ DenseIdx dense_idx(long long p, long long P, bool wor
 __device__ __forceinline__ DenseItem dense_item(const DenseIdx& d, long long p, int c,
                                                 const double* __restrict__ pts,
                                                 const double2* __restrict__ uv,
-                                                const double* __restrict__ wgt,
-                                                const double* __restrict__ extra3 = nullptr) {
+                                                const double* __restrict__ wgt) {
   DenseItem it;
-  it.E[0] = it.E[1] = it.E[2] = 0.0;
   it.w = 0.0;
   it.ob = make_double2(0.0, 0.0);
   it.X[0] = it.X[1] = it.X[2] = 0.0;
@@ -73,7 +70,6 @@ __device__ __forceinline__ DenseItem dense_item(const DenseIdx& d, long long p, 
     it.X[0] = pts[3 * p];
     it.X[1] = pts[3 * p + 1];
     it.X[2] = pts[3 * p + 2];
-    if (extra3) { it.E[0] = extra3[3 * p]; it.E[1] = extra3[3 * p + 1]; it.E[2] = extra3[3 * p + 2]; }
   }
   return it;
 }
@@ -207,98 +203,6 @@ __global__ void k_dense_cam_unpack(const double* __restrict__ red, int C, double
   while (idx < v) { idx += NCP - a; ++a; }
   if (idx == v) camsum[c * CAMSUM + NCP + a] = x;
 }
-
-// ---- residual (fun): cost only ---------------------------------------------------------------
-__global__ void __launch_bounds__(DP_THREADS, 2)
-k_residual_dense(const double* __restrict__ tab, const double* __restrict__ pts,
-                 const double2* __restrict__ uv, const double* __restrict__ wgt,
-                 const uint32_t* __restrict__ obs_start,
-                 const unsigned long long* __restrict__ mask, long long P, int C, int PB,
-                 double* __restrict__ part) {
-  extern __shared__ double s_dyn[];
-  double* s_tab = s_dyn;
-  __shared__ double s_red[32];
-  const int t = threadIdx.x;
-  load_tables_smem(tab, s_tab, C);
-  __syncthreads();
-  const int c = t % C, pl = t / C;
-  const bool worker = pl < PB;
-  double T[CAMTAB];               // only the 17 entries project_tab reads stay live (registers)
-#pragma unroll
-  for (int i = 0; i < CAMTAB; ++i) T[i] = s_tab[c * CAMTAB + i];
-  double acc = 0.0;
-  const long long ntiles = (P + PB - 1) / PB;
-  long long tile = blockIdx.x;
-  const long long G = gridDim.x;
-  DenseItem nxt = dense_item(dense_idx(tile * PB + pl, P, worker && tile < ntiles, obs_start, mask),
-                             tile * PB + pl, c, pts, uv, wgt);
-  DenseIdx idx2 = dense_idx((tile + G) * PB + pl, P, worker && tile + G < ntiles, obs_start, mask);
-  for (; tile < ntiles; tile += G) {
-    const DenseItem cur = nxt;
-    nxt = dense_item(idx2, (tile + G) * PB + pl, c, pts, uv, wgt);
-    idx2 = dense_idx((tile + 2 * G) * PB + pl, P, worker && tile + 2 * G < ntiles, obs_start, mask);
-    if (cur.live) {
-      double pu, pv;
-      project_tab(T, cur.X[0], cur.X[1], cur.X[2], pu, pv);
-      const double ru = cur.w * (pu - cur.ob.x), rv = cur.w * (pv - cur.ob.y);
-      acc = fma(ru, ru, fma(rv, rv, acc));
-    }
-  }
-  const double s = block_sum(acc, s_red);
-  if (t == 0) part[blockIdx.x] = s;
-}
-
-// ---- |J g~|^2 ----------------------------------------------------------------------------------
-__global__ void __launch_bounds__(DP_THREADS, 2)
-k_jdot_dense(const double* __restrict__ tab, const double* __restrict__ pts,
-             const double* __restrict__ wgt, const uint32_t* __restrict__ obs_start,
-             const unsigned long long* __restrict__ mask, const double* __restrict__ gt_c,
-             const double* __restrict__ gt_p, long long P, int C, int PB,
-             double* __restrict__ part) {
-  extern __shared__ double s_dyn[];
-  double* s_tab = s_dyn;
-  __shared__ double s_red[32];
-  const int t = threadIdx.x;
-  load_tables_smem(tab, s_tab, C);
-  __syncthreads();
-  const int c = t % C, pl = t / C;
-  const bool worker = pl < PB;
-  const volatile double* vT = s_tab + c * CAMTAB;
-  double gc[NCP];
-#pragma unroll
-  for (int a = 0; a < NCP; ++a) gc[a] = gt_c[c * NCP + a];
-  double acc = 0.0;
-  const long long ntiles = (P + PB - 1) / PB;
-  long long tile = blockIdx.x;
-  const long long G = gridDim.x;
-  DenseItem nxt = dense_item(dense_idx(tile * PB + pl, P, worker && tile < ntiles, obs_start, mask),
-                             tile * PB + pl, c, pts, nullptr, wgt, gt_p);
-  DenseIdx idx2 = dense_idx((tile + G) * PB + pl, P, worker && tile + G < ntiles, obs_start, mask);
-  for (; tile < ntiles; tile += G) {
-    const DenseItem cur = nxt;
-    nxt = dense_item(idx2, (tile + G) * PB + pl, c, pts, nullptr, wgt, gt_p);
-    idx2 = dense_idx((tile + 2 * G) * PB + pl, P, worker && tile + 2 * G < ntiles, obs_start, mask);
-    if (cur.live) {
-      double T[CAMTAB];
-#pragma unroll
-      for (int i = 0; i < CAMTAB; ++i) T[i] = vT[i];
-      ObsLin L;
-      obs_linearize<false>(T, cur.X[0], cur.X[1], cur.X[2], 0.0, 0.0, cur.w, L);
-      double a0 = cur.w * gc[9], a1 = cur.w * gc[10];
-#pragma unroll
-      for (int a = 0; a < 9; ++a) { a0 = fma(L.Jc[0][a], gc[a], a0); a1 = fma(L.Jc[1][a], gc[a], a1); }
-#pragma unroll
-      for (int a = 0; a < 3; ++a) {
-        a0 = fma(L.Jp[0][a], cur.E[a], a0);
-        a1 = fma(L.Jp[1][a], cur.E[a], a1);
-      }
-      acc = fma(a0, a0, fma(a1, a1, acc));
-    }
-  }
-  const double s = block_sum(acc, s_red);
-  if (t == 0) part[blockIdx.x] = s;
-}
-
 
 // ============================== point-parallel passes ==========================================
 // Residual, |J g~|^2 and the back-substitution have NO per-camera output, so a thread can own a
@@ -471,162 +375,6 @@ k_backsub_pt(const double* __restrict__ tab, const double* __restrict__ pts,
   for (int k = 0; k < BS_K; ++k) {
     const double s = block_sum(acc[k], s_red);
     if (threadIdx.x == 0) part[(size_t)blockIdx.x * BS_K + k] = s;
-  }
-}
-
-// ---- back-substitution + Gram sums ------------------------------------------------------------
-// Same outputs as k_backsub (linearize.cuh): gn_p = (V + lam Dp^2)^-1 (g_p - W^T p_c) per point and
-// part[block][0..8] = (Jg~.Jg~, Jg~.Jp, Jp.Jp | a.a, a.b, b.b | g~.g~, g~.p, p.p) (point parts).
-// Per tile: (1) every (point, camera) thread evaluates Jc, Jp, the 2-vectors A = J g~ and
-// b = Jc p_c, and t = Jp^T b -> shared memory; (2) one thread per point sums t over the cameras
-// (fixed order), solves with the point's factor L^-1 (prefetched with cp.async one tile ahead:
-// Vg, Lz, scl are contiguous per tile) and publishes p_p; (3) the item threads finish b += Jp p_p
-// and accumulate the three Gram sums.  Step (3) of a tile runs together with step (1) of the next.
-constexpr int DB_PT = 9 + 9 + 3;    // per point in the staged tile: Vg (9), Lz (9), scl (3)
-__host__ __device__ inline size_t dense_bs_smem_doubles(int C, int PB) {
-  return (size_t)((C * CAMTAB + 1) & ~1) + (size_t)DP_THREADS * 3 + 2 * (size_t)PB * 3 +
-         2 * (((size_t)PB * DB_PT + 1) & ~1);
-}
-
-__global__ void __launch_bounds__(DP_THREADS, 2)
-k_backsub_dense(const double* __restrict__ tab, const double* __restrict__ pts,
-                const double* __restrict__ wgt, const uint32_t* __restrict__ obs_start,
-                const unsigned long long* __restrict__ mask, long long P, int C, int PB,
-                const double* __restrict__ Vg, const double* __restrict__ Lz,
-                const double* __restrict__ scl, const double* __restrict__ gt_c,
-                const double* __restrict__ gt_p, const double* __restrict__ pc,
-                double* __restrict__ gn_p, double* __restrict__ part) {
-  extern __shared__ __align__(16) double s_dyn[];
-  double* s_tab = s_dyn;
-  double* s_tv = s_dyn + ((C * CAMTAB + 1) & ~1);          // [DP_THREADS][3]
-  double* s_pp = s_tv + DP_THREADS * 3;                    // [2][PB][3]
-  double* s_pt = s_pp + 2 * PB * 3;                        // [2][PB * DB_PT | even]
-  const size_t pt_stride = ((size_t)PB * DB_PT + 1) & ~1;
-  __shared__ double s_red[32];
-  const int t = threadIdx.x;
-  load_tables_smem(tab, s_tab, C);
-  const int c = t % C, pl = t / C;
-  const bool worker = pl < PB;
-  const volatile double* vT = s_tab + c * CAMTAB;
-  double gc[NCP], pcc[NCP];
-#pragma unroll
-  for (int a = 0; a < NCP; ++a) { gc[a] = gt_c[c * NCP + a]; pcc[a] = pc[c * NCP + a]; }
-  double acc[BS_K];
-#pragma unroll
-  for (int k = 0; k < BS_K; ++k) acc[k] = 0.0;
-  const long long ntiles = (P + PB - 1) / PB;
-  const long long G = gridDim.x;
-
-  // cp.async of one tile's per-point inputs (Vg | Lz | scl, each contiguous) into stage `st`
-  auto stage_points = [&](long long tl, int st) {
-    if (tl < ntiles) {
-      const long long p0 = tl * PB;
-      const int npts = (int)min((long long)PB, P - p0);
-      double* dst = s_pt + (size_t)st * pt_stride;
-      const int n9 = npts * 9, n3 = npts * 3;
-      // 8-byte copies: the tile origin p0 * 72 B is 8-byte aligned for every PB
-      for (int i = t; i < 2 * n9 + n3; i += DP_THREADS) {
-        const double* src = i < n9 ? Vg + p0 * 9 + i : (i < 2 * n9 ? Lz + p0 * 9 + (i - n9) : scl + p0 * 3 + (i - 2 * n9));
-        const unsigned d = (unsigned)__cvta_generic_to_shared(dst + i);
-        asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(d), "l"(src) : "memory");
-      }
-    }
-    asm volatile("cp.async.commit_group;" ::: "memory");
-  };
-
-  long long tile = blockIdx.x;
-  stage_points(tile, 0);
-  DenseItem nxt = dense_item(dense_idx(tile * PB + pl, P, worker && tile < ntiles, obs_start, mask),
-                             tile * PB + pl, c, pts, nullptr, wgt, gt_p);
-  DenseIdx idx2 = dense_idx((tile + G) * PB + pl, P, worker && tile + G < ntiles, obs_start, mask);
-  __syncthreads();
-  int buf = 0;
-  double jp[2][3], A0 = 0, A1 = 0, b0 = 0, b1 = 0;
-  int live_prev = 0;
-  for (; tile < ntiles; tile += G, buf ^= 1) {
-    const DenseItem cur = nxt;
-    nxt = dense_item(idx2, (tile + G) * PB + pl, c, pts, nullptr, wgt, gt_p);
-    idx2 = dense_idx((tile + 2 * G) * PB + pl, P, worker && tile + 2 * G < ntiles, obs_start, mask);
-    stage_points(tile + G, buf ^ 1);
-    // (1) this tile's items
-    if (cur.live) {
-      double T[CAMTAB];
-#pragma unroll
-      for (int i = 0; i < CAMTAB; ++i) T[i] = vT[i];
-      ObsLin L;
-      obs_linearize<false>(T, cur.X[0], cur.X[1], cur.X[2], 0.0, 0.0, cur.w, L);
-      A0 = cur.w * gc[9]; A1 = cur.w * gc[10];
-      b0 = cur.w * pcc[9]; b1 = cur.w * pcc[10];
-#pragma unroll
-      for (int a = 0; a < 9; ++a) {
-        A0 = fma(L.Jc[0][a], gc[a], A0);  A1 = fma(L.Jc[1][a], gc[a], A1);
-        b0 = fma(L.Jc[0][a], pcc[a], b0); b1 = fma(L.Jc[1][a], pcc[a], b1);
-      }
-#pragma unroll
-      for (int a = 0; a < 3; ++a) {
-        A0 = fma(L.Jp[0][a], cur.E[a], A0);
-        A1 = fma(L.Jp[1][a], cur.E[a], A1);
-        jp[0][a] = L.Jp[0][a];
-        jp[1][a] = L.Jp[1][a];
-        s_tv[t * 3 + a] = fma(L.Jp[0][a], b0, L.Jp[1][a] * b1);      // J_p^T (J_c p_c)
-      }
-    } else if (worker) {
-      s_tv[t * 3] = 0.0; s_tv[t * 3 + 1] = 0.0; s_tv[t * 3 + 2] = 0.0;
-    }
-    live_prev = cur.live;
-    asm volatile("cp.async.wait_group 1;" ::: "memory");      // this tile's point inputs have landed
-    __syncthreads();
-    // (2) one thread per point
-    const long long p0 = tile * PB;
-    const int npts = (int)min((long long)PB, P - p0);
-    if (t < npts) {
-      const double* src = s_tv + (size_t)t * C * 3;
-      double t0 = 0, t1 = 0, t2 = 0;
-      for (int k = 0; k < C; ++k) { t0 += src[3 * k]; t1 += src[3 * k + 1]; t2 += src[3 * k + 2]; }
-      const double* sp = s_pt + (size_t)buf * pt_stride;
-      const double* v = sp + t * 9;
-      const double* li = sp + npts * 9 + t * 9;
-      const double* sc = sp + 2 * npts * 9 + t * 3;
-      const double r0 = v[6] - t0, r1 = v[7] - t1, r2 = v[8] - t2;
-      const double y0 = li[0] * r0;
-      const double y1 = fma(li[1], r0, li[2] * r1);
-      const double y2 = fma(li[3], r0, fma(li[4], r1, li[5] * r2));
-      const double q0 = fma(li[0], y0, fma(li[1], y1, li[3] * y2));
-      const double q1 = fma(li[2], y1, li[4] * y2);
-      const double q2 = li[5] * y2;
-      double* o = s_pp + ((size_t)buf * PB + t) * 3;
-      o[0] = q0; o[1] = q1; o[2] = q2;
-      const long long p = p0 + t;
-      gn_p[3 * p] = q0; gn_p[3 * p + 1] = q1; gn_p[3 * p + 2] = q2;
-      const double pp[3] = {q0, q1, q2};
-#pragma unroll
-      for (int a = 0; a < 3; ++a) {
-        const double s = sc[a], g = v[6 + a];
-        const double ah = g / s, bh = pp[a] * s, gtl = ah / s;
-        acc[3] = fma(ah, ah, acc[3]);
-        acc[4] = fma(ah, bh, acc[4]);
-        acc[5] = fma(bh, bh, acc[5]);
-        acc[6] = fma(gtl, gtl, acc[6]);
-        acc[7] = fma(gtl, pp[a], acc[7]);
-        acc[8] = fma(pp[a], pp[a], acc[8]);
-      }
-    }
-    __syncthreads();
-    // (3) finish the items of this tile
-    if (live_prev) {
-      const double* pp = s_pp + ((size_t)buf * PB + pl) * 3;
-#pragma unroll
-      for (int a = 0; a < 3; ++a) { b0 = fma(jp[0][a], pp[a], b0); b1 = fma(jp[1][a], pp[a], b1); }
-      acc[0] = fma(A0, A0, fma(A1, A1, acc[0]));
-      acc[1] = fma(A0, b0, fma(A1, b1, acc[1]));
-      acc[2] = fma(b0, b0, fma(b1, b1, acc[2]));
-    }
-  }
-  asm volatile("cp.async.wait_group 0;" ::: "memory");
-#pragma unroll
-  for (int k = 0; k < BS_K; ++k) {
-    const double s = block_sum(acc[k], s_red);
-    if (t == 0) part[(size_t)blockIdx.x * BS_K + k] = s;
   }
 }
 

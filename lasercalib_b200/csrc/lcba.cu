@@ -110,14 +110,12 @@ struct lcba_handle {
   // dense rigs: passes with a fixed camera per thread (dense_passes.cuh)
   bool use_dense = false;
   bool use_pt = false;           // point-parallel residual / jdot / backsub (no repeated pairs)
-  int pt_mode = 1;               // LCBA_PT_PASSES: 0 off, 1 on (default), 2 = (camera, point) variants
   int ptp_grid = 0;
-  int dp_pb = 0, dp_grid_lin = 0, dp_grid = 0;
+  int dp_pb = 0, dp_grid_lin = 0;
   double *d_dpart = nullptr, *d_dred = nullptr;
   double* d_Yg = nullptr;        // Y of every (point, camera) in ring layout (k_make_Y), or null
   // int8 tensor-core Schur path (schur_i8.cuh)
   bool use_i8 = false;
-  bool i8_tma = false;           // operand loads through TMA tensor maps (else 1-D bulk copies)
   I8Maps i8maps;
   I8Plan i8plan;
   I8Work* d_i8work = nullptr;
@@ -338,10 +336,9 @@ extern "C" int lcba_create(lcba_t** out, int device) {
                                       (const void*)k_schur_mma<3, true>, (const void*)k_schur_mma<4, true>,
                                       (const void*)k_schur_mma<5, true>, (const void*)k_schur_mma<6, true>,
                                       (const void*)k_sq_camonly<true>, (const void*)k_sq_camonly<false>,
-                                      (const void*)k_linearize_dense, (const void*)k_residual_dense,
-                                      (const void*)k_jdot_dense, (const void*)k_backsub_dense,
+                                      (const void*)k_linearize_dense,
                                       (const void*)k_residual_pt, (const void*)k_jdot_pt, (const void*)k_backsub_pt,
-                                      (const void*)k_i8_syrk<true>, (const void*)k_i8_syrk<false>, (const void*)k_i8_make,
+                                      (const void*)k_i8_syrk, (const void*)k_i8_make,
                                       (const void*)k_i8_make_ref,
                                       (const void*)k_jdot,      (const void*)k_jacobian_blocks};
     for (const void* f : big_smem_kernels) {
@@ -629,10 +626,9 @@ extern "C" int lcba_set_problem_shard(lcba_t* h, int32_t C, int64_t P, int64_t N
         LCBA_TRY(dev_alloc(h, &h->d_i8progress, ip.work.size()));
         LCBA_CUDA(h, cudaMemsetAsync(h->d_i8progress, 0, ip.work.size() * sizeof(unsigned long long), st));
         LCBA_TRY(dev_alloc(h, &h->d_i8planes, ip.plane_bytes));
-        {
-          const char* te = getenv("LCBA_I8_TMA");
-          h->i8_tma = !(te && atoi(te) == 0) && i8_encode_maps(ip, h->d_i8planes, &h->i8maps);
-          if (!h->i8_tma) memset(&h->i8maps, 0, sizeof(h->i8maps));
+        if (!i8_encode_maps(ip, h->d_i8planes, &h->i8maps)) {
+          set_error(h, "lcba_set_problem: tensor-map encode (cuTensorMapEncodeTiled) of the int8 Schur digit planes failed");
+          return LCBA_E_CUDA;
         }
         LCBA_TRY(dev_alloc(h, &h->d_i8partial, ip.work.size() * 128 * 64));
         LCBA_TRY(dev_alloc(h, &h->d_i8rmax, (size_t)h->i8_gx_max * ip.NRG * 8));
@@ -668,24 +664,19 @@ extern "C" int lcba_set_problem_shard(lcba_t* h, int32_t C, int64_t P, int64_t N
       h->use_mma = true;
     }
   }
-  // dense streaming passes: tensor-path rigs without repeated pairs (LCBA_DENSE_PASSES=0 disables)
-  h->use_dense = false;
-  {
-    const char* env = getenv("LCBA_DENSE_PASSES");
-    if (h->use_mma && h->n_pairs == N && !(env && atoi(env) == 0)) {
-      h->use_dense = true;
-      h->dp_pb = DP_THREADS / C;
-      const long long ntiles = (P + h->dp_pb - 1) / h->dp_pb;
-      h->dp_grid_lin = (int)std::max<long long>(1, std::min<long long>(ntiles, (long long)h->sm_count));
-      h->dp_grid = (int)std::max<long long>(1, std::min<long long>(ntiles, (long long)h->sm_count * 2));
-      LCBA_TRY(dev_alloc(h, &h->d_dpart, (size_t)h->dp_grid_lin * C * DP_CAM_VALS));
-      LCBA_TRY(dev_alloc(h, &h->d_dred, (size_t)C * DP_CAM_VALS));
-    }
+  // dense linearisation (k_linearize_dense, U_c included): tensor-path rigs without repeated pairs
+  h->use_dense = h->use_mma && h->n_pairs == N;
+  if (h->use_dense) {
+    h->dp_pb = DP_THREADS / C;
+    const long long ntiles = (P + h->dp_pb - 1) / h->dp_pb;
+    h->dp_grid_lin = (int)std::max<long long>(1, std::min<long long>(ntiles, (long long)h->sm_count));
+    LCBA_TRY(dev_alloc(h, &h->d_dpart, (size_t)h->dp_grid_lin * C * DP_CAM_VALS));
+    LCBA_TRY(dev_alloc(h, &h->d_dred, (size_t)C * DP_CAM_VALS));
   }
   {
+    // LCBA_PT_PASSES=0 runs the observation-major kernels on rigs without repeated pairs (tests)
     const char* env = getenv("LCBA_PT_PASSES");
-    h->pt_mode = env ? atoi(env) : 1;
-    h->use_pt = h->n_pairs == N && h->pt_mode == 1;
+    h->use_pt = h->n_pairs == N && !(env && atoi(env) == 0);
     h->ptp_grid = (int)std::max<long long>(1, std::min<long long>(nblk(P, PT_THREADS), (long long)h->sm_count * 2));
   }
   LCBA_TRY(dev_alloc(h, &h->d_Spart, h->plan.part_stride * max_slices));
@@ -867,13 +858,6 @@ static int run_residual(lcba_t* h, int which, double2* r_out, bool local = false
     KL(h, "reduce", k_reduce_scalars<<<1, 256, 0, h->stream>>>(h->d_part, h->ptp_grid, 1, h->d_red, 1));
     return local ? LCBA_OK : allreduce(h, h->d_red, 1, NCCL_SUM);
   }
-  if (h->use_dense && h->pt_mode == 2 && !r_out) {
-    KL(h, "residual", k_residual_dense<<<h->dp_grid, DP_THREADS, smem, h->stream>>>(
-          h->d_tab[which], h->d_pts[which], h->d_uv, h->d_w, h->d_obs_start, h->d_mask, h->P, h->C, h->dp_pb,
-          h->d_part));
-    KL(h, "reduce", k_reduce_scalars<<<1, 256, 0, h->stream>>>(h->d_part, h->dp_grid, 1, h->d_red, 1));
-    return local ? LCBA_OK : allreduce(h, h->d_red, 1, NCCL_SUM);
-  }
   KL(h, "residual", k_residual<<<h->obs_grid, 256, smem, h->stream>>>(
         h->d_tab[which], h->d_pts[which], h->d_uv, h->d_cam, h->d_pt, h->d_w, h->d_perm, h->N, h->C,
         r_out, h->d_part));
@@ -986,11 +970,6 @@ static int pass_jdot(lcba_t* h) {
     KL(h, "jdot", k_jdot_pt<<<h->ptp_grid, PT_THREADS, smem, h->stream>>>(
           h->d_tab[w], h->d_pts[w], h->d_w, h->d_obs_start, h->d_mask, h->d_gt_c, h->d_gt_p, h->P, C, h->d_part));
     KL(h, "reduce", k_reduce_scalars<<<1, 256, 0, h->stream>>>(h->d_part, h->ptp_grid, 1, h->d_red, 1));
-  } else if (h->use_dense && h->pt_mode == 2) {
-    KL(h, "jdot", k_jdot_dense<<<h->dp_grid, DP_THREADS, (size_t)C * CAMTAB * 8, h->stream>>>(
-          h->d_tab[w], h->d_pts[w], h->d_w, h->d_obs_start, h->d_mask, h->d_gt_c, h->d_gt_p, h->P, C,
-          h->dp_pb, h->d_part));
-    KL(h, "reduce", k_reduce_scalars<<<1, 256, 0, h->stream>>>(h->d_part, h->dp_grid, 1, h->d_red, 1));
   } else {
   KL(h, "jdot", k_jdot<<<h->obs_grid, 256, smem, h->stream>>>(
         h->d_tab[w], h->d_pts[w], h->d_cam, h->d_pt, h->d_w, h->d_gt_c, h->d_gt_p, h->N, C, h->d_part));
@@ -1047,14 +1026,8 @@ static int pass_schur(lcba_t* h, const double* lam_host_or_null) {
       const I8Plan& ip = h->i8plan;
       launch_i8_rowexp(h);
       launch_i8_make(h, false);
-      if (h->i8_tma)
-        KL(h, "schur", k_i8_syrk<true><<<(unsigned)ip.work.size(), I8_THREADS, ip.smem_bytes, h->stream>>>(
-              h->i8maps, h->d_i8planes, ip.NRG, h->d_i8work, h->d_i8partial, h->d_fail, h->d_i8progress, ip.window,
-              h->d_stats));
-      else
-        KL(h, "schur", k_i8_syrk<false><<<(unsigned)ip.work.size(), I8_THREADS, ip.smem_bytes, h->stream>>>(
-              h->i8maps, h->d_i8planes, ip.NRG, h->d_i8work, h->d_i8partial, h->d_fail, h->d_i8progress, ip.window,
-              h->d_stats));
+      KL(h, "schur", k_i8_syrk<<<(unsigned)ip.work.size(), I8_THREADS, ip.smem_bytes, h->stream>>>(
+            h->i8maps, h->d_i8work, h->d_i8partial, h->d_fail, h->d_i8progress, ip.window, h->d_stats));
       KL(h, "schur_reduce", k_i8_gather<<<dim3((unsigned)ip.tiles.size(), 16), 256, 0, h->stream>>>(
             h->d_i8partial, h->d_i8tiles, C, ip.cover ? 1 : 0, h->d_i8erow, pl.npairs, h->d_Sred));
       KL(h, "schur_reduce", k_add_cam_blocks<<<nblk(C * 121, 128), 128, 0, h->stream>>>(h->d_U, C, h->d_Sred));
@@ -1199,12 +1172,6 @@ static int pass_backsub(lcba_t* h) {
           h->d_tab[w], h->d_pts[w], h->d_w, h->d_obs_start, h->d_mask, h->P, C, h->d_Vg, h->d_Lz, h->d_scl_p,
           h->d_gt_c, h->d_gt_p, h->d_pc, h->d_gn_p, h->d_part));
     KL(h, "reduce", k_reduce_scalars<<<BS_K, 256, 0, h->stream>>>(h->d_part, h->ptp_grid, BS_K, h->d_red, BS_K));
-  } else if (h->use_dense && h->pt_mode == 2) {
-    const size_t smem = dense_bs_smem_doubles(C, h->dp_pb) * 8;
-    KL(h, "backsub", k_backsub_dense<<<h->dp_grid, DP_THREADS, smem, h->stream>>>(
-          h->d_tab[w], h->d_pts[w], h->d_w, h->d_obs_start, h->d_mask, h->P, C, h->dp_pb, h->d_Vg, h->d_Lz,
-          h->d_scl_p, h->d_gt_c, h->d_gt_p, h->d_pc, h->d_gn_p, h->d_part));
-    KL(h, "reduce", k_reduce_scalars<<<BS_K, 256, 0, h->stream>>>(h->d_part, h->dp_grid, BS_K, h->d_red, BS_K));
   } else {
   const size_t smem = ((size_t)C * CAMTAB + 2 * (size_t)C * NCP + 2 * LIN_THREADS * 3) * 8;
   KL(h, "backsub", k_backsub<<<h->lin_grid, LIN_THREADS, smem, h->stream>>>(

@@ -15,11 +15,11 @@
 //                   [K block of 64 kappa = 21 points + 1 zero][slice][row group of 8][k-step 2][k half 2][8][16]
 //   k_i8_syrk     : one CTA = one output tile (128 rows x <= 64 columns, the 7 anti-diagonals d = i + j
 //                   side by side in TMEM) x a range of K blocks; warps 0-3 epilogue (TMEM -> FP64 registers
-//                   before an int32 can overflow), warp 4 producer (up to three tensor loads per K block =
-//                   2 k-steps: all six slices of A (4-D, or 5-D for two row ranges), B1, B2; fallback: one 1-D
-//                   bulk copy per lane), warp 5 MMA issuer (elect.sync, compile-time MMA plan: slice i of the
-//                   rows against slices 0..6-i of the columns in ONE instruction, N <= 256, A kept in the
-//                   collector, widest last); tiles from the strip or the cover plan, CTAs per tile weighted
+//                   before an int32 can overflow), warp 4 producer (up to three TMA tensor loads per K block =
+//                   2 k-steps: all six slices of A (4-D, or 5-D for two row ranges), B1, B2), warp 5 MMA
+//                   issuer (elect.sync, compile-time MMA plan: slice i of the rows against slices 0..6-i of
+//                   the columns in ONE instruction, N <= 256, A kept in the collector, widest last); tiles
+//                   from the strip or the cover plan, CTAs per tile weighted
 //                   by the measured cost of a K block, K blocks dealt K-major in chunks so that all tiles read a
 //                   K block at about the same time, a progress window between the CTAs (i8_deal)
 //   k_i8_gather   : per-CTA partials -> the pair-block layout of Sred (fixed order, no atomics)
@@ -65,8 +65,7 @@ struct I8Work {
 // TMA tensor maps over the digit planes, one per (box height, range distance) that the plan uses.
 // delta = 0: a 4-D tensor (128 u32 = one 512-byte row group, NRG row groups, 6 digits, K blocks); a box of
 // (128, h, 6, 1) lands in shared memory as [digit][h row groups][512 B] = the UMMA operand of all six digits
-// in ONE instruction (the 1-D bulk-copy version needs one copy per digit and operand: 18 per K block, and the
-// ~110 cycles of issue per copy made the copy engine, not the tensor pipe, set the pace).
+// in ONE instruction.
 // delta > 0: the two-range A operand, a 5-D tensor (128 u32, NRG - delta row groups, 2 ranges delta row
 // groups apart, 6 digits, K blocks); a box of (128, h, 2, 6, 1) lands as [digit][2 h row groups][512 B], the same
 // layout as one range of 2 h row groups.
@@ -79,7 +78,7 @@ struct I8Plan {
   long long nkb = 0;
   int map_heights[I8_MAX_MAPS] = {};                   // box heights (row groups per range) of the tensor maps
   int map_delta[I8_MAX_MAPS] = {};                     // 0: one range; > 0: two ranges this many row groups apart
-  int nmaps = 0;                                       // > I8_MAX_MAPS: too many shapes, use 1-D bulk copies
+  int nmaps = 0;                                       // > I8_MAX_MAPS: too many shapes, i8_encode_maps fails
   bool cover = false;                                  // made by make_i8_cover_plan
   bool kmajor = true;                                  // K-major schedule (else one contiguous K range per CTA)
   int window = 0;                                      // K-major: K blocks a CTA may run ahead of the slowest
@@ -286,7 +285,7 @@ inline double i8_executed_ops(const I8Plan& pl) {
 }
 
 // Encode the tensor maps of a plan over `planes` (host).  Returns false when the driver entry point is
-// missing, an encode fails or the plan has more shapes than I8_MAX_MAPS: the caller then uses bulk copies.
+// missing, an encode fails or the plan has more shapes than I8_MAX_MAPS (the plans need at most 16).
 inline bool i8_encode_maps(const I8Plan& pl, void* planes, I8Maps* out) {
   if (pl.nmaps <= 0 || pl.nmaps > I8_MAX_MAPS) return false;
   typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
@@ -357,10 +356,6 @@ __device__ __forceinline__ void i8_mbar_wait(uint32_t bar, uint32_t parity, int*
     if (BACKOFF) __nanosleep(128);      // waiting warps must not compete with the MMA issuer for issue slots
     if (clock64() - t0 > 6000000000LL) { atomicOr(fail, 4); asm volatile("trap;"); }
   }
-}
-__device__ __forceinline__ void i8_bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-               ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
 }
 // COLL: what happens to the A operand in the tensor core's collector: 0 nothing kept (the default), 1 ::fill (read
 // from shared memory and kept), 2 ::use (taken from the collector, kept), 3 ::lastuse (taken from the collector)
@@ -987,10 +982,8 @@ __device__ __forceinline__ int i8_progress_min(const unsigned long long* progres
 
 // partial[cta][128][64] doubles: sum_d 2^-8(d+2) D_d  (row exponents are applied by k_i8_gather).
 // window > 0: the K-major schedule's window in K blocks over progress[gridDim.x]; 0: no window.
-template <bool TMA>
 __global__ void __launch_bounds__(I8_THREADS, 1)
-k_i8_syrk(const __grid_constant__ I8Maps maps, const unsigned char* __restrict__ planes, int NRG,
-          const I8Work* __restrict__ work, double* __restrict__ partial, int* __restrict__ fail,
+k_i8_syrk(const __grid_constant__ I8Maps maps, const I8Work* __restrict__ work, double* __restrict__ partial, int* __restrict__ fail,
           unsigned long long* __restrict__ progress, int window,
           long long* __restrict__ stats /* null, or per CTA: MMA warp (waiting at FULL, total), producer (waiting for the window, total) cycles */) {
   extern __shared__ __align__(1024) uint8_t i8_smem[];
@@ -1025,11 +1018,8 @@ k_i8_syrk(const __grid_constant__ I8Maps maps, const unsigned char* __restrict__
   const int nkb = W.kb1 - W.kb0;
 
   if (wid == 4) {
-    // ---- producer: TMA, one tensor copy per operand (all six digits of A / B1 / B2) issued by lane 0; or 1-D bulk
-    // copies, one per lane: (digit, operand) = A range 1, A range 2, B of block 1, B of block 2.  The whole warp
-    // keeps the window.
-    const int ci = lane / 4, cb = lane - 4 * ci;
-    const bool mine = TMA ? lane == 0 : lane < 4 * I8_NS && (cb == 0 || cb == 2 || (cb == 1 && W.m2_nrg > 0) || (cb == 3 && W.n2_nrg > 0));
+    // ---- producer: TMA, one tensor copy per operand (all six digits of A / B1 / B2) issued by lane 0.  The whole
+    // warp keeps the window.
     const long long t_begin = stats ? clock64() : 0;
     long long t_window = 0;
     unsigned epoch = 0;
@@ -1050,23 +1040,15 @@ k_i8_syrk(const __grid_constant__ I8Maps maps, const unsigned char* __restrict__
           t_window += clock64() - w0;
         }
       }
-      if (it >= I8_STAGES && (TMA ? lane == 0 : true)) i8_mbar_wait<false>(bar_empty + 8 * st, ((it / I8_STAGES) - 1) & 1, fail);
+      if (it >= I8_STAGES && lane == 0) i8_mbar_wait<false>(bar_empty + 8 * st, ((it / I8_STAGES) - 1) & 1, fail);
       if (lane == 0) i8_mbar_expect_tx(bar_full + 8 * st, (uint32_t)I8_NS * (a_bytes + b_bytes + b2_bytes));
       __syncwarp();
-      if (mine) {
+      if (lane == 0) {
         const uint32_t dstA = smem0 + st * STAGE_BYTES, dstB = dstA + A_REGION;
-        if (TMA) {
-          if (W.m2_nrg > 0) i8_tma_5d(dstA, &maps.m[W.map_a], 0, W.m_rg0, 0, 0, kb, bar_full + 8 * st);
-          else i8_tma_4d(dstA, &maps.m[W.map_a], 0, W.m_rg0, 0, kb, bar_full + 8 * st);
-          i8_tma_4d(dstB, &maps.m[W.map_b1], 0, W.n_rg0, 0, kb, bar_full + 8 * st);
-          if (W.n2_nrg > 0) i8_tma_4d(dstB + B2_OFF, &maps.m[W.map_b2], 0, W.n2_rg0, 0, kb, bar_full + 8 * st);
-        } else {
-          const unsigned char* src = planes + (size_t)kb * I8_NS * NRG * I8_RG_BYTES + (size_t)ci * NRG * I8_RG_BYTES;
-          if (cb == 0) i8_bulk_g2s(dstA + ci * a_bytes, src + (size_t)W.m_rg0 * I8_RG_BYTES, a1_bytes, bar_full + 8 * st);
-          else if (cb == 1) i8_bulk_g2s(dstA + ci * a_bytes + a1_bytes, src + (size_t)W.m2_rg0 * I8_RG_BYTES, a_bytes - a1_bytes, bar_full + 8 * st);
-          else if (cb == 2) i8_bulk_g2s(dstB + ci * b_bytes, src + (size_t)W.n_rg0 * I8_RG_BYTES, b_bytes, bar_full + 8 * st);
-          else i8_bulk_g2s(dstB + B2_OFF + ci * b2_bytes, src + (size_t)W.n2_rg0 * I8_RG_BYTES, b2_bytes, bar_full + 8 * st);
-        }
+        if (W.m2_nrg > 0) i8_tma_5d(dstA, &maps.m[W.map_a], 0, W.m_rg0, 0, 0, kb, bar_full + 8 * st);
+        else i8_tma_4d(dstA, &maps.m[W.map_a], 0, W.m_rg0, 0, kb, bar_full + 8 * st);
+        i8_tma_4d(dstB, &maps.m[W.map_b1], 0, W.n_rg0, 0, kb, bar_full + 8 * st);
+        if (W.n2_nrg > 0) i8_tma_4d(dstB + B2_OFF, &maps.m[W.map_b2], 0, W.n2_rg0, 0, kb, bar_full + 8 * st);
       }
     }
     if (window > 0 && lane == 0) i8_progress_put(progress + blockIdx.x, ((unsigned long long)epoch << 32) | I8_DONE);

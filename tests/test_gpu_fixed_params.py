@@ -21,7 +21,7 @@ pytestmark = pytest.mark.gpu
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 # pass routes (LCBA_PT_PASSES) and Schur routes (LCBA_SCHUR_MMA / LCBA_SCHUR_I8) as the other GPU tests select them
-ROUTES = {"pt": {}, "generic": {"LCBA_PT_PASSES": "0"}, "dense": {"LCBA_PT_PASSES": "2"},
+ROUTES = {"pt": {}, "generic": {"LCBA_PT_PASSES": "0"},
           "dfma": {"LCBA_SCHUR_MMA": "0"}, "dmma": {"LCBA_SCHUR_MMA": "1", "LCBA_SCHUR_I8": "0"},
           "i8": {"LCBA_SCHUR_MMA": "1", "LCBA_SCHUR_I8": "1"}}
 MASKS = ["cam0_extrinsics", "intrinsics", "random30", "whole_camera", "camera_sees_held_points", "points10"]
@@ -61,7 +61,7 @@ def _held(cam, pt):
 def test_masked_step_matches_oracle_on_every_route(Engine, monkeypatch, record_property, C, kind):
     """lcba_debug_step with masks against the damped normal equations of J[:, free] (test_gpu_step._check_step:
     normal-equation residual 1e-11, forward error 1e-11 cond, reg_term / Jg2 / Delta, Gram totals 1e-12,
-    subspace scalars), on the pass routes pt / generic / dense and the Schur routes DFMA / DMMA / int8.  Held
+    subspace scalars), on the pass routes pt / generic and the Schur routes DFMA / DMMA / int8.  Held
     entries of the step are exactly 0; the steps agree over the routes to max(1e-12, 1e-13 cond) scaled.
     Measured on a B200 (1000 W): residual <= 2.8e-14, forward error <= 1.5e-15 cond, Gram totals <= 3.7e-14,
     subspace scalars <= 2.9e-13, routes <= 4.8e-12 (int8)."""
@@ -80,8 +80,6 @@ def test_masked_step_matches_oracle_on_every_route(Engine, monkeypatch, record_p
     p_or = cho_solve(cho_factor(H, lower=True), Jf.T @ f)
     steps = {}
     for route, env in ROUTES.items():
-        if route == "dense" and C < 8:
-            continue
         for k, v in env.items():
             monkeypatch.setenv(k, v)
         e = Engine()

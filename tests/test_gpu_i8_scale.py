@@ -1,7 +1,7 @@
 """The int8 tensor-core Schur path (schur_i8.cuh: k_i8_rowmax, k_i8_make, k_i8_syrk, k_i8_gather) at the
 shard sizes where it runs by default (>= 32768 points per shard, lcba.cu), against the FP64 DMMA path and
 the numpy oracle: deep K ranges that flush TMEM several times per CTA, the dispatch switch, ragged and tiny
-K, both operand producers, inputs with a hard dynamic range, and point-sharded runs.
+K, inputs with a hard dynamic range, and point-sharded runs.
 
 Every GPU test prints its observed errors as a fraction of their bounds (run pytest with -s to see them).
 The GPU tests of this file take about 45 s on one B200."""
@@ -27,7 +27,6 @@ LAM = 1e-5
 # plan on a 148-SM B200 needs >= 3 TMEM flushes (4 / 5 / 3), so the epilogue sums several flushes and the
 # MMA warp waits on both parities of bar_tempty
 DEPTH_CASES = [("ring24", 150_000, 1.0, False), ("ring64", 40_000, 0.5, True), ("ring8", 600_000, 1.0, True)]
-PRODUCER_CASE = ("ring24", 100_000)            # 3 flushes per CTA
 HARD_KINDS = ["weights", "outliers", "twoview", "near", "nocam", "combined"]
 
 
@@ -52,7 +51,7 @@ def _run(monkeypatch, pb, lam, w=None, env=None, repeat=False):
     int8 result stood, -1 on the DMMA path."""
     from lasercalib_b200._cabi import Engine
     env = env or {}
-    for k in ("LCBA_SCHUR_I8", "LCBA_I8_TMA", "LCBA_SCHUR_MMA", "LCBA_I8_GUARD"):
+    for k in ("LCBA_SCHUR_I8", "LCBA_SCHUR_MMA", "LCBA_I8_GUARD"):
         monkeypatch.delenv(k, raising=False)
     for k, v in env.items():
         monkeypatch.setenv(k, v)
@@ -211,24 +210,7 @@ def test_int8_path_ragged_and_tiny_k(monkeypatch, P):
     _check("ring24 x %d int8 vs oracle" % P, i8, _oracle(pb, 1e-3, w), S=1e-11, rhs=1e-10)
 
 
-# ------------------------------------------------------------------------------ 4. producer variants
-@pytest.mark.gpu
-def test_bulk_copy_producer_equals_tma_producer(monkeypatch):
-    """LCBA_I8_TMA=0 (one 1-D bulk copy per digit and operand; also what runs when tensor-map encoding fails)
-    loads the same bytes as the TMA tensor copies and the integer products are exact: S and rhs equal to the
-    bit, at a size with 3 TMEM flushes per CTA (measured so on a B200)."""
-    rig, P = PRODUCER_CASE
-    pb = _subset(make_rig(rig, P + 2000, seed=37, variant="volume", p_vis=1.0), P)
-    assert _flushes(pb["n_cams"], P) >= 3
-    tma, k_tma = _run(monkeypatch, pb, LAM)
-    bulk, k_bulk = _run(monkeypatch, pb, LAM, env={"LCBA_I8_TMA": "0"})
-    assert "i8_rowmax" in k_tma and "i8_rowmax" in k_bulk and tma["fell_back"] == 0 == bulk["fell_back"]
-    np.testing.assert_array_equal(bulk["S"], tma["S"])
-    np.testing.assert_array_equal(bulk["rhs"], tma["rhs"])
-    print("%s x %d: bulk-copy producer bit-identical to the TMA producer" % (rig, P))
-
-
-# ---------------------------------------------------------------------------- 5. hard dynamic range
+# ---------------------------------------------------------------------------- 4. hard dynamic range
 def _hard_problem(rig, kinds, P=33_000, seed=41):
     """A rig of P points (plus the near-camera ones) with the inputs that stress the row exponents of the int8
     path (an FP32 estimate of each row maximum, 1e-3 of slack and 2 bits of headroom):
@@ -374,7 +356,7 @@ def test_default_int8_path_on_hard_inputs(monkeypatch, rig, kind):
     _check(label + " int8 vs DMMA", i8, dm, jacobi=1e-12)
 
 
-# ------------------------------------------------------------------------------------------ 6. sharded
+# ------------------------------------------------------------------------------------------ 5. sharded
 @pytest.mark.gpu
 def test_point_sharded_int8_path_matches_single_gpu():
     """Two shards of 40 k points (ring24), each on the int8 path, against the single-GPU run of the same
@@ -397,11 +379,11 @@ def test_point_sharded_int8_path_matches_single_gpu():
         assert "rank %d ok" % r in out.stdout
 
 
-# ----------------------------------------------------------------------------------- 7. CPU: the plans
+# ----------------------------------------------------------------------------------- 6. CPU: the plans
 def test_int8_plans_of_the_scale_tests(lib):
     """Host logic only (make_i8_plan through lcba_debug_i8_plan, 148 SMs as on a B200): the sizes the GPU
     tests above use give the flush counts they rely on, and the two sizes around the dispatch switch plan."""
-    for rig, P, _, _ in DEPTH_CASES + [PRODUCER_CASE + (None, None)]:
+    for rig, P, _, _ in DEPTH_CASES:
         C = sum(r["n"] for r in RIGS[rig]["rings"])
         assert _flushes(C, P, sm_count=148) >= 3, (rig, P)
     for P in (I8_SWITCH - 1, I8_SWITCH):

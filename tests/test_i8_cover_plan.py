@@ -3,8 +3,8 @@ with a two-range A operand instead of row strips with square diagonal blocks.
 
 Host logic (no GPU): the tiles take every lower-triangle entry exactly once under k_i8_gather's rule, the
 shapes fit the kernel, the K ranges form one wave, and the plan that runs is never slower in the cost model
-than the strip plan.  On the GPU: the cover plan against the strip plan, the FP64 DMMA path and itself (both
-operand producers, two calls), at depth."""
+than the strip plan.  On the GPU: the cover plan against the strip plan, the FP64 DMMA path and itself (two
+calls), at depth."""
 import math
 import os
 
@@ -53,6 +53,15 @@ def _taken(pl, C):
     return cnt
 
 
+def _map_shapes(pl):
+    """The tensor-map shapes (box height in row groups, distance of A's second row range or 0) that i8_deal
+    makes for a plan's tiles, restated: A, column block 1 and column block 2; a height of 0 needs no map."""
+    shapes = set()
+    for m0, mn, m20, m2n, n0, nn, n20, n2n, _, _ in pl["tiles"]:
+        shapes |= {(int(mn), int(m20 - m0) if m2n else 0), (int(nn), 0), (int(n2n), 0)}
+    return {s for s in shapes if s[0] > 0}
+
+
 def test_cover_plan_takes_each_lower_entry_once():
     """For every camera count and size, every lower-triangle entry of the (11 C + 1)-row matrix (the z row
     included, its diagonal excluded) is written exactly once and nothing above the diagonal; the strip plan
@@ -72,7 +81,8 @@ def test_cover_plan_shapes_k_ranges_and_choice():
     """Column blocks are multiples of 16 columns, at most 64 in all; A has at most 16 row groups, and two
     ranges only of 8 row groups each in increasing order (the 5-D tensor-map box); every tile's K ranges
     partition [0, nkb) and the grid is one wave; the plan that runs (no LCBA_I8_PLAN) costs no more in the
-    model than the strip plan and reports the executed ops of its tiles.  24 cameras: 8 tiles, the model's
+    model than the strip plan and reports the executed ops of its tiles; both plans need at most 16 tensor-map
+    shapes (I8_MAX_MAPS in schur_i8.cuh: i8_encode_maps fails beyond that).  24 cameras: 8 tiles, the model's
     slowest CTA 17 % below the strip plan's, 7.47e12 executed int8 ops per launch at 1 M points (strip
     8.76e12)."""
     for C in CAMS:
@@ -91,6 +101,8 @@ def test_cover_plan_shapes_k_ranges_and_choice():
                 assert w[0, 1] == 0 and w[-1, 2] == nkb and (w[1:, 1] == w[:-1, 2]).all() and (w[:, 2] > w[:, 1]).all()
                 cols += 8 * int(nn + n2n)
             assert pl["executed_ops"] == 26 * 2 * 128 * cols * 64 * nkb
+            for which, p in ((1, _plan(C, P, 1)), (2, pl)):
+                assert len(_map_shapes(p)) <= 16, (C, P, which, sorted(_map_shapes(p)))
             chosen = _plan(C, P, 0)
             assert chosen["cycles"] <= chosen["strip_cycles"], (C, P)
             assert chosen["cover"] == (chosen["cover_cycles"] < chosen["strip_cycles"])
@@ -114,7 +126,7 @@ def _run(monkeypatch, pb, w, env, repeat=False):
     """linearize(LAM) at x0 under `env`; out["kernels"]: the kernels of one solver iteration, out["fell_back"]
     as in test_gpu_i8_scale."""
     from lasercalib_b200._cabi import Engine
-    for k in ("LCBA_SCHUR_I8", "LCBA_I8_TMA", "LCBA_SCHUR_MMA", "LCBA_I8_GUARD", "LCBA_I8_PLAN"):
+    for k in ("LCBA_SCHUR_I8", "LCBA_SCHUR_MMA", "LCBA_I8_GUARD", "LCBA_I8_PLAN"):
         monkeypatch.delenv(k, raising=False)
     for k, v in env.items():
         monkeypatch.setenv(k, v)
@@ -189,16 +201,3 @@ def test_cover_plan_equals_strip_plan_and_dmma(monkeypatch, rig, P, pvis, weight
     if (rig, P) == ("ring24", 1_000_000):
         dflt = _run(monkeypatch, pb, w, {})
         np.testing.assert_array_equal(dflt["S"], cv["S"])
-
-
-@pytest.mark.gpu
-def test_cover_plan_tma_and_bulk_copy_producers_bit_identical(monkeypatch):
-    """The cover plan's A operand of two row ranges through the 5-D tensor map and through two 1-D bulk
-    copies per digit (LCBA_I8_TMA=0): S and rhs bit-identical, ring24 and ring64."""
-    for rig, P, pvis in (("ring24", 200_000, 1.0), ("ring64", 60_000, 0.5)):
-        pb = _subset(make_rig(rig, int(P / pvis * 1.08) + 1000, seed=43, variant="volume", p_vis=pvis), P)
-        tma = _run(monkeypatch, pb, None, {"LCBA_I8_PLAN": "cover"})
-        blk = _run(monkeypatch, pb, None, {"LCBA_I8_PLAN": "cover", "LCBA_I8_TMA": "0"})
-        assert tma["fell_back"] == 0 and blk["fell_back"] == 0
-        np.testing.assert_array_equal(tma["S"], blk["S"])
-        np.testing.assert_array_equal(tma["rhs"], blk["rhs"])
