@@ -149,6 +149,24 @@ int lcba_set_params(lcba_t* h, const double* cams, const double* pts);
  * LCBA_E_UNSUPPORTED, nothing free LCBA_E_ARG.  Sharded jobs: the camera mask must be the same on every
  * rank (lcba_solve compares its count and checksum over the ranks and fails on every rank otherwise). */
 int lcba_set_fixed(lcba_t* h, const uint8_t* cam_fixed, const uint8_t* pt_fixed);
+/* Box bounds lb <= x <= ub (least_squares(bounds=...)): cam_lb / cam_ub C x 11 (row-major like cams), pt_lb /
+ * pt_ub P x 3 over THIS handle's points (its shard on a point-sharded job).  -inf / +inf are allowed; a NULL
+ * array leaves that side unbounded, four NULLs clear the bounds; a NaN bound is LCBA_E_ARG.  When some free entry
+ * has a finite bound, lcba_solve runs scipy's trf_bounds (the reflective TRF, with the exact Schur solve in place of
+ * LSMR): it moves x0 by make_strictly_feasible(x0, lb, ub, rstep=1e-10) first and returns LCBA_E_ARG when lb >= ub
+ * or x0 lies outside the box on a free entry, LCBA_E_UNSUPPORTED together with fix_cameras or shared_intrinsics.
+ * The result's optimality is then |g v|_inf (v: the Coleman-Li vector), step_norm |step|.  Every bound infinite:
+ * the unbounded loop, unchanged.  Held entries (lcba_set_fixed) ignore their bounds.  lcba_debug_step honours the
+ * bounds' damping at the current x, which must lie strictly inside the box (LCBA_E_ARG otherwise).  Cleared by
+ * lcba_set_problem / lcba_set_problem_shard, kept by lcba_set_params.  Sharded jobs: the camera bounds must be the
+ * same on every rank, a rank without bounds counting as all-infinite (lcba_solve compares a checksum over the
+ * ranks and fails on every rank otherwise); when any rank has a finite bound, every rank runs the bounded loop. */
+int lcba_set_bounds(lcba_t* h, const double* cam_lb, const double* cam_ub, const double* pt_lb,
+                    const double* pt_ub);
+/* find_active_constraints(x, lb, ub, rtol) of scipy at the current x over [cams | this handle's points]: one int8
+ * per entry, -1 at a lower bound, 1 at an upper bound, 0 otherwise (held entries and no bounds: 0).  least_squares
+ * reports it with rtol = xtol. */
+int lcba_get_active_mask(lcba_t* h, double rtol, int8_t* out);
 /* PySBA.optimizedParams (pySBA.py:121-129): copy x back, split. */
 int lcba_get_params(lcba_t* h, double* cams_out, double* pts_out);
 

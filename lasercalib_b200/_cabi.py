@@ -23,7 +23,8 @@ SYMBOLS = ["lcba_version", "lcba_create", "lcba_destroy", "lcba_last_error", "lc
            "lcba_sq_normal", "lcba_debug_schur_stats", "lcba_debug_mma_plan",
            "lcba_set_iteration_callback", "lcba_debug_i8_plan", "lcba_host_is_nondecreasing_i64", "lcba_debug_peer_reduce",
            "lcba_debug_i8_fallback", "lcba_debug_chol", "lcba_debug_step", "lcba_debug_i8_cover_plan",
-           "lcba_debug_i8_make", "lcba_set_fixed", "lcba_debug_i8_schedule"]
+           "lcba_debug_i8_make", "lcba_set_fixed", "lcba_debug_i8_schedule", "lcba_set_bounds",
+           "lcba_get_active_mask"]
 
 # scalars_out of lcba_debug_step, in order (include/lcba.h)
 STEP_SCALARS = ["reg_term", "Delta", "Jg2", "aa", "ab", "bb", "JAA", "JAB", "JBB", "gtgt", "gtp", "pp",
@@ -95,6 +96,8 @@ def load():
     lib.lcba_set_params.argtypes = [vp, vp, vp]
     lib.lcba_get_params.argtypes = [vp, vp, vp]
     lib.lcba_set_fixed.argtypes = [vp, vp, vp]
+    lib.lcba_set_bounds.argtypes = [vp, vp, vp, vp, vp]
+    lib.lcba_get_active_mask.argtypes = [vp, dbl, vp]
     lib.lcba_rotate.argtypes = [vp, i64, vp, vp, vp]
     lib.lcba_project.argtypes = [vp, i64, vp, vp, vp]
     lib.lcba_unproject.argtypes = [vp, i64, vp, vp, i64, vp, vp, vp, vp, vp]
@@ -163,6 +166,7 @@ class Engine:
         self.h = h
         self.C = self.P = self.N = 0
         self.has_fixed = False     # a mask of set_fixed is in place (set_problem clears it)
+        self.has_bounds = False    # bounds of set_bounds are in place (set_problem clears them)
         # bumped by every call that changes what the handle holds (observation set or x): lazy
         # readers (res.fun / res.grad / res.jac) compare it with the value they were created at
         self.generation = 0
@@ -200,6 +204,7 @@ class Engine:
                                                     _ptr(pi), _ptr(w), int(pt_offset)))
         self.C, self.P, self.N = cams.shape[0], pts.shape[0], N
         self.has_fixed = False
+        self.has_bounds = False
         self.generation += 1
 
     def set_params(self, cams, pts):
@@ -218,6 +223,20 @@ class Engine:
             raise ValueError("pt_fixed must have shape (%d,)" % self.P)
         self._check(self.lib.lcba_set_fixed(self.h, _ptr(cm), _ptr(pm)))
         self.has_fixed = cm is not None or pm is not None
+
+    def set_bounds(self, cam_lb=None, cam_ub=None, pt_lb=None, pt_ub=None):
+        """Box bounds for solve() and debug_step() (lcba_set_bounds): (C, 11) camera and (P, 3) point arrays over
+        this handle's points, +-inf allowed; None leaves that side unbounded, four None clear the bounds."""
+        arrs = [None if a is None else _f64(a, shape) for a, shape in
+                ((cam_lb, (self.C, 11)), (cam_ub, (self.C, 11)), (pt_lb, (self.P, 3)), (pt_ub, (self.P, 3)))]
+        self._check(self.lib.lcba_set_bounds(self.h, *[_ptr(a) for a in arrs]))
+        self.has_bounds = any(a is not None for a in arrs)
+
+    def active_mask(self, rtol):
+        """find_active_constraints(x, lb, ub, rtol) at the current x (lcba_get_active_mask), int8 (11 C + 3 P,)."""
+        out = np.empty(11 * self.C + 3 * self.P, dtype=np.int8)
+        self._check(self.lib.lcba_get_active_mask(self.h, float(rtol), _ptr(out)))
+        return out
 
     def get_params(self, x_out=None):
         """(cams, pts) of the current iterate; with `x_out` (11 C + 3 P doubles, contiguous) the

@@ -16,7 +16,7 @@ CSRC = os.path.join(PKG, "csrc")
 LIB = os.path.join(PKG, "liblcba.so")
 SOURCES = ["lcba.cu"]
 HEADERS = ["common.cuh", "model.cuh", "eval.cuh", "ingest.cuh", "linearize.cuh", "schur.cuh", "schur_mma.cuh", "schur_i8.cuh", "peer_reduce.cuh",
-           "dense.cuh", "dense_passes.cuh", "control.cuh", "variants.cuh", os.path.join("..", "..", "include", "lcba.h")]
+           "dense.cuh", "dense_passes.cuh", "control.cuh", "variants.cuh", "bounds.cuh", os.path.join("..", "..", "include", "lcba.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared", "-diag-suppress", "177"]
 

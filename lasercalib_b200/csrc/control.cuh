@@ -184,9 +184,10 @@ __global__ void k_ctl_lin2(const double* __restrict__ red, Ctl* __restrict__ ctl
   }
 }
 
-// reg_term from the 1-D Cauchy model (trf.py:488-492, common.py:251-322)
-__global__ void k_ctl_reg(const double* __restrict__ red, Ctl* __restrict__ ctl) {
-  const double Jg2 = red[0];
+// reg_term from the 1-D Cauchy model (trf.py:488-492, common.py:251-322).  dhg2 (bounded loop only, else NULL):
+// sum diag_h g_h^2, the diagonal's share of the model's curvature (trf.py:327)
+__global__ void k_ctl_reg(const double* __restrict__ red, Ctl* __restrict__ ctl, const double* __restrict__ dhg2) {
+  const double Jg2 = dhg2 ? red[0] + *dhg2 : red[0];
   ctl->Jg2 = Jg2;
   const double a = 0.5 * Jg2, b = -ctl->gh2;
   const double ub = ctl->Delta / sqrt(ctl->gh2);

@@ -25,6 +25,7 @@
 #include "schur_i8.cuh"
 #include "peer_reduce.cuh"
 #include "variants.cuh"
+#include "bounds.cuh"
 
 using namespace lcba;
 
@@ -41,7 +42,7 @@ struct NcclApi {
   const char* (*GetErrorString)(int) = nullptr;
 };
 static NcclApi g_nccl;
-static const int NCCL_FLOAT64 = 8, NCCL_SUM = 0, NCCL_MAX = 2, NCCL_INT64 = 4;
+static const int NCCL_FLOAT64 = 8, NCCL_SUM = 0, NCCL_MAX = 2, NCCL_MIN = 3, NCCL_INT64 = 4;
 
 static bool nccl_load(std::string& err) {
   if (g_nccl.lib) return true;
@@ -164,6 +165,15 @@ struct lcba_handle {
   long long n_cam_held = 0, n_pt_held = 0;
   double cam_fixed_sum = 0.0;      // checksum of the camera mask (the same on every rank of a sharded job)
   bool masks_on = true;
+  std::vector<uint8_t> h_cam_fixed, h_pt_fixed;   // host copies of the masks (empty: nothing held)
+  // box bounds (lcba_set_bounds): host copies over [cameras | points], -inf / +inf where a side is unbounded.  The
+  // device buffers (effective box with held entries unbounded, then the bounded loop's per-entry vectors and
+  // scalars) are allocated by the first bounded solve; `bounded`: the current solve or debug step runs that loop.
+  std::vector<double> h_lb, h_ub;
+  bool has_bounds = false, bounded = false;
+  double *d_blb = nullptr, *d_bub = nullptr, *d_bsd = nullptr, *d_bdh = nullptr, *d_bp = nullptr, *d_br = nullptr;
+  double* d_bred = nullptr;   // [0,6) linearise  [6,9) Gram diagonal  [9,11) step in box  [11,17) reflection  [17,19) J pass
+  Bnd* d_bnd = nullptr;
   double *d_pred = nullptr, *d_scl_red = nullptr;   // shared-intrinsics mode: reduced step / scale
   double *d_sqpart = nullptr, *d_sqout = nullptr, *d_theta = nullptr;   // squared-residual variants
   int sq_grid = 0, sq_K = 0;
@@ -256,7 +266,7 @@ static int check_launch(lcba_t* h, const char* what) {
 
 static int allreduce(lcba_t* h, double* p, size_t n, int op) {
   if (!h->comm) return LCBA_OK;
-  if (g_peer.ok && n <= PEER_SLOT) {
+  if (g_peer.ok && n <= PEER_SLOT && op != NCCL_MIN) {
     // one kernel over NVLink peer memory (peer_reduce.cuh); same call order on every rank, like NCCL
     ++g_peer.epoch;
     k_peer_allreduce<<<peer_grid(n), PEER_THREADS, 0, h->stream>>>(g_peer.ptrs, h->rank, h->nranks, g_peer.epoch, p, n,
@@ -422,6 +432,11 @@ extern "C" int lcba_set_problem_shard(lcba_t* h, int32_t C, int64_t P, int64_t N
   LCBA_CUDA(h, cudaMemsetAsync(h->d_pt_fixed, 0, (size_t)P, h->stream));
   h->n_cam_held = h->n_pt_held = 0;
   h->cam_fixed_sum = 0.0;
+  h->h_cam_fixed.clear(); h->h_pt_fixed.clear();
+  h->h_lb.clear(); h->h_ub.clear();
+  h->has_bounds = h->bounded = false;
+  h->d_blb = h->d_bub = h->d_bsd = h->d_bdh = h->d_bp = h->d_br = h->d_bred = nullptr;
+  h->d_bnd = nullptr;
 
   // temporaries (freed at the end of ingest)
   long long *t_cam = nullptr, *t_pt = nullptr;
@@ -720,6 +735,8 @@ extern "C" int lcba_set_fixed(lcba_t* h, const uint8_t* cam_fixed, const uint8_t
     LCBA_CUDA(h, cudaMemsetAsync(h->d_pt_fixed, 0, (size_t)h->P, h->stream));
   }
   LCBA_CUDA(h, cudaStreamSynchronize(h->stream));
+  if (cam_fixed) h->h_cam_fixed.assign(cam_fixed, cam_fixed + nc); else h->h_cam_fixed.clear();
+  if (pt_fixed) h->h_pt_fixed.assign(pt_fixed, pt_fixed + h->P); else h->h_pt_fixed.clear();
   h->n_cam_held = nch;
   h->n_pt_held = nph;
   h->cam_fixed_sum = (double)chk;
@@ -728,6 +745,161 @@ extern "C" int lcba_set_fixed(lcba_t* h, const uint8_t* cam_fixed, const uint8_t
 
 static const uint8_t* cam_mask(const lcba_t* h) { return h->masks_on ? h->d_cam_fixed : nullptr; }
 static const uint8_t* pt_mask(const lcba_t* h) { return h->masks_on ? h->d_pt_fixed : nullptr; }
+
+extern "C" int lcba_set_bounds(lcba_t* h, const double* cam_lb, const double* cam_ub, const double* pt_lb,
+                               const double* pt_ub) {
+  if (!h || !h->have_problem) { set_error(h, "lcba_set_bounds: no problem set"); return LCBA_E_STATE; }
+  const size_t nc = (size_t)h->C * NCP, n = nc + (size_t)h->P * 3;
+  if (!cam_lb && !cam_ub && !pt_lb && !pt_ub) {
+    h->h_lb.clear(); h->h_ub.clear();
+    h->has_bounds = false;
+    return LCBA_OK;
+  }
+  std::vector<double> lb(n, -INFINITY), ub(n, INFINITY);
+  if (cam_lb) std::copy(cam_lb, cam_lb + nc, lb.begin());
+  if (cam_ub) std::copy(cam_ub, cam_ub + nc, ub.begin());
+  if (pt_lb) std::copy(pt_lb, pt_lb + (n - nc), lb.begin() + nc);
+  if (pt_ub) std::copy(pt_ub, pt_ub + (n - nc), ub.begin() + nc);
+  for (size_t i = 0; i < n; ++i)
+    if (std::isnan(lb[i]) || std::isnan(ub[i])) { set_error(h, "lcba_set_bounds: a bound is NaN"); return LCBA_E_ARG; }
+  h->h_lb.swap(lb);
+  h->h_ub.swap(ub);
+  h->has_bounds = true;
+  return LCBA_OK;
+}
+
+// find_active_constraints (scipy/optimize/_lsq/common.py:414-456) of one entry: -1 lower, 1 upper, 0 neither
+static int active_of(double x, double lb, double ub, double rtol) {
+  if (rtol == 0.0) return x >= ub ? 1 : (x <= lb ? -1 : 0);
+  const double ld = x - lb, ud = ub - x;
+  int a = 0;
+  if (std::isfinite(lb) && ld <= std::min(ud, rtol * std::max(1.0, std::fabs(lb)))) a = -1;
+  if (std::isfinite(ub) && ud <= std::min(ld, rtol * std::max(1.0, std::fabs(ub)))) a = 1;
+  return a;
+}
+
+// the box the solver sees: held entries (and every camera entry under fix_cameras) unbounded
+static void effective_bounds(const lcba_t* h, bool cams_held, std::vector<double>& lb, std::vector<double>& ub) {
+  const size_t nc = (size_t)h->C * NCP, n = nc + (size_t)h->P * 3;
+  lb = h->h_lb; ub = h->h_ub;
+  for (size_t i = 0; i < n; ++i) {
+    const bool held = i < nc ? (cams_held || (!h->h_cam_fixed.empty() && h->h_cam_fixed[i]))
+                             : (!h->h_pt_fixed.empty() && h->h_pt_fixed[(i - nc) / 3]);
+    if (held) { lb[i] = -INFINITY; ub[i] = INFINITY; }
+  }
+}
+
+static int download_x(lcba_t* h, std::vector<double>& x) {
+  const size_t nc = (size_t)h->C * NCP;
+  x.resize(nc + (size_t)h->P * 3);
+  LCBA_CUDA(h, cudaMemcpyAsync(x.data(), h->d_cams[h->cur], nc * 8, cudaMemcpyDeviceToHost, h->stream));
+  LCBA_CUDA(h, cudaMemcpyAsync(x.data() + nc, h->d_pts[h->cur], (size_t)h->P * 3 * 8, cudaMemcpyDeviceToHost, h->stream));
+  LCBA_CUDA(h, cudaStreamSynchronize(h->stream));
+  return LCBA_OK;
+}
+
+// checksum of the camera part [0, nc) of a box: equal boxes give equal sums on every rank
+static double cam_box_sum(const double* lb, const double* ub, size_t nc) {
+  uint32_t chk = 2166136261u;
+  for (size_t i = 0; i < nc; ++i) {
+    uint64_t bits[2];
+    memcpy(&bits[0], &lb[i], 8);
+    memcpy(&bits[1], &ub[i], 8);
+    for (int k = 0; k < 2; ++k) chk = (chk ^ (uint32_t)(bits[k] ^ (bits[k] >> 32))) * 16777619u;
+  }
+  return (double)chk;
+}
+
+// Local part of a bounded solve's set-up: the effective box and the current x.  flags: 1 = a finite bound on a free
+// entry (the bounded loop runs), 2 = lb >= ub on such an entry, 4 = x outside the box there, 8 = x outside or on the
+// boundary there.  cam_sum: checksum of the camera part of the box (must be the same on every rank of a sharded job;
+// a handle without bounds has the all-infinite box, so its sum equals that of a rank with infinite camera bounds).
+struct BoxSetup { std::vector<double> x, lb, ub; int flags = 0; double cam_sum = 0.0; };
+static int box_setup(lcba_t* h, bool cams_held, BoxSetup& b) {
+  const size_t nc = (size_t)h->C * NCP;
+  b.flags = 0;
+  b.x.clear();
+  if (!h->has_bounds) {
+    b.lb.clear(); b.ub.clear();
+    const std::vector<double> lo(nc, -INFINITY), hi(nc, INFINITY);
+    b.cam_sum = cam_box_sum(lo.data(), hi.data(), nc);
+    return LCBA_OK;
+  }
+  effective_bounds(h, cams_held, b.lb, b.ub);
+  LCBA_TRY(download_x(h, b.x));
+  const size_t n = b.x.size();
+  b.cam_sum = cam_box_sum(b.lb.data(), b.ub.data(), nc);
+  for (size_t i = 0; i < n; ++i) {
+    const double l = b.lb[i], u = b.ub[i];
+    if (!std::isfinite(l) && !std::isfinite(u)) continue;
+    b.flags |= 1;
+    if (!(l < u)) b.flags |= 2;
+    else if (!(b.x[i] >= l && b.x[i] <= u)) b.flags |= 4 | 8;
+    else if (!(b.x[i] > l && b.x[i] < u)) b.flags |= 8;
+  }
+  return LCBA_OK;
+}
+
+// Device side of a bounded solve: buffers on first use, the box, and (move_x) x0 moved by
+// make_strictly_feasible(x0, lb, ub, rstep=1e-10) as least_squares does before trf_bounds.
+static int box_upload(lcba_t* h, BoxSetup& b, bool move_x) {
+  const size_t nc = (size_t)h->C * NCP, n = nc + (size_t)h->P * 3;
+  if (b.lb.empty()) {            // no bounds on this rank while another rank has some: the all-infinite box
+    b.lb.assign(n, -INFINITY);
+    b.ub.assign(n, INFINITY);
+    move_x = false;
+  }
+  if (!h->d_blb) {
+    LCBA_TRY(dev_alloc(h, &h->d_blb, n));
+    LCBA_TRY(dev_alloc(h, &h->d_bub, n));
+    LCBA_TRY(dev_alloc(h, &h->d_bsd, n));
+    LCBA_TRY(dev_alloc(h, &h->d_bdh, n));
+    LCBA_TRY(dev_alloc(h, &h->d_bp, n));
+    LCBA_TRY(dev_alloc(h, &h->d_br, n));
+    LCBA_TRY(dev_alloc(h, &h->d_bred, 32));
+    LCBA_TRY(dev_alloc(h, &h->d_bnd, 1));
+  }
+  LCBA_CUDA(h, cudaMemcpyAsync(h->d_blb, b.lb.data(), n * 8, cudaMemcpyHostToDevice, h->stream));
+  LCBA_CUDA(h, cudaMemcpyAsync(h->d_bub, b.ub.data(), n * 8, cudaMemcpyHostToDevice, h->stream));
+  if (move_x) {
+    const double rstep = 1e-10;
+    bool moved = false;
+    for (size_t i = 0; i < n; ++i) {
+      const double l = b.lb[i], u = b.ub[i];
+      const int a = active_of(b.x[i], l, u, rstep);
+      double xn = b.x[i];
+      if (a == -1) xn = l + rstep * std::max(1.0, std::fabs(l));
+      else if (a == 1) xn = u - rstep * std::max(1.0, std::fabs(u));
+      if (xn < l || xn > u) xn = 0.5 * (l + u);
+      if (xn != b.x[i]) { b.x[i] = xn; moved = true; }
+    }
+    if (moved) {
+      LCBA_CUDA(h, cudaMemcpyAsync(h->d_cams[h->cur], b.x.data(), nc * 8, cudaMemcpyHostToDevice, h->stream));
+      LCBA_CUDA(h, cudaMemcpyAsync(h->d_pts[h->cur], b.x.data() + nc, (n - nc) * 8, cudaMemcpyHostToDevice, h->stream));
+    }
+  }
+  LCBA_CUDA(h, cudaStreamSynchronize(h->stream));
+  return LCBA_OK;
+}
+
+extern "C" int lcba_get_active_mask(lcba_t* h, double rtol, int8_t* out) {
+  if (!h || !h->have_problem) { set_error(h, "lcba_get_active_mask: no problem set"); return LCBA_E_STATE; }
+  if (!out) { set_error(h, "lcba_get_active_mask: out is NULL"); return LCBA_E_ARG; }
+  cudaSetDevice(h->device);
+  const size_t n = (size_t)h->C * NCP + (size_t)h->P * 3;
+  if (!h->has_bounds) { memset(out, 0, n); return LCBA_OK; }
+  std::vector<double> x, lb, ub;
+  effective_bounds(h, h->fix_cameras != 0, lb, ub);
+  LCBA_TRY(download_x(h, x));
+  for (size_t i = 0; i < n; ++i) out[i] = (int8_t)active_of(x[i], lb[i], ub[i], rtol);
+  return LCBA_OK;
+}
+
+// per-entry vectors in the bounded loop: 1 / d and diag_h in place of the Jacobi scale and nothing
+static const double* sd_c(const lcba_t* h) { return h->bounded ? h->d_bsd : h->d_scl_c; }
+static const double* sd_p(const lcba_t* h) { return h->bounded ? h->d_bsd + (size_t)h->C * NCP : h->d_scl_p; }
+static const double* dh_c(const lcba_t* h) { return h->bounded ? h->d_bdh : nullptr; }
+static const double* dh_p(const lcba_t* h) { return h->bounded ? h->d_bdh + (size_t)h->C * NCP : nullptr; }
 
 extern "C" int lcba_get_params(lcba_t* h, double* cams_out, double* pts_out) {
   if (!h || !h->have_problem) { set_error(h, "lcba_get_params: no problem set"); return LCBA_E_STATE; }
@@ -921,6 +1093,15 @@ extern "C" int lcba_jacobian_blocks(lcba_t* h, const double* x_or_null, double* 
 }
 
 // ------------------------------------------------------------------------------ solver passes
+// Reduce the columns of a bounded pass's partials (k_reduce_ops) into out[0..K) and all-reduce them over the ranks.
+static int reduce_ops(lcba_t* h, const double* part, int nblocks, int K, int nsum, int nmax, double* out) {
+  KL(h, "reduce", k_reduce_ops<<<K, 256, 0, h->stream>>>(part, nblocks, K, nsum, nmax, out));
+  if (nsum) LCBA_TRY(allreduce(h, out, nsum, NCCL_SUM));
+  if (nmax) LCBA_TRY(allreduce(h, out + nsum, nmax, NCCL_MAX));
+  if (K > nsum + nmax) LCBA_TRY(allreduce(h, out + nsum + nmax, K - nsum - nmax, NCCL_MIN));
+  return LCBA_OK;
+}
+
 static int pass_linearize(lcba_t* h, int first) {
   NvtxRange nvtx_("lcba:linearize");
   const int C = h->C, w = h->cur;
@@ -946,6 +1127,18 @@ static int pass_linearize(lcba_t* h, int first) {
         h->d_campart, h->lin_grid, C * CAMSUM, h->d_camsum));
   KL(h, "reduce", k_reduce_scalars<<<1, 256, 0, h->stream>>>(h->d_part, h->lin_grid, 1,
                                                              h->d_camsum + C * CAMSUM, 1));
+  }
+  if (h->bounded) {
+    const size_t nc = (size_t)C * NCP;
+    KL(h, "point_prep", k_bnd_point_prep<<<h->pt_grid, 256, 0, h->stream>>>(
+          h->d_Vg, h->d_pts[w], h->d_scl_p, h->d_gt_p, h->P, first, pt_mask(h), h->d_blb + nc, h->d_bub + nc,
+          h->d_bsd + nc, h->d_bdh + nc, h->d_part));
+    LCBA_TRY(reduce_ops(h, h->d_part, h->pt_grid, BPP_K, 4, 1, h->d_bred));
+    LCBA_TRY(allreduce(h, h->d_camsum, (size_t)C * CAMSUM + 1, NCCL_SUM));
+    KL(h, "ctl", k_bnd_ctl_lin<<<1, 256, 0, h->stream>>>(h->d_camsum, h->d_cams[w], h->d_scl_c, h->d_gt_c, h->d_g_c, C,
+                                                         cam_mask(h), h->d_blb, h->d_bub, h->d_bsd, h->d_bdh,
+                                                         h->d_bred, h->d_ctl, h->d_bnd, first));
+    return check_launch(h, "linearize pass");
   }
   // per-point scaling does not depend on the camera sums: run it first so that ONE sum
   // all-reduce carries [camera sums | cost | point sums] and one max all-reduce |g|_inf
@@ -976,7 +1169,7 @@ static int pass_jdot(lcba_t* h) {
   KL(h, "reduce", k_reduce_scalars<<<1, 256, 0, h->stream>>>(h->d_part, h->obs_grid, 1, h->d_red, 1));
   }
   LCBA_TRY(allreduce(h, h->d_red, 1, NCCL_SUM));
-  KL(h, "ctl", k_ctl_reg<<<1, 1, 0, h->stream>>>(h->d_red, h->d_ctl));
+  KL(h, "ctl", k_ctl_reg<<<1, 1, 0, h->stream>>>(h->d_red, h->d_ctl, h->bounded ? &h->d_bnd->dhg2 : nullptr));
   return check_launch(h, "jdot pass");
 }
 
@@ -1009,7 +1202,7 @@ static int pass_schur(lcba_t* h, const double* lam_host_or_null) {
   const double lam_arg = lam_host_or_null ? *lam_host_or_null : 0.0;
   const Ctl* ctl_arg = lam_host_or_null ? nullptr : h->d_ctl;
   KL(h, "point_factor", k_point_factor<<<nblk(h->P, 256), 256, 0, h->stream>>>(
-        h->d_Vg, h->d_scl_p, lam_arg, ctl_arg, h->P, pt_mask(h), h->d_Lz));
+        h->d_Vg, sd_p(h), lam_arg, ctl_arg, h->P, pt_mask(h), dh_p(h), h->d_Lz));
   if (h->use_mma) {
     // dense rigs: SYRK on the FP64 tensor path + the camera blocks U from their own pass
     const MmaPlan& mp = h->mplan;
@@ -1107,7 +1300,7 @@ static int pass_schur(lcba_t* h, const double* lam_host_or_null) {
           h->d_scl_red));
   } else {
     KL(h, "assemble", k_assemble_S<<<nblk((long long)n * n, 256), 256, 0, h->stream>>>(
-          h->d_Sred, C, pl.npairs, h->d_camsum, h->d_scl_c, lam_arg, ctl_arg, cam_mask(h), h->d_S, h->d_rhs));
+          h->d_Sred, C, pl.npairs, h->d_camsum, sd_c(h), lam_arg, ctl_arg, cam_mask(h), dh_c(h), h->d_S, h->d_rhs));
   }
   return check_launch(h, "schur pass");
 }
@@ -1169,18 +1362,25 @@ static int pass_backsub(lcba_t* h) {
   if (h->use_pt) {
     const size_t smem = ((size_t)C * CAMTAB + 2 * (size_t)C * NCP) * 8;
     KL(h, "backsub", k_backsub_pt<<<h->ptp_grid, PT_THREADS, smem, h->stream>>>(
-          h->d_tab[w], h->d_pts[w], h->d_w, h->d_obs_start, h->d_mask, h->P, C, h->d_Vg, h->d_Lz, h->d_scl_p,
+          h->d_tab[w], h->d_pts[w], h->d_w, h->d_obs_start, h->d_mask, h->P, C, h->d_Vg, h->d_Lz, sd_p(h),
           h->d_gt_c, h->d_gt_p, h->d_pc, h->d_gn_p, h->d_part));
     KL(h, "reduce", k_reduce_scalars<<<BS_K, 256, 0, h->stream>>>(h->d_part, h->ptp_grid, BS_K, h->d_red, BS_K));
   } else {
   const size_t smem = ((size_t)C * CAMTAB + 2 * (size_t)C * NCP + 2 * LIN_THREADS * 3) * 8;
   KL(h, "backsub", k_backsub<<<h->lin_grid, LIN_THREADS, smem, h->stream>>>(
         h->d_tab[w], h->d_pts[w], h->d_cam, h->d_pt, h->d_w, h->d_obs_start, h->d_bins, h->nbins, C,
-        h->d_Vg, h->d_Lz, h->d_scl_p, h->d_gt_c, h->d_gt_p, h->d_pc, h->d_gn_p, h->d_part));
+        h->d_Vg, h->d_Lz, sd_p(h), h->d_gt_c, h->d_gt_p, h->d_pc, h->d_gn_p, h->d_part));
   KL(h, "reduce", k_reduce_scalars<<<BS_K, 256, 0, h->stream>>>(h->d_part, h->lin_grid, BS_K, h->d_red, BS_K));
   }
   LCBA_TRY(allreduce(h, h->d_red, BS_K, NCCL_SUM));
-  KL(h, "ctl", k_ctl_sub<<<1, 256, 0, h->stream>>>(h->d_red, h->d_g_c, h->d_gt_c, h->d_pc, h->d_scl_c, C,
+  if (h->bounded) {   // B_S gains S^T diag_h S: added to the Gram totals JAA, JAB, JBB
+    const int nc = C * NCP;
+    KL(h, "bnd_gram", k_bnd_gram<<<h->pt_grid, 256, 0, h->stream>>>(
+          h->d_g_c, h->d_pc, h->d_Vg, h->d_gn_p, h->d_bsd, h->d_bdh, nc, nc + h->P * 3, h->rank == 0, h->d_part));
+    LCBA_TRY(reduce_ops(h, h->d_part, h->pt_grid, 3, 3, 0, h->d_bred + 6));
+    KL(h, "ctl", k_bnd_gram_add<<<1, 1, 0, h->stream>>>(h->d_red, h->d_bred + 6));
+  }
+  KL(h, "ctl", k_ctl_sub<<<1, 256, 0, h->stream>>>(h->d_red, h->d_g_c, h->d_gt_c, h->d_pc, sd_c(h), C,
                                                    h->d_ctl, h->d_fail, h->d_coef, h->shared_intr));
   return check_launch(h, "backsub pass");
 }
@@ -1189,10 +1389,34 @@ static int pass_trial(lcba_t* h) {
   NvtxRange nvtx_("lcba:trial");
   const int w = h->cur, t = 1 - h->cur;
   const long long nc = (long long)h->C * NCP, np = h->P * 3;
+  if (h->bounded) {
+    // select_step: the subspace step, its reflection off the first bound it crosses (the reflection's J pass only
+    // does work when the step leaves the box) and the anti-gradient; then the strictly feasible trial point
+    const int C = h->C;
+    const long long n = nc + np;
+    KL(h, "bnd_select", k_bnd_a<<<h->pt_grid, 256, 0, h->stream>>>(
+          h->d_cams[w], h->d_pts[w], h->d_gt_c, h->d_gt_p, h->d_pc, h->d_gn_p, h->d_coef, h->d_blb, h->d_bub, (int)nc,
+          n, h->d_bp, h->d_part));
+    LCBA_TRY(reduce_ops(h, h->d_part, h->pt_grid, 2, 0, 1, h->d_bred + 9));
+    KL(h, "ctl", k_bnd_ctl_a<<<1, 1, 0, h->stream>>>(h->d_bred + 9, h->d_bnd));
+    KL(h, "bnd_select", k_bnd_b<<<h->pt_grid, 256, 0, h->stream>>>(
+          h->d_cams[w], h->d_pts[w], h->d_g_c, h->d_Vg, h->d_bp, h->d_bsd, h->d_bdh, h->d_blb, h->d_bub, (int)nc, n,
+          h->rank == 0, h->d_bnd, h->d_br, h->d_part));
+    LCBA_TRY(reduce_ops(h, h->d_part, h->pt_grid, BB_K, 5, 0, h->d_bred + 11));
+    const size_t smem = ((size_t)C * CAMTAB + 2 * (size_t)C * NCP) * 8;
+    KL(h, "bnd_jdot", k_bnd_jdot<<<h->obs_grid, 256, smem, h->stream>>>(
+          h->d_tab[w], h->d_pts[w], h->d_cam, h->d_pt, h->d_w, h->d_bp, h->d_br, h->N, C, h->d_bnd, h->d_part));
+    LCBA_TRY(reduce_ops(h, h->d_part, h->obs_grid, 2, 2, 0, h->d_bred + 17));
+    KL(h, "ctl", k_bnd_select<<<1, 1, 0, h->stream>>>(h->d_bred + 11, h->d_bred + 17, h->d_ctl, h->d_bnd));
+    KL(h, "make_trial", k_bnd_trial<<<h->pt_grid, 256, 0, h->stream>>>(
+          h->d_cams[w], h->d_pts[w], h->d_gt_c, h->d_gt_p, h->d_bp, h->d_blb, h->d_bub, (int)nc, n, h->d_bnd,
+          h->d_cams[t], h->d_pts[t]));
+  } else {
   KL(h, "make_trial", k_make_trial<<<1, 256, 0, h->stream>>>(h->d_cams[w], h->d_gt_c, h->d_pc, h->d_coef, nc,
                                                              h->d_cams[t]));
   KL(h, "make_trial", k_make_trial<<<h->pt_grid, 256, 0, h->stream>>>(h->d_pts[w], h->d_gt_p, h->d_gn_p,
                                                                       h->d_coef, np, h->d_pts[t]));
+  }
   LCBA_TRY(build_tables(h, t));
   LCBA_TRY(run_residual(h, t, nullptr));
   KL(h, "ctl", k_ctl_trial<<<1, 1, 0, h->stream>>>(h->d_red, h->d_ctl, h->d_coef));
@@ -1279,14 +1503,21 @@ extern "C" int lcba_solve(lcba_t* h, const lcba_options* opt_in, lcba_result* re
   h->prof_on = opt.profile != 0;
   const long long launches0 = h->launches, replays0 = h->graph_replays;
   long long pt_held_total = h->n_pt_held;
+  h->fix_cameras = opt.fix_cameras ? 1 : 0;
+  h->shared_intr = (opt.shared_intrinsics && !h->fix_cameras) ? 1 : 0;
+  h->masks_on = true;
+  BoxSetup box;
+  LCBA_TRY(box_setup(h, h->fix_cameras != 0, box));
   if (h->comm) {
-    // total point and held-point counts over the ranks (max_nfev = 100 n_free); the camera mask must be the
-    // same on every rank: max of (count, checksum) and of their negatives, so that every rank sees a mismatch
-    double v[6] = {(double)h->P, (double)h->n_pt_held, (double)h->n_cam_held, h->cam_fixed_sum,
-                   -(double)h->n_cam_held, -h->cam_fixed_sum};
+    // total point and held-point counts over the ranks (max_nfev = 100 n_free); the camera mask and the camera
+    // bounds must be the same on every rank: max of (count, checksum) and of their negatives, so that every rank
+    // sees a mismatch; the box flags of box_setup: max over the ranks (every rank runs the same loop and fails alike)
+    double v[10] = {(double)h->P, (double)h->n_pt_held, (double)h->n_cam_held, h->cam_fixed_sum,
+                    -(double)h->n_cam_held, -h->cam_fixed_sum, (double)(box.flags & 1), (double)(box.flags & 6),
+                    box.cam_sum, -box.cam_sum};
     LCBA_CUDA(h, cudaMemcpyAsync(h->d_red, v, sizeof(v), cudaMemcpyHostToDevice, h->stream));
     LCBA_TRY(allreduce(h, h->d_red, 2, NCCL_SUM));
-    LCBA_TRY(allreduce(h, h->d_red + 2, 4, NCCL_MAX));
+    LCBA_TRY(allreduce(h, h->d_red + 2, 8, NCCL_MAX));
     LCBA_CUDA(h, cudaMemcpyAsync(v, h->d_red, sizeof(v), cudaMemcpyDeviceToHost, h->stream));
     LCBA_CUDA(h, cudaStreamSynchronize(h->stream));
     h->P_total = (long long)(v[0] + 0.5);
@@ -1295,10 +1526,29 @@ extern "C" int lcba_solve(lcba_t* h, const lcba_options* opt_in, lcba_result* re
       set_error(h, "lcba_solve: the ranks hold different camera masks (lcba_set_fixed)");
       return LCBA_E_ARG;
     }
+    box.flags = (v[6] != 0.0 ? 1 : 0) | (int)v[7];
+    if (v[6] != 0.0 && v[8] != -v[9]) {
+      set_error(h, "lcba_solve: the ranks hold different camera bounds (lcba_set_bounds)");
+      return LCBA_E_ARG;
+    }
   }
-  h->fix_cameras = opt.fix_cameras ? 1 : 0;
-  h->shared_intr = (opt.shared_intrinsics && !h->fix_cameras) ? 1 : 0;
-  h->masks_on = true;
+  h->bounded = false;
+  if (box.flags & 1) {
+    if (h->fix_cameras || h->shared_intr) {
+      set_error(h, "lcba_solve: box bounds together with fix_cameras or shared_intrinsics are not supported");
+      return LCBA_E_UNSUPPORTED;
+    }
+    if (box.flags & 2) {
+      set_error(h, "lcba_solve: each lower bound must be strictly less than each upper bound (lcba_set_bounds)");
+      return LCBA_E_ARG;
+    }
+    if (box.flags & 4) {
+      set_error(h, "lcba_solve: the initial guess is outside of the bounds (lcba_set_bounds)");
+      return LCBA_E_ARG;
+    }
+    LCBA_TRY(box_upload(h, box, true));
+    h->bounded = true;
+  }
   if (h->shared_intr && h->n_cam_held) {
     set_error(h, "lcba_solve: a camera mask together with shared_intrinsics is not supported");
     return LCBA_E_UNSUPPORTED;
@@ -1312,7 +1562,7 @@ extern "C" int lcba_solve(lcba_t* h, const lcba_options* opt_in, lcba_result* re
   // 2.12 vs 1.80 at 8) and fewer than 8 M observations (above, an iteration is several ms of long kernels: A/B on
   // one box, ring24 x 1 M: 8.06 / 8.36 vs 8.12 / 8.13 ms, and the capture + instantiation of the four graphs
   // would fall into the second solve)
-  const bool graphs = h->solves_on_problem >= 1 && !h->comm && h->N < (8LL << 20);
+  const bool graphs = h->solves_on_problem >= 1 && !h->comm && h->N < (8LL << 20) && !h->bounded;
   h->solves_on_problem++;
   const int gkey = h->fix_cameras * 2 + h->shared_intr;
   const long long n_cam = h->fix_cameras ? 0 : (h->shared_intr ? 3 + 8LL * h->C : (long long)h->C * NCP - h->n_cam_held);
@@ -1376,7 +1626,7 @@ extern "C" int lcba_solve(lcba_t* h, const lcba_options* opt_in, lcba_result* re
       if (h->fix_cameras) {
         // points only: the normal equations are block diagonal, p_p = (V + lam Dp^2)^-1 g_p
         KL(h, "point_factor", k_point_factor<<<nblk(h->P, 256), 256, 0, h->stream>>>(
-              h->d_Vg, h->d_scl_p, 0.0, h->d_ctl, h->P, pt_mask(h), h->d_Lz));
+              h->d_Vg, h->d_scl_p, 0.0, h->d_ctl, h->P, pt_mask(h), nullptr, h->d_Lz));
         LCBA_CUDA(h, cudaMemsetAsync(h->d_pc, 0, (size_t)h->C * NCP * 8, h->stream));
         LCBA_CUDA(h, cudaMemsetAsync(h->d_fail, 0, 2 * sizeof(int), h->stream));
       } else {
@@ -1541,6 +1791,7 @@ extern "C" int lcba_linearize(lcba_t* h, double lam, double* S_out, double* rhs_
   h->fix_cameras = 0;
   h->shared_intr = 0;
   h->masks_on = false;
+  h->bounded = false;
   LCBA_TRY(pass_linearize(h, 1));
   LCBA_TRY(pass_schur(h, &lam));
   const int n = h->C * NCP;
@@ -1994,11 +2245,27 @@ extern "C" int lcba_debug_step(lcba_t* h, double lam, double mu, int32_t mode, d
     set_error(h, "lcba_debug_step: every parameter is held (lcba_set_fixed)");
     return LCBA_E_ARG;
   }
+  // the bounded loop's damping and Gram diagonal at the current x (which must lie inside the box)
+  BoxSetup box;
+  LCBA_TRY(box_setup(h, h->fix_cameras != 0, box));
+  h->bounded = false;
+  if (box.flags & 1) {
+    if (mode != 0) {
+      set_error(h, "lcba_debug_step: box bounds are supported in mode 0 only");
+      return LCBA_E_UNSUPPORTED;
+    }
+    if (box.flags & (2 | 8)) {    // on a bound, v = 0 and d = 0: the tap needs x strictly inside
+      set_error(h, "lcba_debug_step: an empty box, or x not strictly inside the bounds (lcba_set_bounds)");
+      return LCBA_E_ARG;
+    }
+    LCBA_TRY(box_upload(h, box, false));
+    h->bounded = true;
+  }
   LCBA_TRY(pass_linearize(h, 1));
   LCBA_TRY(pass_jdot(h));
   if (h->fix_cameras) {
     KL(h, "point_factor", k_point_factor<<<nblk(h->P, 256), 256, 0, h->stream>>>(
-          h->d_Vg, h->d_scl_p, lam, nullptr, h->P, pt_mask(h), h->d_Lz));
+          h->d_Vg, h->d_scl_p, lam, nullptr, h->P, pt_mask(h), nullptr, h->d_Lz));
     LCBA_CUDA(h, cudaMemsetAsync(h->d_pc, 0, (size_t)h->C * NCP * 8, h->stream));
     LCBA_CUDA(h, cudaMemsetAsync(h->d_fail, 0, 2 * sizeof(int), h->stream));
   } else {
@@ -2038,9 +2305,10 @@ extern "C" int lcba_debug_i8_make(lcba_t* h, double lam, int32_t ref, int32_t re
   init.term = -1;
   LCBA_CUDA(h, cudaMemcpyAsync(h->d_ctl, &init, sizeof(Ctl), cudaMemcpyHostToDevice, h->stream));
   h->masks_on = true;
+  h->bounded = false;
   LCBA_TRY(pass_linearize(h, 1));
   KL(h, "point_factor", k_point_factor<<<nblk(h->P, 256), 256, 0, h->stream>>>(
-        h->d_Vg, h->d_scl_p, lam, nullptr, h->P, pt_mask(h), h->d_Lz));
+        h->d_Vg, h->d_scl_p, lam, nullptr, h->P, pt_mask(h), nullptr, h->d_Lz));
   launch_i8_rowexp(h);
   if (poison >= 0) LCBA_CUDA(h, cudaMemsetAsync(h->d_i8planes, poison, h->i8plan.plane_bytes, h->stream));
   cudaEvent_t e0, e1;

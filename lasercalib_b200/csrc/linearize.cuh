@@ -294,10 +294,12 @@ k_jdot(const double* __restrict__ tab, const double* __restrict__ pts,
 // trip) when `ctl` is given, from the argument otherwise (lcba_linearize debug tap).
 // A held point (pt_fixed[p] != 0; pt_fixed may be NULL) gets L^-1 = 0 and z = 0: its Y = W L^-T
 // vanishes, so it subtracts nothing from S, and its step L^-T L^-1 (.) is exactly 0.
+// dh (bounded loop only, else NULL): diag_h per coordinate; the damping becomes (lam + diag_h) scl^2 with
+// scl = 1 / d (bounds.cuh).
 __global__ void __launch_bounds__(256)
 k_point_factor(const double* __restrict__ Vg, const double* __restrict__ scl, double lam,
                const Ctl* __restrict__ ctl, long long P, const uint8_t* __restrict__ pt_fixed,
-               double* __restrict__ Lz) {
+               const double* __restrict__ dh, double* __restrict__ Lz) {
   const long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (p >= P) return;
   if (pt_fixed && pt_fixed[p]) {
@@ -308,8 +310,10 @@ k_point_factor(const double* __restrict__ Vg, const double* __restrict__ scl, do
   if (ctl) lam = ctl->reg_term;
   const double* v = Vg + p * 9;
   const double s0 = scl[3 * p], s1 = scl[3 * p + 1], s2 = scl[3 * p + 2];
-  const double v00 = fma(lam * s0, s0, v[0]), v11 = fma(lam * s1, s1, v[3]),
-               v22 = fma(lam * s2, s2, v[5]);
+  const double l0 = dh ? lam + dh[3 * p] : lam, l1 = dh ? lam + dh[3 * p + 1] : lam,
+               l2 = dh ? lam + dh[3 * p + 2] : lam;
+  const double v00 = fma(l0 * s0, s0, v[0]), v11 = fma(l1 * s1, s1, v[3]),
+               v22 = fma(l2 * s2, s2, v[5]);
   const double v01 = v[1], v02 = v[2], v12 = v[4];
   const double tiny = 1e-300;
   const double l00 = sqrt(fmax(v00, tiny));

@@ -494,11 +494,13 @@ k_schur(const double* __restrict__ tab, const double* __restrict__ pts,
 // those of the identity and rhs[i] into 0: dropping camera columns commutes with eliminating the
 // points, so the free block is the reduced system of the free parameters, and the Cholesky returns
 // an exact 0 for entry i (scl_c[i] = 1 there, so the retries' mu damping keeps the row diagonal).
+// dh (bounded loop only, else NULL): diag_h per camera entry; the damping becomes (lam + diag_h) scl_c^2 with
+// scl_c = 1 / d (bounds.cuh).
 __global__ void k_assemble_S(const double* __restrict__ red, int C, int npairs,
                              const double* __restrict__ camsum, const double* __restrict__ scl_c,
                              double lam, const Ctl* __restrict__ ctl,
-                             const uint8_t* __restrict__ cam_fixed, double* __restrict__ S,
-                             double* __restrict__ rhs) {
+                             const uint8_t* __restrict__ cam_fixed, const double* __restrict__ dh,
+                             double* __restrict__ S, double* __restrict__ rhs) {
   if (ctl) lam = ctl->reg_term;
   const int n = C * NCP;
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -520,7 +522,7 @@ __global__ void k_assemble_S(const double* __restrict__ red, int C, int npairs,
   }
   if (r == c) {
     const double s = scl_c[r];
-    v = fma(lam * s, s, v);
+    v = fma((dh ? lam + dh[r] : lam) * s, s, v);
     rhs[r] = camsum[(r / NCP) * 22 + (r % NCP)] + red[(size_t)npairs * 121 + r];
   }
   S[idx] = v;

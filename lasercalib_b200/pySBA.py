@@ -114,6 +114,35 @@ def normalize_fixed(fixed_camera_params, fixed_points, n_cameras, n_points):
     return cam, pt
 
 
+def normalize_bounds(bounds, x0, held=None):
+    """``bounds`` of ``bundleAdjust`` as ``least_squares`` takes it (a 2-tuple of scalars or arrays, or
+    ``scipy.optimize.Bounds``) -> (lb, ub) float arrays of x0's shape, or None when every bound of a free entry is
+    infinite (the unbounded loop runs, as scipy dispatches to trf_no_bounds).  ``held``: bool mask of the held
+    entries of x0, which are not checked.  Raises ValueError with least_squares' messages
+    (scipy/optimize/_lsq/least_squares.py:883-901)."""
+    from scipy.optimize import Bounds
+    from scipy.optimize._lsq.least_squares import prepare_bounds
+    if bounds is None:
+        return None
+    if isinstance(bounds, Bounds):
+        lb, ub = prepare_bounds((bounds.lb, bounds.ub), x0.shape[0])
+    elif len(bounds) == 2:
+        lb, ub = prepare_bounds(bounds, x0.shape[0])
+    else:
+        raise ValueError("`bounds` must contain 2 elements.")
+    if lb.shape != x0.shape or ub.shape != x0.shape:
+        raise ValueError("Inconsistent shapes between bounds and `x0`.")
+    free = np.ones(x0.shape, dtype=bool) if held is None else ~held
+    lf, uf, xf = lb[free], ub[free], x0[free]
+    if np.any(lf >= uf):
+        raise ValueError("Each lower bound must be strictly less than each upper bound.")
+    if not np.all((xf >= lf) & (xf <= uf)):
+        raise ValueError("Initial guess is outside of provided bounds")
+    if np.all(np.isneginf(lf)) and np.all(np.isposinf(uf)):
+        return None
+    return lb, ub
+
+
 def _print_header():
     # scipy/optimize/_lsq/common.py:545-548
     print("{:^15}{:^15}{:^15}{:^15}{:^15}{:^15}".format(
@@ -278,7 +307,7 @@ class PySBA:
     # ---- solver (pySBA.py:132-147) ----
     def bundleAdjust(self, ftol=1e-4, xtol=1e-8, gtol=1e-8, max_nfev=None, verbose=2,
                      profile=False, max_iterations=0, _fix_cameras=False, _shared=False,
-                     fixed_camera_params=None, fixed_points=None):
+                     fixed_camera_params=None, fixed_points=None, bounds=None):
         """Returns the bundle adjusted parameters (scipy ``OptimizeResult`` layout) and
         stores them on ``self.cameraArray`` / ``self.points3D``.
 
@@ -292,12 +321,28 @@ class PySBA:
         trust radius, ``|x|`` and ``|g|_inf`` over free entries, ``max_nfev`` = 100 * free count).
         ``x`` and ``jac`` keep the full layout, held entries of ``x`` equal the input bit for bit,
         ``grad`` is 0 there.  Holding camera 0's extrinsics and three non-collinear points (or one
-        scale coordinate) removes the 7-dimensional gauge freedom."""
+        scale coordinate) removes the 7-dimensional gauge freedom.
+
+        ``bounds`` (what ``least_squares`` takes: a 2-tuple of scalars or (n,) arrays over the layout
+        ``[cameraArray.ravel(), points3D.ravel()]``, or ``scipy.optimize.Bounds``) keeps x in the box: the solve is
+        scipy's ``trf_bounds`` (reflective TRF) with the exact Schur solve in place of LSMR; x0 is first moved strictly
+        inside as least_squares does.  ``optimality`` is then ``|g v|_inf`` (v: the Coleman-Li vector) and
+        ``active_mask`` marks the entries on a bound.  Held entries ignore their bounds.  Every bound infinite:
+        the unbounded solve, unchanged."""
         numCameras = self.cameraArray.shape[0]
         numPoints = self.points3D.shape[0]
         cam_fixed, pt_fixed = normalize_fixed(fixed_camera_params, fixed_points, numCameras, numPoints)
         cams0 = np.ascontiguousarray(self.cameraArray, dtype=np.float64)
         pts0 = np.ascontiguousarray(self.points3D, dtype=np.float64)
+        nc = numCameras * N_CAM_PARAMS
+        held = None
+        if cam_fixed is not None or pt_fixed is not None:
+            held = np.zeros(nc + 3 * numPoints, dtype=bool)
+            if cam_fixed is not None and not _fix_cameras:
+                held[:nc] = cam_fixed.ravel()
+            if pt_fixed is not None:
+                held[nc:] = np.repeat(pt_fixed, 3)
+        box = normalize_bounds(bounds, np.hstack((cams0.ravel(), pts0.ravel())), held)
         if _shared:
             # x0 of the reference: the mean (f, k1, k2) for every camera (pySBA.py:300)
             cams0 = cams0.copy()
@@ -343,6 +388,12 @@ class PySBA:
             pt_fixed_local = pt_fixed
         if cam_fixed is not None or pt_fixed_local is not None or eng.has_fixed:
             eng.set_fixed(cam_fixed, pt_fixed_local)
+        if box is not None:
+            lo, hi = (0, numPoints) if shard is None else (shard["lo"], shard["hi"])
+            eng.set_bounds(box[0][:nc], box[1][:nc], box[0][nc:].reshape(-1, 3)[lo:hi],
+                           box[1][nc:].reshape(-1, 3)[lo:hi])
+        elif eng.has_bounds:
+            eng.set_bounds()
         t_in1 = _time.perf_counter()
         live = None
         if verbose == 2:
@@ -361,7 +412,6 @@ class PySBA:
         self.last_trace = trace
         t_sol = _time.perf_counter()
         x_direct = None
-        nc = numCameras * N_CAM_PARAMS
         if not _fix_cameras and not _shared:
             # the reference's x = [cameras | points]: filled in place, the arrays are views
             x_direct = np.empty(nc + numPoints * 3)
@@ -401,14 +451,6 @@ class PySBA:
         def lazy_fun():
             return engine_at_result().residuals(None, want_cost=False)[0]
 
-        held = None
-        if cam_fixed is not None or pt_fixed is not None:
-            held = np.zeros(nc + 3 * numPoints, dtype=bool)
-            if cam_fixed is not None and not _fix_cameras:
-                held[:nc] = cam_fixed.ravel()
-            if pt_fixed is not None:
-                held[nc:] = np.repeat(pt_fixed, 3)
-
         def lazy_grad():
             e = engine_at_result()
             g = e.grad() if e.generation == gen else e.linearize(1.0)["grad"]
@@ -440,7 +482,14 @@ class PySBA:
         x = x_direct if x_direct is not None else np.hstack((cams.ravel(), pts.ravel()))
         out = BAResult(x=x, cost=res.cost, optimality=res.optimality,
                        nfev=int(res.nfev), njev=int(res.njev), status=int(res.status))
-        out.set_lazy("active_mask", lambda: np.zeros_like(x))
+        if box is None:
+            out.set_lazy("active_mask", lambda: np.zeros_like(x))
+        else:
+            from scipy.optimize._lsq.common import find_active_constraints
+            active = find_active_constraints(x, box[0], box[1], rtol=xtol)
+            if held is not None:
+                active[held] = 0
+            out["active_mask"] = active
         out["message"] = TERMINATION_MESSAGES[int(res.status)]
         out["success"] = int(res.status) > 0
         out["solve_ms"] = res.solve_ms
