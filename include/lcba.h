@@ -44,7 +44,9 @@ enum {
   LCBA_E_UNSUPPORTED = -4,/* >64 cameras, duplicate (camera, point) observation, ... */
   LCBA_E_NONFINITE = -5,  /* residuals not finite at the initial point
                              (scipy raises ValueError: _lsq/least_squares.py:945-946) */
-  LCBA_E_NCCL = -6
+  LCBA_E_NCCL = -6,
+  LCBA_E_SINGULAR = -7    /* lcba_covariance: the free parameters are not determined (gauge not fixed, a
+                             point seen by fewer than two cameras, an unconstrained camera entry) */
 };
 
 /* scipy termination codes (scipy/optimize/_lsq/least_squares.py:23-31) */
@@ -230,6 +232,14 @@ typedef void (*lcba_iteration_cb)(const lcba_trace_row* row, void* user);
 int lcba_set_iteration_callback(lcba_t* h, lcba_iteration_cb cb, void* user);
 int lcba_get_grad(lcba_t* h, double* g_out /* 11C + 3P, at the current x */);
 int lcba_get_profile(lcba_t* h, lcba_kernel_stat* stats, int32_t max_stats, int32_t* n_out);
+
+/* Unscaled covariance (J_f^T J_f)^-1 at the current x over the free entries of lcba_set_fixed's masks
+ * (bounds ignored).  cam_cov_out (11C)^2 full symmetric, held rows/columns 0; pt_cov_out P x 6 over THIS handle's
+ * points (00 01 02 11 12 22), held points 0; either may be NULL.  cost_out: 0.5|f|^2 over all ranks.
+ * min_pivot_out: min over free camera rows of l_jj^2 / S_jj.  LCBA_E_SINGULAR when an unheld point has < 2
+ * distinct cameras or S is not numerically positive definite; LCBA_E_ARG when everything is held.
+ * Collective on a point-sharded job. */
+int lcba_covariance(lcba_t* h, double* cam_cov_out, double* pt_cov_out, double* cost_out, double* min_pivot_out);
 
 /* ---- debug / parity taps -----------------------------------------------------------
  * Linearise at the current x and form the damped reduced camera system

@@ -12,7 +12,8 @@ LIB_PATH = os.path.join(_PKG, "liblcba.so")
 
 LCBA_MAX_TRACE = 512
 E_NAMES = {-1: "LCBA_E_ARG", -2: "LCBA_E_CUDA", -3: "LCBA_E_STATE", -4: "LCBA_E_UNSUPPORTED",
-           -5: "LCBA_E_NONFINITE", -6: "LCBA_E_NCCL"}
+           -5: "LCBA_E_NONFINITE", -6: "LCBA_E_NCCL", -7: "LCBA_E_SINGULAR"}
+E_SINGULAR = -7
 
 # every symbol include/lcba.h declares (tests/test_cabi.py checks the export list)
 SYMBOLS = ["lcba_version", "lcba_create", "lcba_destroy", "lcba_last_error", "lcba_default_options",
@@ -24,7 +25,7 @@ SYMBOLS = ["lcba_version", "lcba_create", "lcba_destroy", "lcba_last_error", "lc
            "lcba_set_iteration_callback", "lcba_debug_i8_plan", "lcba_host_is_nondecreasing_i64", "lcba_debug_peer_reduce",
            "lcba_debug_i8_fallback", "lcba_debug_chol", "lcba_debug_step", "lcba_debug_i8_cover_plan",
            "lcba_debug_i8_make", "lcba_set_fixed", "lcba_debug_i8_schedule", "lcba_set_bounds",
-           "lcba_get_active_mask"]
+           "lcba_get_active_mask", "lcba_covariance"]
 
 # scalars_out of lcba_debug_step, in order (include/lcba.h)
 STEP_SCALARS = ["reg_term", "Delta", "Jg2", "aa", "ab", "bb", "JAA", "JAB", "JBB", "gtgt", "gtp", "pp",
@@ -98,6 +99,7 @@ def load():
     lib.lcba_set_fixed.argtypes = [vp, vp, vp]
     lib.lcba_set_bounds.argtypes = [vp, vp, vp, vp, vp]
     lib.lcba_get_active_mask.argtypes = [vp, dbl, vp]
+    lib.lcba_covariance.argtypes = [vp, vp, vp, pd, pd]
     lib.lcba_rotate.argtypes = [vp, i64, vp, vp, vp]
     lib.lcba_project.argtypes = [vp, i64, vp, vp, vp]
     lib.lcba_unproject.argtypes = [vp, i64, vp, vp, i64, vp, vp, vp, vp, vp]
@@ -376,6 +378,18 @@ class Engine:
         self._check(self.lib.lcba_linearize(self.h, float(lam), _ptr(S), _ptr(rhs), _ptr(g),
                                             _ptr(sc), C.byref(cost)))
         return dict(S=S, rhs=rhs, grad=g, scale_inv=sc, cost=cost.value)
+
+    def covariance(self, points=True):
+        """Unscaled covariance (J_f^T J_f)^-1 at the current x over the entries lcba_set_fixed leaves free
+        (lcba_covariance; bounds ignored): (camera block (11 C, 11 C), this handle's point blocks (P, 6) as
+        00 01 02 11 12 22 or None, cost, min_pivot).  Held entries are 0.  Raises LcbaError with code E_SINGULAR
+        when the free parameters are not determined.  Collective on a point-sharded job."""
+        n = 11 * self.C
+        cam = np.empty((n, n))
+        pt = np.empty((self.P, 6)) if points else None
+        cost, piv = C.c_double(), C.c_double()
+        self._check(self.lib.lcba_covariance(self.h, _ptr(cam), _ptr(pt), C.byref(cost), C.byref(piv)))
+        return cam, pt, cost.value, piv.value
 
     def i8_fell_back(self):
         """1: the last Schur pass of the int8 path was recomputed on DMMA (rows finer than its digits resolve),

@@ -253,6 +253,81 @@ k_chol_fused(double* A, int n, double* __restrict__ out, int* sync, long long* d
 #undef CH_TICK
 }
 
+// ---- inverse of the factor (lcba_covariance) ---------------------------------------------
+// X = L^-1 from k_chol_fused's factor (A: ld n, strict lower L, diagonal 1 / l_jj), one CTA per column j of X:
+// blocked forward substitution L x = e_j, 32 rows at a time (one warp solves the diagonal block, every thread
+// updates the rows below).  X: ldx x ldx row-major, cleared by the caller; rows and columns i with held[i] != 0
+// (held may be NULL) stay 0, so that held camera entries drop out of S^-1 = X^T X and of Z_p = X Y_p.
+__global__ void __launch_bounds__(256)
+k_chol_inverse(const double* __restrict__ A, int n, const uint8_t* __restrict__ held, int ldx, double* __restrict__ X) {
+  __shared__ double x[CH_MAXN + CH_NB];
+  const int j = blockIdx.x, t = threadIdx.x, lane = t & 31, wid = t >> 5;
+  if (held && held[j]) return;
+  for (int i = t; i < n; i += 256) x[i] = (i == j) ? 1.0 : 0.0;
+  __syncthreads();
+  for (int i0 = j / CH_NB * CH_NB; i0 < n; i0 += CH_NB) {
+    const int nb = min(CH_NB, n - i0);
+    if (wid == 0) {
+      double l[CH_NB];
+      const double* row = A + (size_t)(i0 + lane) * n + i0;
+#pragma unroll
+      for (int c = 0; c < CH_NB; ++c) l[c] = (lane < nb && c <= lane) ? row[c] : 0.0;
+      double v = lane < nb ? x[i0 + lane] : 0.0;
+#pragma unroll
+      for (int c = 0; c < CH_NB; ++c) {
+        if (lane == c) v *= l[c];
+        const double xc = __shfl_sync(0xffffffffu, v, c);
+        if (lane > c) v = fma(-l[c], xc, v);
+      }
+      if (lane < nb) x[i0 + lane] = v;
+    }
+    __syncthreads();
+    for (int r = i0 + nb + t; r < n; r += 256) {
+      const double* row = A + (size_t)r * n + i0;
+      double s = x[r];
+#pragma unroll 8
+      for (int c = 0; c < nb; ++c) s = fma(-row[c], x[i0 + c], s);
+      x[r] = s;
+    }
+    __syncthreads();
+  }
+  for (int i = j + t; i < n; i += 256) X[(size_t)i * ldx + j] = (held && held[i]) ? 0.0 : x[i];
+}
+
+// Sinv (n x n, both triangles) = X^T X for a lower-triangular X (ld ldx): 32 x 32 output tiles (ti >= tj), the sum
+// over k >= 32 ti in a fixed order
+__global__ void __launch_bounds__(256)
+k_chol_inverse_gram(const double* __restrict__ X, int n, int ldx, double* __restrict__ Sinv) {
+  const int ti = blockIdx.x, tj = blockIdx.y;
+  if (tj > ti) return;
+  __shared__ double Xa[CH_NB][CH_NB + 1], Xb[CH_NB][CH_NB + 1];
+  const int t = threadIdx.x, lane = t & 31, wid = t >> 5;
+  double s[4] = {0.0, 0.0, 0.0, 0.0};
+  for (int k0 = ti * CH_NB; k0 < n; k0 += CH_NB) {
+    __syncthreads();
+    for (int e = t; e < CH_NB * CH_NB; e += 256) {
+      const int kk = e / CH_NB, c = e % CH_NB, k = k0 + kk;
+      Xa[kk][c] = (k < n && ti * CH_NB + c < n) ? X[(size_t)k * ldx + ti * CH_NB + c] : 0.0;
+      Xb[kk][c] = (k < n && tj * CH_NB + c < n) ? X[(size_t)k * ldx + tj * CH_NB + c] : 0.0;
+    }
+    __syncthreads();
+#pragma unroll 8
+    for (int kk = 0; kk < CH_NB; ++kk) {
+      const double b = Xb[kk][lane];
+#pragma unroll
+      for (int m = 0; m < 4; ++m) s[m] = fma(Xa[kk][wid + 8 * m], b, s[m]);
+    }
+  }
+#pragma unroll
+  for (int m = 0; m < 4; ++m) {
+    const int a = ti * CH_NB + wid + 8 * m, b = tj * CH_NB + lane;
+    if (a < n && b < n && b <= a) {
+      Sinv[(size_t)a * n + b] = s[m];
+      Sinv[(size_t)b * n + a] = s[m];
+    }
+  }
+}
+
 // A_out (n + 1 rows) = [A_in + mu * diag(d^2) ; rhs]
 __global__ void k_copy_damped_rhs(const double* __restrict__ Ain, int n, double mu,
                                   const double* __restrict__ d, const double* __restrict__ rhs,

@@ -26,6 +26,7 @@
 #include "peer_reduce.cuh"
 #include "variants.cuh"
 #include "bounds.cuh"
+#include "covariance.cuh"
 
 using namespace lcba;
 
@@ -176,6 +177,9 @@ struct lcba_handle {
   Bnd* d_bnd = nullptr;
   double *d_pred = nullptr, *d_scl_red = nullptr;   // shared-intrinsics mode: reduced step / scale
   double *d_sqpart = nullptr, *d_sqout = nullptr, *d_theta = nullptr;   // squared-residual variants
+  // lcba_covariance, allocated by its first call (no captured graph references them): X = L_S^-1 (n_pad^2),
+  // S^-1 (n^2), the per-point blocks (P x 6)
+  double *d_cov_X = nullptr, *d_cov_Sinv = nullptr, *d_cov_pt = nullptr;
   int sq_grid = 0, sq_K = 0;
 };
 
@@ -350,7 +354,8 @@ extern "C" int lcba_create(lcba_t** out, int device) {
                                       (const void*)k_residual_pt, (const void*)k_jdot_pt, (const void*)k_backsub_pt,
                                       (const void*)k_i8_syrk, (const void*)k_i8_make,
                                       (const void*)k_i8_make_ref,
-                                      (const void*)k_jdot,      (const void*)k_jacobian_blocks};
+                                      (const void*)k_jdot,      (const void*)k_jacobian_blocks,
+                                      (const void*)k_point_cov<16>, (const void*)k_point_cov<8>};
     for (const void* f : big_smem_kernels) {
       cudaFuncAttributes fa;
       e = cudaFuncGetAttributes(&fa, f);
@@ -412,6 +417,7 @@ extern "C" int lcba_set_problem_shard(lcba_t* h, int32_t C, int64_t P, int64_t N
   h->have_problem = false;
   h->d_rout = nullptr; h->d_Jc = nullptr; h->d_Jp = nullptr;
   h->d_sqpart = nullptr; h->d_sqout = nullptr; h->d_theta = nullptr; h->sq_grid = 0; h->sq_K = 0;
+  h->d_cov_X = h->d_cov_Sinv = h->d_cov_pt = nullptr;
   h->C = C; h->P = P; h->N = N; h->P_total = P; h->cur = 0;
   cudaStream_t st = h->stream;
 
@@ -1806,6 +1812,127 @@ extern "C" int lcba_linearize(lcba_t* h, double lam, double* S_out, double* rhs_
     LCBA_CUDA(h, cudaStreamSynchronize(h->stream));
   }
   return check_launch(h, "lcba_linearize");
+}
+
+// Smallest Jacobi-relative pivot l_jj^2 / S_jj of the free camera rows below which S counts as singular.  At the
+// gauge-fixed solutions of the golden rigs it is 5e-4 .. 9e-4; with the gauge free it is rounding noise of
+// either sign, |.| <= 2e-10 (tests/test_covariance.py recomputes both).
+static const double COV_PIVOT_TOL = 1e-7;
+
+extern "C" int lcba_covariance(lcba_t* h, double* cam_cov_out, double* pt_cov_out, double* cost_out,
+                               double* min_pivot_out) {
+  if (!h || !h->have_problem) { set_error(h, "lcba_covariance: no problem set"); return LCBA_E_STATE; }
+  cudaSetDevice(h->device);
+  const int C = h->C, n = C * NCP, npad = cov_npad(n);
+  cudaStream_t st = h->stream;
+  // free-entry counts over the ranks; the camera mask must be the same on every rank (as in lcba_solve)
+  long long pt_free = h->P - h->n_pt_held;
+  if (h->comm) {
+    double v[5] = {(double)pt_free, (double)h->n_cam_held, h->cam_fixed_sum, -(double)h->n_cam_held, -h->cam_fixed_sum};
+    LCBA_CUDA(h, cudaMemcpyAsync(h->d_red, v, sizeof(v), cudaMemcpyHostToDevice, st));
+    LCBA_TRY(allreduce(h, h->d_red, 1, NCCL_SUM));
+    LCBA_TRY(allreduce(h, h->d_red + 1, 4, NCCL_MAX));
+    LCBA_CUDA(h, cudaMemcpyAsync(v, h->d_red, sizeof(v), cudaMemcpyDeviceToHost, st));
+    LCBA_CUDA(h, cudaStreamSynchronize(st));
+    if (v[1] != -v[3] || v[2] != -v[4]) {
+      set_error(h, "lcba_covariance: the ranks hold different camera masks (lcba_set_fixed)");
+      return LCBA_E_ARG;
+    }
+    pt_free = (long long)(v[0] + 0.5);
+  }
+  const long long cam_free = n - h->n_cam_held;
+  if (cam_free + 3 * pt_free <= 0) {
+    set_error(h, "lcba_covariance: every parameter is held (lcba_set_fixed): nothing to estimate");
+    return LCBA_E_ARG;
+  }
+  // LCBA_COV_PROFILE=1: CUDA-event time of every launch of this call (synchronising after each), for
+  // lcba_get_profile (tools/cov_time.py); off again on every return
+  struct ProfOff { lcba_t* h; ~ProfOff() { h->prof_on = false; } } prof_off{h};
+  {
+    const char* pe = getenv("LCBA_COV_PROFILE");
+    h->prof_on = pe && atoi(pe) != 0;
+    if (h->prof_on) h->prof.clear();
+  }
+  Ctl init;
+  memset(&init, 0, sizeof(init));
+  init.term = -1;
+  LCBA_CUDA(h, cudaMemcpyAsync(h->d_ctl, &init, sizeof(Ctl), cudaMemcpyHostToDevice, st));
+  h->fix_cameras = 0;
+  h->shared_intr = 0;
+  h->masks_on = true;
+  h->bounded = false;
+  LCBA_TRY(pass_linearize(h, 1));
+  // unheld points with fewer than two distinct cameras (k_point_factor would clamp their pivots)
+  double* views = h->d_red + 40;
+  KL(h, "cov_views", k_cov_views<<<h->pt_grid, 256, 0, st>>>(h->d_mask, h->d_pt_fixed, h->P, h->d_part));
+  KL(h, "reduce", k_reduce_scalars<<<1, 256, 0, st>>>(h->d_part, h->pt_grid, 1, views, 1));
+  LCBA_TRY(allreduce(h, views, 1, NCCL_SUM));
+  // the exact undamped reduced camera system on the problem's Schur route, and its Cholesky factor
+  const double lam = 0.0;
+  LCBA_TRY(pass_schur(h, &lam));
+  LCBA_TRY(pass_camera_solve(h, 0.0));
+  double nviews = 0.0;
+  int fail = 0;
+  std::vector<double> dinv(n), sdiag(n);
+  LCBA_CUDA(h, cudaMemcpyAsync(&nviews, views, 8, cudaMemcpyDeviceToHost, st));
+  LCBA_CUDA(h, cudaMemcpyAsync(&fail, h->d_fail, sizeof(int), cudaMemcpyDeviceToHost, st));
+  LCBA_CUDA(h, cudaMemcpy2DAsync(dinv.data(), 8, h->d_Lf, (size_t)(n + 1) * 8, 8, n, cudaMemcpyDeviceToHost, st));
+  LCBA_CUDA(h, cudaMemcpy2DAsync(sdiag.data(), 8, h->d_S, (size_t)(n + 1) * 8, 8, n, cudaMemcpyDeviceToHost, st));
+  LCBA_TRY(read_ctl(h));
+  if (fail & 2) { set_error(h, "k_chol_fused: grid barrier timed out"); return LCBA_E_CUDA; }
+  if (cost_out) *cost_out = h->h_ctl->cost;
+  // Jacobi-relative pivots of the free rows (the diagonal of the factor stores 1 / l_jj); a non-positive pivot
+  // (fail bit 0) reports 0
+  double min_pivot = INFINITY;
+  for (int j = 0; j < n; ++j)
+    if (h->h_cam_fixed.empty() || !h->h_cam_fixed[j]) min_pivot = std::min(min_pivot, 1.0 / (dinv[j] * dinv[j] * sdiag[j]));
+  if (fail & 1) min_pivot = 0.0;
+  if (min_pivot_out) *min_pivot_out = min_pivot;
+  if (nviews > 0.0) {
+    set_error(h, "lcba_covariance: " + std::to_string((long long)(nviews + 0.5)) +
+                     " unheld point(s) seen by fewer than two distinct cameras: their position is not determined; "
+                     "hold them (fixed_points) or drop them");
+    return LCBA_E_SINGULAR;
+  }
+  if (cam_free > 0 && !(min_pivot >= COV_PIVOT_TOL)) {
+    char buf[96];
+    snprintf(buf, sizeof(buf), "(smallest Jacobi-relative pivot %.3g < %.0e)", min_pivot, COV_PIVOT_TOL);
+    set_error(h, std::string("lcba_covariance: the reduced camera system is singular ") + buf +
+                     ": the gauge (rotation, translation, scale) is not fixed or a camera entry is unconstrained; "
+                     "hold camera 0's extrinsics and three points or one scale coordinate (fixed_camera_params, "
+                     "fixed_points), and every entry of a camera that sees no point");
+    return LCBA_E_SINGULAR;
+  }
+  if (!h->d_cov_X) {
+    LCBA_TRY(dev_alloc(h, &h->d_cov_X, (size_t)npad * npad));
+    LCBA_TRY(dev_alloc(h, &h->d_cov_Sinv, (size_t)n * n));
+    LCBA_TRY(dev_alloc(h, &h->d_cov_pt, (size_t)h->P * 6));
+  }
+  LCBA_CUDA(h, cudaMemsetAsync(h->d_cov_X, 0, (size_t)npad * npad * 8, st));
+  KL(h, "chol_inverse", k_chol_inverse<<<n, 256, 0, st>>>(h->d_Lf, n, h->d_cam_fixed, npad, h->d_cov_X));
+  const unsigned nt = (unsigned)((n + CH_NB - 1) / CH_NB);
+  KL(h, "chol_inverse_gram", k_chol_inverse_gram<<<dim3(nt, nt), 256, 0, st>>>(h->d_cov_X, n, npad, h->d_cov_Sinv));
+  if (pt_cov_out) {
+    const int w = h->cur;
+    const bool b16 = cov_smem_doubles(C, 16) * 8 + 2048 <= h->smem_optin;
+    const size_t smem = cov_smem_doubles(C, b16 ? 16 : 8) * 8;
+    const long long nbatch = (h->P + (b16 ? 16 : 8) - 1) / (b16 ? 16 : 8);
+    const int per_sm = std::max(1, (int)(h->smem_optin / (smem + 1024)));
+    const int grid = (int)std::max<long long>(1, std::min<long long>(nbatch, (long long)h->sm_count * per_sm));
+    if (b16)
+      KL(h, "point_cov", k_point_cov<16><<<grid, COV_THREADS, smem, st>>>(
+            h->d_cov_X, h->d_tab[w], h->d_pts[w], h->d_pair_w, h->d_pair_start, h->d_mask, h->d_Lz, h->P, C,
+            h->d_cov_pt));
+    else
+      KL(h, "point_cov", k_point_cov<8><<<grid, COV_THREADS, smem, st>>>(
+            h->d_cov_X, h->d_tab[w], h->d_pts[w], h->d_pair_w, h->d_pair_start, h->d_mask, h->d_Lz, h->P, C,
+            h->d_cov_pt));
+    LCBA_CUDA(h, cudaMemcpyAsync(pt_cov_out, h->d_cov_pt, (size_t)h->P * 6 * 8, cudaMemcpyDeviceToHost, st));
+  }
+  if (cam_cov_out)
+    LCBA_CUDA(h, cudaMemcpyAsync(cam_cov_out, h->d_cov_Sinv, (size_t)n * n * 8, cudaMemcpyDeviceToHost, st));
+  LCBA_CUDA(h, cudaStreamSynchronize(st));
+  return check_launch(h, "lcba_covariance");
 }
 
 extern "C" int lcba_time_device(lcba_t* h, int32_t what, int32_t reps, double* ms_out) {

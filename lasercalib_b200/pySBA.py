@@ -143,6 +143,40 @@ def normalize_bounds(bounds, x0, held=None):
     return lb, ub
 
 
+def covariance_result(cam_cov, pt6, cost, min_pivot, m, cam_fixed=None, pt_fixed=None, absolute_sigma=False):
+    """``PySBA.covariance``'s result from lcba_covariance's unscaled blocks: cam_cov (11 C, 11 C), pt6 (P, 6) as
+    00 01 02 11 12 22, cost = 0.5 |f|^2, m residuals, the held masks of ``normalize_fixed`` (or None).  Applies
+    curve_fit's ``s^2 = 2 cost / (m - n_free)`` unless ``absolute_sigma``; ``dof <= 0`` fills the free entries with
+    inf and warns (scipy/optimize/_minpack_py.py, curve_fit)."""
+    n_cam = cam_cov.shape[0]
+    P = pt6.shape[0]
+    cam_free = np.ones(n_cam, dtype=bool) if cam_fixed is None else ~np.asarray(cam_fixed).ravel()
+    pt_free = np.ones(P, dtype=bool) if pt_fixed is None else ~np.asarray(pt_fixed)
+    n_free = int(cam_free.sum()) + 3 * int(pt_free.sum())
+    dof = int(m) - n_free
+    iu = np.array([[0, 1, 2], [1, 3, 4], [2, 4, 5]])
+    point_cov = np.asarray(pt6)[:, iu]
+    camera_cov = np.array(cam_cov, dtype=np.float64)
+    sigma2 = 1.0
+    if not absolute_sigma:
+        if dof > 0:
+            sigma2 = 2.0 * cost / dof
+            camera_cov *= sigma2
+            point_cov *= sigma2
+        else:
+            import warnings
+            from scipy.optimize import OptimizeWarning
+            sigma2 = np.inf
+            camera_cov[np.ix_(cam_free, cam_free)] = np.inf
+            point_cov[pt_free] = np.inf
+            warnings.warn("Covariance of the parameters could not be estimated", category=OptimizeWarning,
+                          stacklevel=3)
+    return OptimizeResult(camera_cov=camera_cov,
+                          camera_std=np.sqrt(np.diag(camera_cov)).reshape(-1, N_CAM_PARAMS),
+                          point_cov=point_cov, point_std=np.sqrt(np.einsum("paa->pa", point_cov)),
+                          sigma2=sigma2, dof=dof, cost=cost, min_pivot=min_pivot)
+
+
 def _print_header():
     # scipy/optimize/_lsq/common.py:545-548
     print("{:^15}{:^15}{:^15}{:^15}{:^15}{:^15}".format(
@@ -264,6 +298,35 @@ class PySBA:
             self._keep = (ci, pi, p2, w, pointWeights)   # keep the keyed buffers alive
         return eng
 
+    def _ensure_shard(self, cams0, pts0, rank, ws):
+        """Point-sharded counterpart of _ensure_problem (collective): one process per GPU, this rank keeps a
+        contiguous range of points and their observations; cameras are replicated; the library all-reduces with
+        NCCL.  x is (cams0, this rank's rows of pts0).  Returns (engine, shard)."""
+        w = self._weights_arg(self._pointWeights)
+        eng = self._get_engine()
+        key = ("shard", ws, cams0.shape[0], pts0.shape[0], id(self.points2D),
+               id(self.cameraIndices), id(self.point2DIndices), None if w is None else id(self._pointWeights))
+        reuse = (self.observations_static and key == self._problem_key and eng._owner is self
+                 and eng._owner_token == self._owner_token)
+        if reuse:
+            shard = self._shard
+            eng.set_params(cams0, shard["pts0_of"](pts0))
+        else:
+            shard = _dist.shard_problem(pts0, self.points2D, self.cameraIndices,
+                                        self.point2DIndices, w, rank, ws, collective=True)
+            lo, hi = shard["lo"], shard["hi"]
+            shard["pts0_of"] = lambda p, lo=lo, hi=hi: np.ascontiguousarray(p[lo:hi])
+            eng.set_problem(cams0, shard["pts"], shard["points_2d"], shard["camera_ind"],
+                            shard["point_ind"], shard["weights"], pt_offset=shard["pt_offset"])
+            self._problem_key = key
+            self._shard = shard
+            eng._owner = self
+            self._owner_token = eng._owner_token = object()
+        if not eng._comm_ready:
+            _dist.connect_engine(eng)
+            eng._comm_ready = True
+        return eng, shard
+
     # ---- model (pySBA.py:61-89) ----
     def rotate(self, points, rot_vecs):
         """Rotate points by given rotation vectors (Rodrigues), row by row."""
@@ -352,31 +415,7 @@ class PySBA:
         rank, ws, _ = _dist.world()
         shard = None
         if ws > 1:
-            # one process per GPU: this rank keeps a contiguous range of points and their
-            # observations; cameras are replicated; the library all-reduces with NCCL
-            w = self._weights_arg(self._pointWeights)
-            eng = self._get_engine()
-            key = ("shard", ws, cams0.shape[0], pts0.shape[0], id(self.points2D),
-                   id(self.cameraIndices), id(self.point2DIndices), None if w is None else id(self._pointWeights))
-            reuse = (self.observations_static and key == self._problem_key and eng._owner is self
-                     and eng._owner_token == self._owner_token)
-            if reuse:
-                shard = self._shard
-                eng.set_params(cams0, shard["pts0_of"](pts0))
-            else:
-                shard = _dist.shard_problem(pts0, self.points2D, self.cameraIndices,
-                                            self.point2DIndices, w, rank, ws, collective=True)
-                lo, hi = shard["lo"], shard["hi"]
-                shard["pts0_of"] = lambda p, lo=lo, hi=hi: np.ascontiguousarray(p[lo:hi])
-                eng.set_problem(cams0, shard["pts"], shard["points_2d"], shard["camera_ind"],
-                                shard["point_ind"], shard["weights"], pt_offset=shard["pt_offset"])
-                self._problem_key = key
-                self._shard = shard
-                eng._owner = self
-                self._owner_token = eng._owner_token = object()
-            if not eng._comm_ready:
-                _dist.connect_engine(eng)
-                eng._comm_ready = True
+            eng, shard = self._ensure_shard(cams0, pts0, rank, ws)
             if verbose and rank != 0:
                 verbose = 0
             pt_fixed_local = None if pt_fixed is None else pt_fixed[shard["lo"]:shard["hi"]]
@@ -527,6 +566,55 @@ class PySBA:
         self.cameraArray = camera_params
         self.points3D = points_3d
         return out
+
+    # ---- uncertainty of the solution ----
+    def covariance(self, fixed_camera_params=None, fixed_points=None, absolute_sigma=False):
+        """Covariance of the least-squares estimate at ``cameraArray`` / ``points3D`` (after ``bundleAdjust``: the
+        solution), as ``scipy.optimize.curve_fit`` returns ``pcov``: ``s^2 (J_f^T J_f)^-1`` over the free
+        parameters, ``J_f`` the Jacobian of ``fun`` (weights included) over the entries that
+        ``fixed_camera_params`` / ``fixed_points`` (as in ``bundleAdjust``) leave free and
+        ``s^2 = 2 cost / (m - n_free)``, m = 2 N residuals.  ``absolute_sigma=True``: no ``s^2`` (the weights are
+        1 / sigma of the pixel noise).  Bounds are ignored, as curve_fit ignores them.
+
+        Returns an ``OptimizeResult`` with ``camera_cov`` (11 C, 11 C), ``camera_std`` (C, 11), ``point_cov``
+        (P, 3, 3) (the 3 x 3 diagonal blocks; no camera-point or point-point cross terms), ``point_std`` (P, 3),
+        ``sigma2``, ``dof``, ``cost`` and ``min_pivot`` (the smallest Jacobi-relative pivot ``l_jj^2 / S_jj`` of the
+        reduced camera system).  Held entries are 0.  With ``dof <= 0`` and ``absolute_sigma=False`` the free
+        entries are ``inf`` and an ``OptimizeWarning`` is issued, as curve_fit does.
+
+        The covariance depends on the gauge: the 7 free modes of the problem (rotation, translation, scale) have
+        to be held, e.g. camera 0's extrinsics and three non-collinear points; the result describes the other
+        parameters relative to what is held.  Raises ``numpy.linalg.LinAlgError`` when the free parameters are
+        not determined (gauge not fixed, an unheld point seen by fewer than two cameras, an unconstrained camera
+        entry), ``ValueError`` on malformed masks.  Holding every camera gives the points-only covariance."""
+        numCameras = self.cameraArray.shape[0]
+        numPoints = self.points3D.shape[0]
+        cam_fixed, pt_fixed = normalize_fixed(fixed_camera_params, fixed_points, numCameras, numPoints)
+        cams0 = np.ascontiguousarray(self.cameraArray, dtype=np.float64)
+        pts0 = np.ascontiguousarray(self.points3D, dtype=np.float64)
+        rank, ws, _ = _dist.world()
+        shard = None
+        if ws > 1:
+            eng, shard = self._ensure_shard(cams0, pts0, rank, ws)
+            pt_fixed_local = None if pt_fixed is None else pt_fixed[shard["lo"]:shard["hi"]]
+        else:
+            eng = self._ensure_problem(cams0, pts0, self.cameraIndices, self.point2DIndices,
+                                       self.points2D, self._pointWeights)
+            if not self._fresh_problem:
+                eng.set_params(cams0, pts0)
+            pt_fixed_local = pt_fixed
+        if cam_fixed is not None or pt_fixed_local is not None or eng.has_fixed:
+            eng.set_fixed(cam_fixed, pt_fixed_local)
+        try:
+            cam_cov, pt6, cost, min_pivot = eng.covariance()
+        except _cabi.LcbaError as e:
+            if e.code == _cabi.E_SINGULAR:
+                raise np.linalg.LinAlgError(str(e)) from e
+            raise
+        if shard is not None:
+            pt6 = _dist.allgather_rows(pt6, shard["bounds"])
+        m = 2 * np.asarray(self.cameraIndices).size
+        return covariance_result(cam_cov, pt6, cost, min_pivot, m, cam_fixed, pt_fixed, absolute_sigma)
 
     # ---- variants of the reference that are not on the production path (SURVEY 8f) ----
     # ---- the two dense squared-residual variants (pySBA.py:151-206) ----
